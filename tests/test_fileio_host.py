@@ -1,6 +1,7 @@
 """CPU: bioen_b200.fileio -- the reference's pickle / HDF5 interface (bioen/fileio.py) and the problem-file layout of
 its optimisation tests (test/optimize/test_fileio_logw.py, test_fileio_forces.py)."""
-import os
+import pickle
+import struct
 
 import numpy as np
 import pytest
@@ -68,16 +69,46 @@ def test_hdf5_interface(tmp_path):
     assert np.array_equal(fio.load(fn, hdf5_keys=["yTilde"])[0], data[3])
 
 
-def test_reference_problem_files_load():
-    """The reference's own legacy (Python 2) pickles, where the reference tree is mounted (build container)."""
+def _py2_pickle(items):
+    """A list pickled the way Python 2 wrote the reference's problem files (protocol 2): np.matrix objects whose
+    dtype codes and raw data are Python 2 `str`s (SHORT_BINSTRING / BINSTRING), floats as BINFLOAT.  Python 3
+    reads such a file only with encoding="latin1"."""
+    def s(b):
+        return b"U" + bytes([len(b)]) + b if len(b) < 256 else b"T" + struct.pack("<i", len(b)) + b
+
+    def i(v):
+        return b"K" + bytes([v]) if 0 <= v < 256 else b"J" + struct.pack("<i", v)
+
+    def matrix(a):
+        a = np.ascontiguousarray(a, dtype="<f8")
+        dtype = (b"cnumpy\ndtype\n" + s(b"f8") + i(0) + i(1) + b"\x87R(" + i(3) + s(b"<") + b"NNN" + i(-1) + i(-1)
+                 + i(0) + b"tb")
+        return (b"cnumpy.core.multiarray\n_reconstruct\ncnumpy.matrixlib.defmatrix\nmatrix\n" + i(0) + b"\x85" + s(b"b")
+                + b"\x87R(" + i(1) + b"(" + b"".join(i(n) for n in a.shape) + b"t" + dtype + b"\x89" + s(a.tobytes())
+                + b"tb")
+    body = b"".join(matrix(v) if isinstance(v, np.ndarray) else b"G" + struct.pack(">d", v) for v in items)
+    return b"\x80\x02](" + body + b"e."
+
+
+def test_reference_problem_files_load(tmp_path):
+    """The reference's legacy (Python 2) problem files: data_deer_test_logw_M808xN10.pkl and data_forces_M64xN64.pkl,
+    rebuilt in Python 2's pickle layout from their entries stored in tests/golden."""
+    from conftest import load_golden
     from bioen_b200 import fileio as fio
-    root = "/root/reference/test/optimize/data"
-    if not os.path.isdir(root):
-        pytest.skip("reference tree not present")
-    P = fio.load_problem(os.path.join(root, "data_deer_test_logw_M808xN10.pkl"))
+    d = load_golden("data_deer_test_logw_M808xN10")
+    fn = tmp_path / "data_deer_test_logw_M808xN10.pkl"
+    fn.write_bytes(_py2_pickle([d[k] for k in fio.LOGW_KEYS[:-1]] + [float(d["theta"])]))
+    with pytest.raises(UnicodeDecodeError):
+        pickle.loads(fn.read_bytes())
+    P = fio.load_problem(str(fn))
     assert P["kind"] == "logw" and P["yTilde"].shape[0] == 808 and P["GInit"].shape == (P["yTilde"].shape[1], 1)
-    F = fio.load_problem(os.path.join(root, "data_forces_M64xN64.pkl"))
+    assert all(np.array_equal(P[k], d[k]) for k in fio.LOGW_KEYS[:-1]) and P["theta"] == d["theta"]
+    d = load_golden("data_forces_M64xN64")
+    fn = tmp_path / "data_forces_M64xN64.pkl"
+    fn.write_bytes(_py2_pickle([d[k] for k in fio.FORCES_KEYS[:-1]] + [float(d["theta"])]))
+    F = fio.load_problem(str(fn))
     assert F["kind"] == "forces" and F["yTilde"].shape == (64, 64) and F["forces_init"].shape == (64, 1)
+    assert all(np.array_equal(F[k], d[k]) for k in fio.FORCES_KEYS[:-1]) and F["theta"] == d["theta"]
 
 
 def test_open_matrix_npy(tmp_path):
