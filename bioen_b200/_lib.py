@@ -39,6 +39,10 @@ class visual_params(C.Structure):  # c_bioen_common.h:89-92
     _fields_ = [("debug", C.c_size_t), ("verbose", C.c_size_t)]
 
 
+class bioen_b200_batch(C.Structure):  # include/bioen_b200.h: per-problem inputs of a batch (NULL = shared vector)
+    _fields_ = [("K", C.c_int), ("thetas", _dp), ("YTilde", _dp), ("row_weights", _dp), ("w0", _dp)]
+
+
 # name -> (restype, argtypes); mirrors include/bioen_b200.h one to one (tests/test_abi.py checks the set)
 _vp = C.c_void_p
 SIGNATURES = {
@@ -93,6 +97,11 @@ SIGNATURES = {
                                         _ip, _ip, _dp]),
     "bioen_b200_time_scan_evals": (C.c_int, [_vp, C.c_int, C.c_int, _dp, _dp, C.c_int, C.c_int, C.POINTER(C.c_float),
                                              C.POINTER(C.c_float), C.POINTER(C.c_longlong)]),
+    "bioen_b200_batch_minimize": (C.c_int, [_vp, C.c_int, C.POINTER(bioen_b200_batch), _dp, _dp, lbfgs_config_params,
+                                            visual_params, _dp, _ip, _ip, _dp, _dp, _dp, _dp]),
+    "bioen_b200_batch_eval": (C.c_int, [_vp, C.c_int, C.POINTER(bioen_b200_batch), _dp, _dp, _dp, _dp, _dp, _dp]),
+    "bioen_b200_time_batch_evals": (C.c_int, [_vp, C.c_int, C.POINTER(bioen_b200_batch), _dp, C.c_int, C.c_int,
+                                              C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_longlong)]),
     "bioen_b200_dmma_peak": (C.c_int, [C.c_int, _dp]),
     "bioen_b200_read_stream_peak": (C.c_int, [_vp, C.c_int, _dp]),
     "bioen_b200_selftest_linesearch": (C.c_int, [lbfgs_config_params, C.c_double, C.c_double, C.c_double,

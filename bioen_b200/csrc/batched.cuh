@@ -1,7 +1,8 @@
-// batched.cuh -- the theta scan (L-curve): K log-weights problems that share yTilde, G and YTilde and differ in
-// theta (and in their iterates) are minimised TOGETHER, so that the two matrix passes of an evaluation become
-// skinny fp64 GEMMs  avg[M x K] = Y . W[N x K]  and  c[N x K] = Yt . R[M x K]  and yTilde is streamed from HBM
-// once per pass for all K problems instead of K times.  This is the only place the library uses tensor cores:
+// batched.cuh -- K <= 32 problems that share yTilde are minimised TOGETHER, so that the two matrix passes of an
+// evaluation become skinny fp64 GEMMs  avg[M x K] = Y . W[N x K]  and  c[N x K] = Yt . R[M x K]  and yTilde is
+// streamed from HBM once per pass for all K problems instead of K times.  The problems differ in theta and start
+// point (the theta scan, the L-curve) and, optionally, in YTilde, in observable weights c_i of chi^2 = 1/2 sum c r^2,
+// and (forces) in the reference weights w0: bootstrap and cross-validation replicates (DESIGN.md section 4g).  This is the only place the library uses tensor cores:
 // fp64 has no tcgen05 kind on Blackwell, so the GEMMs are warp-level DMMA (mma.sync.m8n8k4.f64) fed by TMA.
 //
 // What the reference does for the same job: a Python loop over theta calling find_optimum once per value
@@ -26,6 +27,8 @@
 #pragma once
 #include <algorithm>
 #include <cmath>
+#include <cstdio>
+#include <stdexcept>
 #include <vector>
 
 #include "context.cuh"
@@ -187,6 +190,7 @@ __global__ void __launch_bounds__(kGThreads, 1)
 // ------------------------------------------------------------------------------------------------
 // batched vector kernels: blockIdx.y = problem k.  Per-problem scalars live in scb[k][SC_COUNT] with the same
 // slot numbers as the single-problem path (vector_kernels.cuh); per-problem launch parameters travel by value.
+// Per-problem inputs (YTilde, observable weights, forces w0) are planes read at base + k * stride (BatchBufs).
 // ------------------------------------------------------------------------------------------------
 struct KVec {
     double stp[kBMaxK];
@@ -207,14 +211,19 @@ struct BatchBufs {
     double* partials;           // [KP][pstride]
     unsigned int* ticket;       // [KP]
     long long pstride;
-    const double* G;            // shared reference log-weights (logw) / reference weights w0 (forces)
-    const double* Yobs;
+    // Per-problem inputs.  Problem k reads its plane at base + k * stride; stride 0 = every problem reads the shared
+    // vector.  Cw == nullptr: no observable weights (chi^2 = 1/2 r.r, nothing is multiplied).
+    const double* G;            // reference log-weights (logw, always shared) / reference weights w0 (forces)
+    long long gld = 0;          // 0 or ldN (forces only)
+    const double* Yobs;         // YTilde
+    long long yld = 0;          // 0 or ldo
+    const double* Cw = nullptr; // [KP][ldo] observable weights c_k,i: chi^2 = 1/2 sum_i c r^2, gradients use c r
     // forces scan only: the variables are M-dimensional planes; these are the structure-axis work planes
     int nN = 0;                 // structures
     long long ldN = 0;
     double *Xn = nullptr, *LR = nullptr, *Tn = nullptr;   // [KP][ldN]: x_j = (Yt f)_j, log(w_j/w0_j), t_j
     double* Ff = nullptr;       // fragment-major forces (index = i)
-    double* avgk = nullptr;     // [KP][ldo]
+    double* avgk = nullptr;     // [KP][ldo] averages of the last objective half (both methods)
     long long ldo = 0;
 };
 
@@ -305,20 +314,26 @@ __global__ void __launch_bounds__(1024) kb_finalize(const BatchBufs b, const KVe
     const int k = blockIdx.x;
     if (!p.mask[k]) return;
     __shared__ double red[2 * 32];
+    const double* Y = b.Yobs + (size_t)k * b.yld;
+    const double* c = b.Cw ? b.Cw + (size_t)k * b.ldo : nullptr;
     double v[2] = {0.0, 0.0};
     for (int i = threadIdx.x; i < m; i += blockDim.x) {
         double s = 0.0;
         for (int q = 0; q < nseg; ++q) s += b.avgp[((size_t)q * b.KP + k) * ldo + i];
-        const double r = s - b.Yobs[i];
-        b.Rf[frag_index(i, k, b.NT)] = r;
-        v[0] = fma(r, r, v[0]);
-        v[1] = fma(r, s, v[1]);
+        b.avgk[(size_t)k * b.ldo + i] = s;
+        const double r = s - Y[i];
+        const double cr = c ? c[i] * r : r;
+        b.Rf[frag_index(i, k, b.NT)] = cr;
+        v[0] = fma(cr, r, v[0]);
+        v[1] = fma(cr, s, v[1]);
     }
     block_sum<2>(v, red);
     if (threadIdx.x == 0) {
         double* sc = b.scb + (size_t)k * SC_COUNT;
         const double chi2 = 0.5 * v[0];
-        const double prior = (sc[SC_TMP0] - (sc[SC_GMAX] + log(sc[SC_S])) + sc[SC_LOGS0]) * p.theta[k];
+        const double kl = sc[SC_TMP0] - (sc[SC_GMAX] + log(sc[SC_S])) + sc[SC_LOGS0];
+        const double prior = kl * p.theta[k];
+        sc[SC_KL] = kl;
         sc[SC_CHI2] = chi2;
         sc[SC_PRIOR] = prior;
         sc[SC_F] = prior + chi2;
@@ -471,9 +486,10 @@ __global__ void __launch_bounds__(kVecThreads) kbf_lse(const BatchBufs b, const 
     __shared__ double red[3 * 32];
     __shared__ bool is_last;
     const double* x = b.Xn + (size_t)k * b.ldN;
+    const double* w0p = b.G + (size_t)k * b.gld;
     double m = -DBL_MAX, s = 0.0, dummy = 0.0;
     for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < b.nN; j += gridDim.x * blockDim.x) {
-        const double v = x[j], pw = b.G[j];
+        const double v = x[j], pw = w0p[j];
         if (v > m) { s = s * exp(m - v) + pw; m = v; }
         else s += pw * exp(v - m);
     }
@@ -510,6 +526,7 @@ __global__ void __launch_bounds__(kVecThreads) kbf_weights(const BatchBufs b, co
     const double M = sc[SC_GMAX], inv = 1.0 / sc[SC_S], logS = log(sc[SC_S]);
     const double* x = b.Xn + (size_t)k * b.ldN;
     double* lrp = b.LR + (size_t)k * b.ldN;
+    const double* w0p = b.G + (size_t)k * b.gld;
     double v[1] = {0.0};
     const int nq = (b.nN + 3) >> 2;
     for (int q = blockIdx.x * blockDim.x + threadIdx.x; q < nq; q += gridDim.x * blockDim.x) {
@@ -519,7 +536,7 @@ __global__ void __launch_bounds__(kVecThreads) kbf_weights(const BatchBufs b, co
             const int j = 4 * q + e;
             double w = 0.0;
             if (j < b.nN) {
-                const double xj = x[j], w0 = b.G[j];
+                const double xj = x[j], w0 = w0p[j];
                 w = inv * (w0 * exp(xj - M));
                 const double lr = (w >= DBL_MIN && w0 >= DBL_MIN) ? (xj - M - logS) : 0.0;
                 lrp[j] = lr;
@@ -539,14 +556,17 @@ __global__ void __launch_bounds__(1024) kbf_finalize(const BatchBufs b, const KV
     const int k = blockIdx.x;
     if (!p.mask[k]) return;
     __shared__ double red[32];
+    const double* Y = b.Yobs + (size_t)k * b.yld;
+    const double* c = b.Cw ? b.Cw + (size_t)k * b.ldo : nullptr;
     double v[1] = {0.0};
     for (int i = threadIdx.x; i < m; i += blockDim.x) {
         double s = 0.0;
         for (int q = 0; q < nseg; ++q) s += b.avgp[((size_t)q * b.KP + k) * b.ldo + i];
         b.avgk[(size_t)k * b.ldo + i] = s;
-        const double r = s - b.Yobs[i];
-        b.Rf[frag_index(i, k, b.NT)] = r;
-        v[0] = fma(r, r, v[0]);
+        const double r = s - Y[i];
+        const double cr = c ? c[i] * r : r;
+        b.Rf[frag_index(i, k, b.NT)] = cr;      // t_j = sum_i y_ij c_i r_i: kbf_E and kbf_grad need nothing else
+        v[0] = fma(cr, r, v[0]);
     }
     block_sum<1>(v, red);
     if (threadIdx.x == 0) {
@@ -568,6 +588,7 @@ __global__ void __launch_bounds__(kVecThreads) kbf_E(const BatchBufs b, const KV
     const double* x = b.Xn + (size_t)k * b.ldN;
     const double* lrp = b.LR + (size_t)k * b.ldN;
     const double* t = b.Tn + (size_t)k * b.ldN;
+    const double* w0p = b.G + (size_t)k * b.gld;
     double v[1] = {0.0};
     const int nq = (b.nN + 3) >> 2;
     for (int q = blockIdx.x * blockDim.x + threadIdx.x; q < nq; q += gridDim.x * blockDim.x) {
@@ -577,7 +598,7 @@ __global__ void __launch_bounds__(kVecThreads) kbf_E(const BatchBufs b, const KV
             const int j = 4 * q + e;
             double E = 0.0;
             if (j < b.nN) {
-                const double w = inv * (b.G[j] * exp(x[j] - M));
+                const double w = inv * (w0p[j] * exp(x[j] - M));
                 E = ((1.0 + lrp[j]) * theta + t[j]) * w;
                 v[0] += E;
             }
@@ -660,6 +681,44 @@ __global__ void __launch_bounds__(256) kb_reduce_avg(const double* avgp, double*
     out[(size_t)k * ldo + i] = s;
 }
 
+// Per-problem inputs of a batch: host arrays of K rows, nullptr = every problem reads the context's shared vector.
+struct BatchPlanes {
+    const double* YTilde = nullptr;        // [K][M]  observed data (noise replicates)
+    const double* row_weights = nullptr;   // [K][M]  c_k,i >= 0 (observable resampling, held-out folds)
+    const double* w0 = nullptr;            // [K][N]  reference weights >= 0 (structure resampling), forces only
+};
+
+// Host-side checks of a batch's planes (before anything is allocated or enqueued)
+inline void check_planes(const BatchPlanes& in, int K, int M, int N, bool forces) {
+    auto bad = [](const char* what, int k, long long i) {
+        char buf[200];
+        snprintf(buf, sizeof buf, "bioen_b200: %s (problem %d, entry %lld)", what, k, i);
+        throw std::invalid_argument(buf);
+    };
+    if (in.w0 && !forces)
+        throw std::invalid_argument("bioen_b200: per-problem reference weights w0 need the forces method (log-weights "
+                                    "would need G_j = -inf for a structure of weight zero)");
+    for (int k = 0; k < K; ++k) {
+        if (in.YTilde)
+            for (int i = 0; i < M; ++i)
+                if (!std::isfinite(in.YTilde[(size_t)k * M + i])) bad("YTilde must be finite", k, i);
+        if (in.row_weights)
+            for (int i = 0; i < M; ++i) {
+                const double c = in.row_weights[(size_t)k * M + i];
+                if (!(std::isfinite(c) && c >= 0.0)) bad("row weights must be finite and >= 0", k, i);
+            }
+        if (in.w0) {
+            double sum = 0.0;
+            for (long long j = 0; j < N; ++j) {
+                const double w = in.w0[(size_t)k * N + j];
+                if (!(std::isfinite(w) && w >= 0.0)) bad("w0 must be finite and >= 0", k, j);
+                sum += w;
+            }
+            if (!(sum > 0.0)) bad("w0 must have a positive sum", k, -1);
+        }
+    }
+}
+
 struct ScanResult {
     int code = 0, iterations = 0, evaluations = 0;
     double fmin = 0.0;
@@ -675,6 +734,8 @@ class ThetaScan {
     int verbose = 0;
     long long ldn, ldN;
     DevBuf<double> planes, hist, Wf, Rf, avgp, scb, partials, nplanes, Ff, avgk, redbuf, lsebuf, lse_all;
+    DevBuf<double> yplanes, cplanes, wplanes;   // per-problem YTilde, row weights, w0 (allocated when given)
+    bool started = false;       // run() got past the parameter check: the X planes hold the problems' points
     int vblocksN = 1;
     bool reduce = false;        // N sharded over ranks
     DevBuf<unsigned int> ticket;
@@ -685,12 +746,13 @@ class ThetaScan {
     int vblocks;
     long long rounds = 0, gemm_launches = 0;
 
-    ThetaScan(Context& ctx, int k, const LbfgsParams& p, bool is_forces = false)
+    ThetaScan(Context& ctx, int k, const LbfgsParams& p, bool is_forces = false, const BatchPlanes& in = {})
         : C(ctx), forces(is_forces), K(k), KP((k + 7) & ~7), NT(((k + 7) & ~7) / 8),
           n(is_forces ? ctx.M : ctx.N), NN(ctx.N), MM(ctx.M), prm(p) {
         if (k < 1 || k > kBMaxK) throw std::invalid_argument("bioen_b200: theta scan batches 1..32 problems");
         if (!forces && !C.have_logw) throw std::logic_error("bioen_b200: log-weights data not set");
         if (forces && !C.have_forces) throw std::logic_error("bioen_b200: forces data not set");
+        check_planes(in, K, MM, NN, forces);
         if (!C.yt_valid) C.make_transposed();
         ldn = ((long long)n + 63) & ~63LL;
         ldN = ((long long)NN + 63) & ~63LL;
@@ -729,11 +791,21 @@ class ThetaScan {
         if (forces) {
             nplanes.alloc((size_t)3 * KP * ldN);
             Ff.alloc((size_t)mq * KP);
-            avgk.alloc((size_t)KP * gRow.ldo);
             B.nN = NN; B.ldN = ldN; B.Xn = nplanes.p; B.LR = B.Xn + (size_t)KP * ldN; B.Tn = B.LR + (size_t)KP * ldN;
-            B.Ff = Ff.p; B.avgk = avgk.p;
+            B.Ff = Ff.p;
         }
+        avgk.alloc((size_t)KP * gRow.ldo);
+        B.avgk = avgk.p;
         B.ldo = gRow.ldo;
+        // per-problem planes; the padding problems k >= K are masked and keep zeros
+        auto upload_planes = [&](DevBuf<double>& buf, const double* src, int len, long long ld) {
+            buf.alloc((size_t)KP * ld);
+            for (int q = 0; q < K; ++q) C.h2d(buf.p + (size_t)q * ld, src + (size_t)q * len, len);
+            return buf.p;
+        };
+        if (in.YTilde) { B.Yobs = upload_planes(yplanes, in.YTilde, MM, B.ldo); B.yld = B.ldo; }
+        if (in.row_weights) B.Cw = upload_planes(cplanes, in.row_weights, MM, B.ldo);
+        if (in.w0) { B.G = upload_planes(wplanes, in.w0, NN, ldN); B.gld = ldN; }
         reduce = C.nranks > 1;
         if (reduce) {
             redbuf.alloc((size_t)KP * gRow.ldo + 4 * KP);
@@ -832,8 +904,8 @@ class ThetaScan {
         return v;
     }
 
-    // one batched f+g evaluation of the masked problems; move: x = xp + stp*d first
-    void evaluate(const KVec& kv, bool move) {
+    // one batched f+g evaluation of the masked problems; move: x = xp + stp*d first; grad = false: objective half only
+    void evaluate(const KVec& kv, bool move, bool grad = true) {
         int nseg = 0;
         if (forces) {
             const dim3 gridN(vblocksN, KP);
@@ -848,6 +920,11 @@ class ThetaScan {
             {
                 const BatchBufs v = reduce_rows(kv, {SC_KL}, nseg);
                 kbf_finalize<<<KP, 1024, 0, C.stream>>>(v, kv, MM, nseg);
+            }
+            if (!grad) {
+                CUDA_CHECK(cudaGetLastError());
+                C.kernels_launched += 4;
+                return;
             }
             g.B = Rf.p; g.out = B.Tn;
             launch_gemm(tmapCol, g);                                   // t_j = sum_i r_i y_ij
@@ -870,6 +947,11 @@ class ThetaScan {
             const BatchBufs v = reduce_rows(kv, {SC_TMP0, SC_GBAR, SC_CAPGBAR, SC_XNORM2}, nseg);
             kb_finalize<<<KP, 1024, 0, C.stream>>>(v, kv, C.M, nseg, gRow.ldo);
         }
+        if (!grad) {
+            CUDA_CHECK(cudaGetLastError());
+            C.kernels_launched += 3;
+            return;
+        }
         launch_gemm(tmapCol, gCol);
         kb_grad<<<gridv, kVecThreads, 0, C.stream>>>(B, kv);
         if (reduce) allreduce_tab(tab_uniform({SC_DG, SC_GNORM2}, kv), redbuf.p);
@@ -881,6 +963,27 @@ class ThetaScan {
         C.spin_sync();
     }
     const double* hs(int k) const { return h_scb + (size_t)k * SC_COUNT; }
+
+    // One evaluation of all K problems at the points in the X planes (x_host: [K][n] uploaded first when given),
+    // copied out per problem: f[K], grad[K][n] (its presence selects the gradient half), avg[K][M] = yTilde . w,
+    // chi2[K] (weighted by the row weights), kl[K] (the prior without the theta factor).  Any output may be nullptr.
+    void evaluate_all(const double* thetas, const double* x_host, double* f, double* grad, double* avg, double* chi2,
+                      double* kl) {
+        if (x_host)
+            for (int q = 0; q < K; ++q) C.h2d(B.X + (size_t)q * ldn, x_host + (size_t)q * n, n);
+        KVec kv{};
+        for (int q = 0; q < KP; ++q) { kv.mask[q] = q < K; kv.theta[q] = q < K ? thetas[q] : 0.0; }
+        evaluate(kv, false, grad != nullptr);
+        fetch();
+        for (int q = 0; q < K; ++q) {
+            if (f) f[q] = hs(q)[SC_F];
+            if (chi2) chi2[q] = hs(q)[SC_CHI2];
+            if (kl) kl[q] = hs(q)[SC_KL];
+            if (grad) C.d2h(grad + (size_t)q * n, B.Gr + (size_t)q * ldn, n);
+            if (avg) C.d2h(avg + (size_t)q * MM, avgk.p + (size_t)q * B.ldo, MM);
+        }
+        C.sync();
+    }
 
     // bench.py: time `steps` batched evaluations of all K problems at fresh points (x = xp + (k+1)*d with a tiny d)
     void time_evals(const double* thetas, const double* x0_host, int warmup, int steps, float* ms, float* gemm_ms,
@@ -924,6 +1027,7 @@ class ThetaScan {
             for (auto& r : res) r.code = perr;
             return res;
         }
+        started = true;
         const int m = prm.m;
         struct P {
             int state = 0;   // 1 active, 0 done

@@ -601,48 +601,125 @@ int bioen_b200_opt_gsl(bioen_b200_ctx* ctx, int method, const double* x0_host, d
     return ret;
 }
 
+// the lockstep L-BFGS of K problems (theta scan and batched replicates); avg / chi2 / kl: one objective half at the
+// returned points, NaN for a batch whose L-BFGS parameters were refused
+static void scan_minimize(bioen_b200_ctx* ctx, int method, int K, const double* thetas, const BatchPlanes& in,
+                          const double* x0_host, double* x_host, lbfgs_config_params config, visual_params visual,
+                          double* fmin, int* codes, int* info, double* stats, double* avg, double* chi2, double* kl,
+                          const char* what) {
+    ctx->pending_gen = -1;
+    Context& C = ctx->C;
+    CUDA_CHECK(cudaSetDevice(C.device));
+    C.require_row_major("the batched theta scan");
+    const auto t0 = std::chrono::steady_clock::now();
+    ThetaScan scan(C, K, to_params(config), method == BIOEN_B200_FORCES, in);
+    scan.verbose = (int)visual.verbose;
+    const std::vector<ScanResult> res = scan.run(thetas, x0_host, x_host);
+    if (avg || chi2 || kl) {
+        if (scan.started) {
+            scan.evaluate_all(thetas, nullptr, nullptr, nullptr, avg, chi2, kl);
+        } else {
+            if (avg) std::fill(avg, avg + (size_t)K * C.M, kNaN);
+            if (chi2) std::fill(chi2, chi2 + K, kNaN);
+            if (kl) std::fill(kl, kl + K, kNaN);
+        }
+    }
+    const double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+    for (int q = 0; q < K; ++q) {
+        if (fmin) fmin[q] = res[q].fmin;
+        if (codes) codes[q] = res[q].code;
+        if (info) { info[2 * q] = res[q].iterations; info[2 * q + 1] = res[q].evaluations; }
+    }
+    if (stats) {
+        stats[0] = (double)scan.rounds;
+        stats[1] = (double)scan.gemm_launches;
+        stats[2] = secs;
+        stats[3] = 0.0;
+    }
+    if (visual.verbose) {
+        printf("%s: %d problems, %lld lockstep rounds, %.6f s\n", what, K, scan.rounds, secs);
+        for (int q = 0; q < K; ++q)
+            printf("\ttheta = %-12g %s  f = %.6lf  iterations %d\n", thetas[q], lbfgs_strerror(res[q].code),
+                   res[q].fmin, res[q].iterations);
+    }
+}
+
+// the per-problem inputs of a bioen_b200_batch, after the checks that do not depend on the data
+static BatchPlanes batch_planes(const bioen_b200_ctx* ctx, const bioen_b200_batch* batch) {
+    if (!batch || !batch->thetas) throw std::invalid_argument("bioen_b200: batch and batch->thetas are required");
+    if (ctx->C.nranks > 1)
+        throw std::invalid_argument("bioen_b200: batched replicates are not supported on sharded problems");
+    BatchPlanes in;
+    in.YTilde = batch->YTilde;
+    in.row_weights = batch->row_weights;
+    in.w0 = batch->w0;
+    return in;
+}
+
 int bioen_b200_theta_scan(bioen_b200_ctx* ctx, int method, int K, const double* thetas, const double* x0_host,
                           double* x_host,
                           lbfgs_config_params config, visual_params visual, double* fmin, int* codes, int* info,
                           double* stats) {
     return guarded("bioen_b200_theta_scan", [&] {
+        scan_minimize(ctx, method, K, thetas, BatchPlanes(), x0_host, x_host, config, visual, fmin, codes, info, stats,
+                      nullptr, nullptr, nullptr, "theta scan");
+    });
+}
+
+int bioen_b200_batch_minimize(bioen_b200_ctx* ctx, int method, const bioen_b200_batch* batch, const double* x0_host,
+                              double* x_host, lbfgs_config_params config, visual_params visual, double* fmin,
+                              int* codes, int* info, double* stats, double* avg, double* chi2, double* kl) {
+    return guarded("bioen_b200_batch_minimize", [&] {
+        const BatchPlanes in = batch_planes(ctx, batch);
+        scan_minimize(ctx, method, batch->K, batch->thetas, in, x0_host, x_host, config, visual, fmin, codes, info,
+                      stats, avg, chi2, kl, "batch minimisation");
+    });
+}
+
+// a batch that is only evaluated, never minimised: no L-BFGS history planes (m = 0 allocates none)
+static LbfgsParams evaluation_only() {
+    LbfgsParams p;
+    p.m = 0;
+    return p;
+}
+
+int bioen_b200_batch_eval(bioen_b200_ctx* ctx, int method, const bioen_b200_batch* batch, const double* x_host,
+                          double* f, double* grad_host, double* avg, double* chi2, double* kl) {
+    return guarded("bioen_b200_batch_eval", [&] {
+        const BatchPlanes in = batch_planes(ctx, batch);
+        if (!x_host) throw std::invalid_argument("bioen_b200: x is required");
         ctx->pending_gen = -1;
         Context& C = ctx->C;
         CUDA_CHECK(cudaSetDevice(C.device));
         C.require_row_major("the batched theta scan");
-        const auto t0 = std::chrono::steady_clock::now();
-        ThetaScan scan(C, K, to_params(config), method == BIOEN_B200_FORCES);
-        scan.verbose = (int)visual.verbose;
-        const std::vector<ScanResult> res = scan.run(thetas, x0_host, x_host);
-        const double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-        for (int q = 0; q < K; ++q) {
-            if (fmin) fmin[q] = res[q].fmin;
-            if (codes) codes[q] = res[q].code;
-            if (info) { info[2 * q] = res[q].iterations; info[2 * q + 1] = res[q].evaluations; }
-        }
-        if (stats) {
-            stats[0] = (double)scan.rounds;
-            stats[1] = (double)scan.gemm_launches;
-            stats[2] = secs;
-            stats[3] = 0.0;
-        }
-        if (visual.verbose) {
-            printf("theta scan: %d problems, %lld lockstep rounds, %.6f s\n", K, scan.rounds, secs);
-            for (int q = 0; q < K; ++q)
-                printf("\ttheta = %-12g %s  f = %.6lf  iterations %d\n", thetas[q], lbfgs_strerror(res[q].code),
-                       res[q].fmin, res[q].iterations);
-        }
+        ThetaScan scan(C, batch->K, evaluation_only(), method == BIOEN_B200_FORCES, in);
+        scan.evaluate_all(batch->thetas, x_host, f, grad_host, avg, chi2, kl);
+    });
+}
+
+// `steps` timed batched f+g evaluations (bioen_b200_time_scan_evals: no planes, sharded contexts allowed)
+static void time_batched_evals(bioen_b200_ctx* ctx, int method, int K, const double* thetas, const BatchPlanes& in,
+                               const double* x0_host, int warmup, int steps, float* ms, float* gemm_ms, long long* launches) {
+    ctx->pending_gen = -1;
+    Context& C = ctx->C;
+    CUDA_CHECK(cudaSetDevice(C.device));
+    C.require_row_major("the batched theta scan");
+    ThetaScan scan(C, K, evaluation_only(), method == BIOEN_B200_FORCES, in);
+    scan.time_evals(thetas, x0_host, warmup, steps, ms, gemm_ms, launches);
+}
+
+int bioen_b200_time_batch_evals(bioen_b200_ctx* ctx, int method, const bioen_b200_batch* batch, const double* x0_host,
+                                int warmup, int steps, float* ms, float* gemm_ms, long long* launches) {
+    return guarded("bioen_b200_time_batch_evals", [&] {
+        const BatchPlanes in = batch_planes(ctx, batch);
+        time_batched_evals(ctx, method, batch->K, batch->thetas, in, x0_host, warmup, steps, ms, gemm_ms, launches);
     });
 }
 
 int bioen_b200_time_scan_evals(bioen_b200_ctx* ctx, int method, int K, const double* thetas, const double* x0_host,
                                int warmup, int steps, float* ms, float* gemm_ms, long long* launches) {
     return guarded("bioen_b200_time_scan_evals", [&] {
-        ctx->pending_gen = -1;
-        Context& C = ctx->C;
-        CUDA_CHECK(cudaSetDevice(C.device));
-        ThetaScan scan(C, K, LbfgsParams(), method == BIOEN_B200_FORCES);
-        scan.time_evals(thetas, x0_host, warmup, steps, ms, gemm_ms, launches);
+        time_batched_evals(ctx, method, K, thetas, BatchPlanes(), x0_host, warmup, steps, ms, gemm_ms, launches);
     });
 }
 

@@ -82,6 +82,8 @@ class Problem:
             _lib.clear_pending()
             raise RuntimeError("bioen_b200_create failed: " + msg)
         self.method = None
+        self.YTilde = None      # host copies of the data set_logw / set_forces put on the device (replicates.py)
+        self.w0 = None
         self.nranks = 1
         if structure_major_only:
             _lib.check(self._lib.bioen_b200_set_option(self._ctx, 11, 1), "set_option")
@@ -155,6 +157,7 @@ class Problem:
             raise ValueError("G must have n and YTilde m entries")
         _lib.check(self._lib.bioen_b200_set_logw(self._ctx, _lib.ptr(G), _lib.ptr(Y), float(theta)), "set_logw")
         self.method = LOGW
+        self.YTilde, self.w0 = Y.copy(), None
 
     def set_forces(self, w0, YTilde, theta):
         w0, Y = _lib.vec(w0), _lib.vec(YTilde)
@@ -162,6 +165,7 @@ class Problem:
             raise ValueError("w0 must have n and YTilde m entries")
         _lib.check(self._lib.bioen_b200_set_forces(self._ctx, _lib.ptr(w0), _lib.ptr(Y), float(theta)), "set_forces")
         self.method = FORCES
+        self.YTilde, self.w0 = Y.copy(), w0.copy()
 
     def set_option(self, option, value):
         """Tuning switches of include/bioen_b200.h (1 = fused two-pass forces kernels, default on)."""
@@ -369,6 +373,73 @@ class Problem:
         return X, fmin, np.array(codes[:]), dict(iterations=np.array(info[0::2]), evaluations=np.array(info[1::2]),
                                                  rounds=int(stats[0]), gemm_launches=int(stats[1]),
                                                  seconds=float(stats[2]))
+
+    # ---- batched replicates: K <= 32 problems with per-problem YTilde, observable weights, w0 ----------------------
+    def _batch(self, method, thetas, X, YTilde, row_weights, w0):
+        """The bioen_b200_batch of a call and the arrays it points to: thetas (K,), X (K, n), and (K, M) / (K, N)
+        planes or None.  A scalar theta and single vectors are broadcast; K comes from whichever argument has rows."""
+        n = self._dim(method)
+        args = [("thetas", np.asarray(thetas, dtype=np.float64), 0), ("x", np.asarray(X, dtype=np.float64), n),
+                ("YTilde", YTilde, self.m), ("row_weights", row_weights, self.m), ("w0", w0, self.n)]
+        args = [(name, None if a is None else np.asarray(a, dtype=np.float64), width) for name, a, width in args]
+        Ks = {a.shape[0] for name, a, width in args if a is not None and a.ndim == (1 if width == 0 else 2)} - {1}
+        if len(Ks) > 1:
+            raise ValueError("per-problem arguments disagree on the number of problems: %s" % sorted(Ks))
+        K = Ks.pop() if Ks else 1
+        if not 1 <= K <= 32:
+            raise ValueError("a batch holds 1..32 problems, got %d" % K)
+        out = {}
+        for name, a, width in args:
+            if a is None:
+                out[name] = None
+                continue
+            want = (K,) if width == 0 else (K, width)
+            if a.shape not in (want, want[1:], (1,) + want[1:]):
+                raise ValueError("%s must have shape %s or %s, got %s" % (name, want[1:] or "()", want, a.shape))
+            out[name] = np.ascontiguousarray(np.broadcast_to(a, want))
+        b = _lib.bioen_b200_batch(K, _lib.ptr(out["thetas"]), *(None if out[k] is None else _lib.ptr(out[k])
+                                                                   for k in ("YTilde", "row_weights", "w0")))
+        return K, n, b, out
+
+    def batch_minimize(self, thetas, x0=None, YTilde=None, row_weights=None, w0=None, method=None, verbose=0, **cfg):
+        """Minimise up to 32 problems that share yTilde TOGETHER (the theta scan's lockstep L-BFGS and batched fp64
+        tensor-core evaluations).  Per problem k, optionally: YTilde[k] (M,) in place of the shared YTilde,
+        observable weights row_weights[k] (M,) >= 0 with chi^2 = 1/2 sum_i c_i r_i^2, and (forces only) reference
+        weights w0[k] (N,) >= 0.  Scalars / single vectors are broadcast.  Returns (X (K, n), fmin (K,), codes (K,),
+        info) like theta_scan; info also holds averages (K, M) = yTilde . w, chi2 (K,) and kl (K,) at the returned
+        points (NaN when the L-BFGS parameters are refused)."""
+        method = self._method(method)
+        K, n, b, a = self._batch(method, thetas, np.zeros(self._dim(method)) if x0 is None else x0, YTilde,
+                                 row_weights, w0)
+        p = dict(LBFGS_DEFAULTS)
+        p.update(cfg)
+        c = _lib.lbfgs_config_params(**{k: p[k] for k, _ in _lib.lbfgs_config_params._fields_})
+        v = _lib.visual_params(0, int(bool(verbose)))
+        X = np.empty((K, n), dtype=np.float64)
+        fmin, chi2, kl = np.empty(K), np.empty(K), np.empty(K)
+        avg = np.empty((K, self.m), dtype=np.float64)
+        codes = (C.c_int * K)()
+        info = (C.c_int * (2 * K))()
+        stats = np.zeros(4, dtype=np.float64)
+        _lib.check(self._lib.bioen_b200_batch_minimize(self._ctx, method, C.byref(b), _lib.ptr(a["x"]), _lib.ptr(X), c, v,
+                                                       _lib.ptr(fmin), codes, info, _lib.ptr(stats), _lib.ptr(avg),
+                                                       _lib.ptr(chi2), _lib.ptr(kl)), "batch_minimize")
+        return X, fmin, np.array(codes[:]), dict(iterations=np.array(info[0::2]), evaluations=np.array(info[1::2]),
+                                                 rounds=int(stats[0]), gemm_launches=int(stats[1]),
+                                                 seconds=float(stats[2]), averages=avg, chi2=chi2, kl=kl)
+
+    def batch_evaluate(self, X, thetas, YTilde=None, row_weights=None, w0=None, gradient=True, method=None):
+        """One batched evaluation of up to 32 problems (arguments as batch_minimize) at the points X (K, n).
+        Returns (f (K,), grad (K, n) or None, dict(averages (K, M), chi2 (K,), kl (K,)))."""
+        method = self._method(method)
+        K, n, b, a = self._batch(method, thetas, X, YTilde, row_weights, w0)
+        f, chi2, kl = np.empty(K), np.empty(K), np.empty(K)
+        g = np.empty((K, n), dtype=np.float64) if gradient else None
+        avg = np.empty((K, self.m), dtype=np.float64)
+        _lib.check(self._lib.bioen_b200_batch_eval(self._ctx, method, C.byref(b), _lib.ptr(a["x"]), _lib.ptr(f),
+                                                   _lib.ptr(g) if gradient else None, _lib.ptr(avg), _lib.ptr(chi2),
+                                                   _lib.ptr(kl)), "batch_eval")
+        return f, g, dict(averages=avg, chi2=chi2, kl=kl)
 
     # ---- device-pointer entry points (bench.py) -----------------------------------------------------------
     def time_evals(self, x_dev_ptr, grad_dev_ptr, warmup, steps, method=None):

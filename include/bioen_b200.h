@@ -263,11 +263,42 @@ int bioen_b200_theta_scan(bioen_b200_ctx *ctx, int method, int K, const double *
                           double *x_host, lbfgs_config_params config, visual_params visual, double *fmin, int *codes, int *info,
                           double *stats);
 
+/* batched replicates: K <= 32 problems of one method that share the resident yTilde and differ in theta, start
+ * point and, per problem, in any of the arrays below (row-major host arrays; NULL = every problem uses the vector the
+ * context holds).  The bootstrap (resampled observables, structures or experimental noise) and cross-validation over
+ * observables are batches of this kind; they run on the theta scan's lockstep engine.
+ *   YTilde      [K][M]  observed data of each problem (noise replicates); finite
+ *   row_weights [K][M]  observable weights c_i >= 0, finite: chi^2 = 1/2 sum_i c_i r_i^2 (resampled or held-out rows)
+ *   w0          [K][N]  reference weights >= 0, finite, positive sum (resampled structures); BIOEN_B200_FORCES only:
+ *                       the log-weights parametrisation cannot represent a structure of weight zero
+ * Invalid arrays, and sharded contexts, are refused before anything runs. */
+typedef struct bioen_b200_batch {
+    int K;
+    const double *thetas;        /* [K] */
+    const double *YTilde;
+    const double *row_weights;
+    const double *w0;
+} bioen_b200_batch;
+
+/* lockstep L-BFGS of the batch: x0_host / x_host, fmin, codes, info, stats as for bioen_b200_theta_scan (which is this
+ * call with every array NULL).  Then one objective evaluation at the returned points gives, per problem,
+ * avg[K][M] = yTilde . w(x_k), chi2[K] (with the row weights) and kl[K] (the relative entropy, without theta); each
+ * may be NULL.  All three are NaN when the L-BFGS parameters are refused. */
+int bioen_b200_batch_minimize(bioen_b200_ctx *ctx, int method, const bioen_b200_batch *batch, const double *x0_host,
+                              double *x_host, lbfgs_config_params config, visual_params visual, double *fmin,
+                              int *codes, int *info, double *stats, double *avg, double *chi2, double *kl);
+/* one batched evaluation at x_host[K][n]: f[K], grad_host[K][n] (NULL: objective half only), avg[K][M], chi2[K],
+ * kl[K] (each may be NULL) */
+int bioen_b200_batch_eval(bioen_b200_ctx *ctx, int method, const bioen_b200_batch *batch, const double *x_host,
+                          double *f, double *grad_host, double *avg, double *chi2, double *kl);
+
 /* bench.py: time `steps` batched f+g evaluations of K problems (CUDA events); *gemm_ms = mean duration of one
- * skinny-GEMM launch.  bioen_b200_dmma_peak: fp64 tensor-core peak of the device, measured with a
+ * skinny-GEMM launch.  bioen_b200_time_batch_evals: the same for a batch with per-problem arrays.  bioen_b200_dmma_peak: fp64 tensor-core peak of the device, measured with a
  * register-resident mma.sync.m8n8k4.f64 loop (the roofline denominator of the GEMMs). */
 int bioen_b200_time_scan_evals(bioen_b200_ctx *ctx, int method, int K, const double *thetas, const double *x0_host,
                                int warmup, int steps, float *ms, float *gemm_ms, long long *launches);
+int bioen_b200_time_batch_evals(bioen_b200_ctx *ctx, int method, const bioen_b200_batch *batch, const double *x0_host,
+                                int warmup, int steps, float *ms, float *gemm_ms, long long *launches);
 int bioen_b200_dmma_peak(int device, double *tflops);
 /* mean GB/s of `reps` launches of a plain read-only stream (16-byte loads, nothing written) over the resident
  * yTilde: what a read-only pass can reach on this device, next to the copy figure of MEASURED_PEAKS.json */
