@@ -19,8 +19,10 @@
 //   forces        A: f = xp + stp d;  x_j = sum_i f_i y_ij;  m_c, u_j = w0_j e^{x_j - m_c}, S_c, K_c, A_c,i | barrier |
 //                 B: m, S, KL, avg, r, chi^2, f;  w_j, lr_j;  t_j = sum_i r_i y_ij;  E_j;
 //                    g_c,i = sum_j (y_ij - avg_i) E_j                                                      -> ticket
-//                 (KL = sum_j w_j lr_j is formed from K_c = sum_j (x_j - m_c) u_j, i.e. without the reference's
-//                  guard lr_j = 0 for w_j < DBL_MIN: those terms are < 1e-305, c_bioen_kernels_forces.c:246-274)
+//                 (KL = sum_j w_j lr_j is formed from K_c = sum_j (x_j - m_c) u_j over the structures with
+//                  w0_j >= DBL_MIN and U_c = sum u_j over the others, i.e. with the reference's guard lr_j = 0 for
+//                  w0_j < DBL_MIN but without its guard lr_j = 0 for w_j < DBL_MIN: those terms are < 1e-305,
+//                  c_bioen_kernels_forces.c:246-274)
 //
 // Reference lines this restates: c_bioen_kernels_logw.c:29-217, 525-561; c_bioen_kernels_forces.c:93-340.
 // All reductions are fixed-order (geometry-dependent only): results are bit-reproducible run to run, and the
@@ -426,16 +428,19 @@ __global__ void __launch_bounds__(kSliceThreads, 1) slice_eval_kernel(const Slic
         double m = -DBL_MAX;
         for (int jj = tid; jj < nv; jj += kSliceThreads) m = fmax(m, vx[jj]);
         const double mloc = slice_block_max(m, red);
-        double v[2] = {0.0, 0.0};
+        // S_c = sum u_j, K_c = sum (x_j - m_c) u_j over the structures with w0_j >= DBL_MIN (the reference's guard
+        // lr_j = 0 otherwise), U_c = sum u_j over the others: their weight counts in S, their log-ratio does not
+        double v[3] = {0.0, 0.0, 0.0};
         for (int jj = tid; jj < nv; jj += kSliceThreads) {
-            const double xr = vx[jj] - mloc;
-            const double u = vg[jj] * exp(xr);
+            const double xr = vx[jj] - mloc, w0 = vg[jj];
+            const double u = w0 * exp(xr);
             ve[jj] = u;
             v[0] += u;
-            v[1] = fma(xr, u, v[1]);
+            if (w0 >= DBL_MIN) v[1] = fma(xr, u, v[1]);
+            else v[2] += u;
         }
-        block_sum<2>(v, red);
-        if (tid == 0) { mytab[0] = mloc; mytab[1] = v[0]; mytab[2] = v[1]; }
+        block_sum<3>(v, red);
+        if (tid == 0) { mytab[0] = mloc; mytab[1] = v[0]; mytab[2] = v[1]; mytab[3] = v[2]; }
         __syncthreads();   // ve complete
         slice_row_reduce<false>(sl, ncs, M, nv, ve, nullptr, a.l_log2,
                                 [&](int i, double sum) { mytab[kSliceHdr + i] = sum; });
@@ -443,24 +448,26 @@ __global__ void __launch_bounds__(kSliceThreads, 1) slice_eval_kernel(const Slic
         const bool ok = slice_grid_barrier(a.bar);
         slice_mark(a, mk);
         // ---- B: global (max, S), KL, avg, r, chi^2, objective -- in every CTA, CTA order
-        double mc = -DBL_MAX, Sc = 0.0, Kc = 0.0;
+        double mc = -DBL_MAX, Sc = 0.0, Kc = 0.0, Uc = 0.0;
         if (tid < G) {
             const double* rec = a.tab + (size_t)tid * ms;
-            mc = __ldcg(rec); Sc = __ldcg(rec + 1); Kc = __ldcg(rec + 2);
+            mc = __ldcg(rec); Sc = __ldcg(rec + 1); Kc = __ldcg(rec + 2); Uc = __ldcg(rec + 3);
         }
         const double mx = slice_block_max(mc, red);
-        double t[2] = {0.0, 0.0};
+        double t[3] = {0.0, 0.0, 0.0};
         if (tid < G) {
             const double s = exp(mc - mx);
             s_scale[tid] = s;
             t[0] = Sc * s;
-            t[1] = s * fma(mc - mx, Sc, Kc);
+            t[1] = s * fma(mc - mx, Sc - Uc, Kc);
+            t[2] = Uc * s;
         }
-        block_sum<2>(t, red);
+        block_sum<3>(t, red);
         if (tid == 0) {
             const double inv = 1.0 / t[0], logS = log(t[0]);
             s_val[0] = t[0]; s_val[1] = inv; s_val[2] = logS;
-            s_val[3] = t[1] * inv - logS;   // KL
+            // KL = sum_{w0_j >= DBL_MIN} w_j (x_j - m - log S) = K / S - log S (1 - U / S); U = 0 leaves the bits of K / S - log S
+            s_val[3] = t[1] * inv - logS + logS * (t[2] * inv);
         }
         __syncthreads();
         const double S = s_val[0], inv = s_val[1], logS = s_val[2];
