@@ -1019,6 +1019,87 @@ class ThetaScan {
         cudaEventDestroy(e1);
     }
 
+    // The L-BFGS update of the problems in upd.mask (lbfgs.c:543-598): problem q's new pair goes to ring slot
+    // upd.slot[q], then the two-loop recursion over bound[q] pairs as 2*bound+1 fused steps.  The problems of one
+    // launch may sit at different (slot, bound); the others' planes are not touched.  run() and
+    // bioen_b200_selftest_lbfgs_update call this.
+    void update_directions(const KSlots& upd, const std::vector<int>& bound) {
+        const int m = prm.m;
+        const dim3 gridv(vblocks, KP);
+        int maxbound = 0;
+        for (int q = 0; q < K; ++q)
+            if (upd.mask[q]) maxbound = std::max(maxbound, bound[q]);
+        kb_pair<<<gridv, kVecThreads, 0, C.stream>>>(B, upd);
+        if (reduce && !forces) {
+            // y.s and y.y are sums over the structure axis; the ring copy ys[slot] follows the reduced value
+            KSlotTab t{};
+            t.n = 3;
+            t.row[0] = 0; t.row[1] = 1; t.row[2] = 0;
+            for (int q = 0; q < kBMaxK; ++q) {
+                const bool on = q < K && upd.mask[q];
+                t.slot[0][q] = on ? (signed char)SC_YS : (signed char)-1;
+                t.slot[1][q] = on ? (signed char)SC_YY : (signed char)-1;
+                t.slot[2][q] = on ? (signed char)(SC_YS0 + upd.slot[q]) : (signed char)-1;
+            }
+            KSlotTab pk = t;
+            pk.n = 2;
+            kb_pack<<<2, kBMaxK, 0, C.stream>>>(scb.p, redbuf.p, pk, KP);
+            C.comm->allreduce_sum(redbuf.p, (size_t)2 * KP, C.stream);
+            kb_unpack<<<3, kBMaxK, 0, C.stream>>>(scb.p, redbuf.p, t, KP);
+        }
+        // two-loop recursion (lbfgs.c:572-598) as 2*bound+1 fused steps per problem
+        for (int t = 0; t <= 2 * maxbound; ++t) {
+            KStep st{};
+            for (int q = 0; q < K; ++q) {
+                if (!upd.mask[q]) continue;
+                const int bnd = bound[q], end = (upd.slot[q] + 1) % m;   // the ring end after this update
+                if (t > 2 * bnd) continue;
+                auto js = [&](int i) { return ((end - 1 - i) % m + m) % m; };   // newest ... oldest
+                st.op[q] = 1;
+                st.c2_num[q] = -1;
+                if (t == 0) {
+                    st.init[q] = 1;
+                    st.v_kind[q] = 1; st.v_slot[q] = (signed char)js(0); st.out[q] = (signed char)(SC_ALPHA0 + js(0));
+                } else if (t <= bnd) {
+                    const int i = t - 1;
+                    st.u_kind[q] = 2; st.u_slot[q] = (signed char)js(i);
+                    st.c_num[q] = (signed char)(SC_ALPHA0 + js(i)); st.c_den[q] = (signed char)(SC_YS0 + js(i));
+                    st.csign[q] = -1;
+                    if (i + 1 < bnd) {
+                        st.v_kind[q] = 1; st.v_slot[q] = (signed char)js(i + 1);
+                        st.out[q] = (signed char)(SC_ALPHA0 + js(i + 1));
+                    } else {
+                        st.scale[q] = 1;
+                        st.v_kind[q] = 2; st.v_slot[q] = (signed char)js(i); st.out[q] = (signed char)SC_BETA;
+                    }
+                } else {
+                    const int i = bnd - (t - bnd);          // bnd-1 ... 0
+                    const int which = (t - bnd - 1) & 1;     // beta slots alternate
+                    st.u_kind[q] = 1; st.u_slot[q] = (signed char)js(i);
+                    st.c_num[q] = (signed char)(SC_ALPHA0 + js(i)); st.c_den[q] = (signed char)(SC_YS0 + js(i));
+                    st.csign[q] = 1;
+                    st.c2_num[q] = (signed char)(which ? SC_BETA2 : SC_BETA);
+                    if (i > 0) {
+                        st.v_kind[q] = 2; st.v_slot[q] = (signed char)js(i - 1);
+                        st.out[q] = (signed char)(which ? SC_BETA : SC_BETA2);
+                    } else {
+                        st.v_kind[q] = 3; st.out[q] = (signed char)SC_DGINIT;
+                    }
+                }
+            }
+            kb_twoloop<<<gridv, kVecThreads, 0, C.stream>>>(B, st);
+            if (reduce && !forces) {
+                KSlotTab t{};
+                t.n = 1;
+                t.row[0] = 0;
+                for (int q = 0; q < kBMaxK; ++q)
+                    t.slot[0][q] = (q < K && st.op[q] && st.v_kind[q]) ? st.out[q] : (signed char)-1;
+                allreduce_tab(t, redbuf.p);
+            }
+        }
+        CUDA_CHECK(cudaGetLastError());
+    }
+
     // x0 / x_out: [K][n] host arrays.  Returns per-problem results (liblbfgs codes).
     std::vector<ScanResult> run(const double* thetas, const double* x0_host, double* x_host) {
         std::vector<ScanResult> res(K);
@@ -1077,7 +1158,6 @@ class ThetaScan {
             KSlots upd{};
             KVec revert{};
             bool any_upd = false, any_rev = false;
-            int maxbound = 0;
             std::vector<int> bound(K, 0);
             for (int q = 0; q < K; ++q) {
                 P& p = ps[q];
@@ -1124,7 +1204,6 @@ class ThetaScan {
                 upd.slot[q] = p.end;
                 any_upd = true;
                 bound[q] = (m <= p.k) ? m : p.k;
-                maxbound = std::max(maxbound, bound[q]);
                 ++p.k;
                 p.end = (p.end + 1) % m;
                 p.step = 1.0;
@@ -1135,77 +1214,7 @@ class ThetaScan {
                 kb_scale_copy<<<gridv, kVecThreads, 0, C.stream>>>(n, ldn, B.XP, B.X, 1.0, revert);
                 kb_scale_copy<<<gridv, kVecThreads, 0, C.stream>>>(n, ldn, B.GP, B.Gr, 1.0, revert);
             }
-            if (any_upd) {
-                kb_pair<<<gridv, kVecThreads, 0, C.stream>>>(B, upd);
-                if (reduce && !forces) {
-                    // y.s and y.y are sums over the structure axis; the ring copy ys[slot] follows the reduced value
-                    KSlotTab t{};
-                    t.n = 3;
-                    t.row[0] = 0; t.row[1] = 1; t.row[2] = 0;
-                    for (int q = 0; q < kBMaxK; ++q) {
-                        const bool on = q < K && upd.mask[q];
-                        t.slot[0][q] = on ? (signed char)SC_YS : (signed char)-1;
-                        t.slot[1][q] = on ? (signed char)SC_YY : (signed char)-1;
-                        t.slot[2][q] = on ? (signed char)(SC_YS0 + upd.slot[q]) : (signed char)-1;
-                    }
-                    KSlotTab pk = t;
-                    pk.n = 2;
-                    kb_pack<<<2, kBMaxK, 0, C.stream>>>(scb.p, redbuf.p, pk, KP);
-                    C.comm->allreduce_sum(redbuf.p, (size_t)2 * KP, C.stream);
-                    kb_unpack<<<3, kBMaxK, 0, C.stream>>>(scb.p, redbuf.p, t, KP);
-                }
-                // two-loop recursion (lbfgs.c:572-598) as 2*bound+1 fused steps per problem
-                for (int t = 0; t <= 2 * maxbound; ++t) {
-                    KStep st{};
-                    for (int q = 0; q < K; ++q) {
-                        if (!upd.mask[q]) continue;
-                        const int bnd = bound[q], end = ps[q].end;   // `end` already advanced
-                        if (t > 2 * bnd) continue;
-                        auto js = [&](int i) { return ((end - 1 - i) % m + m) % m; };   // newest ... oldest
-                        st.op[q] = 1;
-                        st.c2_num[q] = -1;
-                        if (t == 0) {
-                            st.init[q] = 1;
-                            st.v_kind[q] = 1; st.v_slot[q] = (signed char)js(0); st.out[q] = (signed char)(SC_ALPHA0 + js(0));
-                        } else if (t <= bnd) {
-                            const int i = t - 1;
-                            st.u_kind[q] = 2; st.u_slot[q] = (signed char)js(i);
-                            st.c_num[q] = (signed char)(SC_ALPHA0 + js(i)); st.c_den[q] = (signed char)(SC_YS0 + js(i));
-                            st.csign[q] = -1;
-                            if (i + 1 < bnd) {
-                                st.v_kind[q] = 1; st.v_slot[q] = (signed char)js(i + 1);
-                                st.out[q] = (signed char)(SC_ALPHA0 + js(i + 1));
-                            } else {
-                                st.scale[q] = 1;
-                                st.v_kind[q] = 2; st.v_slot[q] = (signed char)js(i); st.out[q] = (signed char)SC_BETA;
-                            }
-                        } else {
-                            const int i = bnd - (t - bnd);          // bnd-1 ... 0
-                            const int which = (t - bnd - 1) & 1;     // beta slots alternate
-                            st.u_kind[q] = 1; st.u_slot[q] = (signed char)js(i);
-                            st.c_num[q] = (signed char)(SC_ALPHA0 + js(i)); st.c_den[q] = (signed char)(SC_YS0 + js(i));
-                            st.csign[q] = 1;
-                            st.c2_num[q] = (signed char)(which ? SC_BETA2 : SC_BETA);
-                            if (i > 0) {
-                                st.v_kind[q] = 2; st.v_slot[q] = (signed char)js(i - 1);
-                                st.out[q] = (signed char)(which ? SC_BETA : SC_BETA2);
-                            } else {
-                                st.v_kind[q] = 3; st.out[q] = (signed char)SC_DGINIT;
-                            }
-                        }
-                    }
-                    kb_twoloop<<<gridv, kVecThreads, 0, C.stream>>>(B, st);
-                    if (reduce && !forces) {
-                        KSlotTab t{};
-                        t.n = 1;
-                        t.row[0] = 0;
-                        for (int q = 0; q < kBMaxK; ++q)
-                            t.slot[0][q] = (q < K && st.op[q] && st.v_kind[q]) ? st.out[q] : (signed char)-1;
-                        allreduce_tab(t, redbuf.p);
-                    }
-                }
-                CUDA_CHECK(cudaGetLastError());
-            }
+            if (any_upd) update_directions(upd, bound);
             if (verbose && rounds % 100 == 0) printf("\t\ttheta scan round %lld\n", rounds);
         }
         for (int q = 0; q < K; ++q) {

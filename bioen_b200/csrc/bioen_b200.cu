@@ -860,6 +860,146 @@ int bioen_b200_selftest_slice_plan(int m, int n, int sms, long long max_dyn_smem
     return p.ok ? 1 : 0;
 }
 
+// One L-BFGS direction update from a given state, on the engine the minimisers would run it on (tests compare it with
+// an extended-precision two-loop recursion).  Engines 0-2 drive Lbfgs::update_direction on the context's store,
+// engine 3 ThetaScan::update_directions on a batch's planes: the same host code as the minimisers.
+int bioen_b200_selftest_lbfgs_update(bioen_b200_ctx* ctx, int engine, int method, int K, const int* end_old,
+                                     const int* bound, const double* x, const double* g, double* xp, double* gp,
+                                     double* S, double* Y, const double* ys_ring, double* d, double* scalars) {
+    return guarded("bioen_b200_selftest_lbfgs_update", [&] {
+        ctx->pending_gen = -1;
+        Context& C = ctx->C;
+        CUDA_CHECK(cudaSetDevice(C.device));
+        const bool forces = method == BIOEN_B200_FORCES;
+        const int n = ctx->dim(method), m = kGramM;
+        const size_t nm = (size_t)n * m;
+        if (engine < 0 || engine > 3) throw std::invalid_argument("bioen_b200: engine must be 0..3");
+        if (K < 1 || K > (engine == 3 ? kBMaxK : 1))
+            throw std::invalid_argument("bioen_b200: K must be 1 (engines 0-2) or 1..32 (engine 3)");
+        for (int q = 0; q < K; ++q)
+            if (end_old[q] < 0 || end_old[q] >= m || bound[q] < (engine == 3 ? 0 : 1) || bound[q] > m)
+                throw std::invalid_argument("bioen_b200: end_old must be in 0..5 and bound in 1..6 (0: inactive, "
+                                            "engine 3)");
+        auto scalar_file = [&](int q, double* dst) {
+            for (int k = 0; k < SC_COUNT; ++k) dst[k] = scalars[(size_t)q * SC_COUNT + k];
+            for (int t = 0; t < m; ++t) dst[SC_YS0 + t] = ys_ring[(size_t)q * m + t];
+        };
+        if (engine == 3) {
+            if (C.nranks > 1)
+                throw std::invalid_argument("bioen_b200: the batched engine runs on unsharded contexts only (a local "
+                                            "group cannot carry its messages)");
+            C.require_row_major("the batched theta scan");
+            ThetaScan scan(C, K, LbfgsParams(), forces);
+            const BatchBufs& B = scan.B;
+            const long long KP = scan.KP, ldn = scan.ldn;
+            auto hist = [&](double* base, int t, int q) { return base + ((size_t)t * KP + q) * ldn; };
+            std::vector<double> row(SC_COUNT);
+            for (int q = 0; q < K; ++q) {
+                const size_t o = (size_t)q * n;
+                C.h2d(B.X + q * ldn, x + o, n);
+                C.h2d(B.Gr + q * ldn, g + o, n);
+                C.h2d(B.XP + q * ldn, xp + o, n);
+                C.h2d(B.GP + q * ldn, gp + o, n);
+                C.h2d(B.D + q * ldn, d + o, n);
+                for (int t = 0; t < m; ++t) {
+                    C.h2d(hist(B.S, t, q), S + q * nm + (size_t)t * n, n);
+                    C.h2d(hist(B.Yv, t, q), Y + q * nm + (size_t)t * n, n);
+                }
+                scalar_file(q, row.data());
+                C.h2d(B.scb + q * SC_COUNT, row.data(), SC_COUNT);
+            }
+            KSlots upd{};
+            std::vector<int> bnd(K, 0);
+            for (int q = 0; q < K; ++q) {
+                upd.mask[q] = bound[q] > 0;
+                upd.slot[q] = end_old[q];
+                bnd[q] = bound[q];
+            }
+            scan.update_directions(upd, bnd);
+            for (int q = 0; q < K; ++q) {
+                const size_t o = (size_t)q * n;
+                C.d2h(xp + o, B.XP + q * ldn, n);
+                C.d2h(gp + o, B.GP + q * ldn, n);
+                C.d2h(d + o, B.D + q * ldn, n);
+                for (int t = 0; t < m; ++t) {
+                    C.d2h(S + q * nm + (size_t)t * n, hist(B.S, t, q), n);
+                    C.d2h(Y + q * nm + (size_t)t * n, hist(B.Yv, t, q), n);
+                }
+                C.d2h(scalars + (size_t)q * SC_COUNT, B.scb + q * SC_COUNT, SC_COUNT);
+            }
+            C.sync();
+            return;
+        }
+        Lbfgs opt(C, forces, LbfgsParams());
+        if (engine == 1 && (n > kSmallUpdateMaxN || opt.reduce))
+            throw std::invalid_argument("bioen_b200: the small engine takes unsharded problems of n <= 1024");
+        if (engine == 2 && opt.reduce && !C.fuse_exchange())
+            throw std::invalid_argument("bioen_b200: the Gram engine on a sharded context needs the fused exchange");
+        // the Gram kernels take ring slots [0, bound) as the valid ones, which holds for the states a minimisation
+        // reaches: the ring fills slots 0, 1, ... in order before it wraps
+        if (engine == 2 && bound[0] < m && end_old[0] != bound[0] - 1)
+            throw std::invalid_argument("bioen_b200: the Gram engine takes reachable states only (bound < 6 needs "
+                                        "end_old = bound - 1)");
+        // select the engine through the context's switches, as a minimisation would see them; restored below
+        const bool gram0 = C.lbfgs_gram_opt, small0 = C.lbfgs_small_opt;
+        C.lbfgs_gram_opt = engine == 2;
+        C.lbfgs_small_opt = engine == 1;
+        try {
+            opt.x = ctx->x_for(method);
+            opt.bind_store();
+            C.h2d(opt.x, x, n);
+            C.h2d(opt.g, g, n);
+            C.h2d(opt.xp, xp, n);
+            C.h2d(opt.gp, gp, n);
+            C.h2d(opt.d, d, n);
+            for (int t = 0; t < m; ++t) {
+                C.h2d(opt.S[t], S + (size_t)t * n, n);
+                C.h2d(opt.Yv[t], Y + (size_t)t * n, n);
+            }
+            std::vector<double> row(SC_COUNT);
+            scalar_file(0, row.data());
+            C.h2d(C.sc.p, row.data(), SC_COUNT);
+            if (engine == 2) {
+                // the resident Gram matrix of the pairs already in the ring, b = [s_0..s_5, y_0..y_5, g]: one device dot
+                // per entry (three per launch along a row), summed over the ranks when sharded.  Its diagonal s_t . y_t
+                // is then set to the ring's ys_t: in a minimisation both are the one value k_lbfgs_gram_pair stored.
+                double* Gm = C.lbfgs_gram.p;
+                auto basis = [&](int k) { return k < m ? opt.S[k] : opt.Yv[k - m]; };
+                for (int a = 0; a < 2 * m; ++a)
+                    for (int b = 0; b < 2 * m; b += 3) {
+                        Dot3Args da{n, basis(a), basis(b), basis(a), basis(b + 1), basis(a), basis(b + 2),
+                                    Gm + a * kGramB + b, C.red_partials.p, C.ticket.p};
+                        k_dot3<<<opt.vec_blocks, kVecThreads, 0, C.stream>>>(da);
+                    }
+                CUDA_CHECK(cudaGetLastError());
+                if (opt.reduce) C.comm->allreduce_sum(Gm, kGramB * kGramB, C.stream);
+                for (int t = 0; t < bound[0]; ++t) {
+                    if (t == end_old[0]) continue;
+                    C.h2d(Gm + t * kGramB + m + t, ys_ring + t, 1);
+                    C.h2d(Gm + (m + t) * kGramB + t, ys_ring + t, 1);
+                }
+            }
+            opt.update_direction(end_old[0], bound[0], m);
+            CUDA_CHECK(cudaGetLastError());
+            C.d2h(xp, opt.xp, n);
+            C.d2h(gp, opt.gp, n);
+            C.d2h(d, opt.d, n);
+            for (int t = 0; t < m; ++t) {
+                C.d2h(S + (size_t)t * n, opt.S[t], n);
+                C.d2h(Y + (size_t)t * n, opt.Yv[t], n);
+            }
+            C.d2h(scalars, C.sc.p, SC_COUNT);
+            C.sync();
+        } catch (...) {
+            C.lbfgs_gram_opt = gram0;
+            C.lbfgs_small_opt = small0;
+            throw;
+        }
+        C.lbfgs_gram_opt = gram0;
+        C.lbfgs_small_opt = small0;
+    });
+}
+
 int bioen_b200_nccl_unique_id(char id[128]) {
     return guarded("bioen_b200_nccl_unique_id", [&] { Comm::unique_id(id); });
 }
@@ -1080,6 +1220,7 @@ int bioen_b200_debug_read(bioen_b200_ctx* ctx, int what, double* out_host, size_
             case 2: src = C.avg.p; cap = C.M; break;
             case 3: src = C.aux_n.p; cap = C.aux_n.n; break;
             case 4: src = C.aux_n2.p; cap = C.aux_n2.n; break;
+            case 5: src = C.lbfgs_store.p; cap = C.lbfgs_store.n; break;
             default: throw std::invalid_argument("bioen_b200: unknown debug buffer");
         }
         if (count > cap) throw std::invalid_argument("bioen_b200: debug read too long");

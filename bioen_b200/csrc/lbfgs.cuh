@@ -317,20 +317,9 @@ class Lbfgs {
         int ret = lbfgs_check_params(n, prm);
         if (ret) { *fx_out = 0.0; return ret; }
         const int m = prm.m;
-        const size_t np = ((size_t)n + 15) & ~(size_t)15;
-        // the work vectors live in the context and are reused by the next minimisation of the same size (every
-        // vector is written before it is read, so no clearing is needed)
-        C.lbfgs_store.reserve(np * (4 + 2 * (size_t)m));
-        g = C.lbfgs_store.p; xp = g + np; gp = xp + np; d = gp + np;
-        S.resize(m); Yv.resize(m);
-        for (int i = 0; i < m; ++i) { S[i] = d + np * (1 + i); Yv[i] = d + np * (1 + m + i); }
+        bind_store();
         std::vector<double> pf(prm.past > 0 ? prm.past : 0);
         const double* h = C.h_sc;
-        if (gram_mode()) {
-            C.lbfgs_gram.reserve(kGramB * kGramB + kGramB + 3);
-            C.lbfgs_gram_partials.reserve((size_t)vec_blocks * kGramK + 8);
-            CUDA_CHECK(cudaMemsetAsync(C.lbfgs_gram.p, 0, (kGramB * kGramB + kGramB) * sizeof(double), C.stream));
-        }
 
         // initial evaluation (lbfgs.c:412)
         eval(nullptr, nullptr, 0.0, nullptr);
@@ -385,6 +374,63 @@ class Lbfgs {
         }
         *fx_out = fx;
         return ret;
+    }
+
+    // point g, xp, gp, d and the (s, y) ring at the context's L-BFGS store (bioen_b200_debug_read 5 reads it back):
+    // [g | xp | gp | d | s_0 .. s_{m-1} | y_0 .. y_{m-1}], each n rounded up to 16.  The work vectors are reused by the
+    // next minimisation of the same size (every vector is written before it is read, so no clearing is needed); the
+    // Gram matrix of the coefficient-space update starts from zero.
+    void bind_store() {
+        const int m = prm.m;
+        const size_t np = ((size_t)n + 15) & ~(size_t)15;
+        C.lbfgs_store.reserve(np * (4 + 2 * (size_t)m));
+        g = C.lbfgs_store.p; xp = g + np; gp = xp + np; d = gp + np;
+        S.resize(m); Yv.resize(m);
+        for (int i = 0; i < m; ++i) { S[i] = d + np * (1 + i); Yv[i] = d + np * (1 + m + i); }
+        if (gram_mode()) {
+            C.lbfgs_gram.reserve(kGramB * kGramB + kGramB + 3);
+            C.lbfgs_gram_partials.reserve((size_t)vec_blocks * kGramK + 8);
+            CUDA_CHECK(cudaMemsetAsync(C.lbfgs_gram.p, 0, (kGramB * kGramB + kGramB) * sizeof(double), C.stream));
+        }
+    }
+
+    // the new pair into ring slot end_old and the two-loop recursion over `bound` pairs, on whichever engine the
+    // context selects (Gram, small, multi-kernel; CUDA graphs when enabled).  Also bioen_b200_selftest_lbfgs_update.
+    void update_direction(int end_old, int bound, int m) {
+        if (gram_mode()) {
+            enqueue_update_gram(end_old, bound);
+            return;
+        }
+        if (small_mode()) {
+            enqueue_update_small(end_old, bound);
+            return;
+        }
+        if (use_graphs) {
+            const int key = end_old * 64 + bound;
+            auto it = g_update.find(key);
+            if (it == g_update.end()) {
+                long long nk = 0;
+                cudaGraphExec_t ex = capture([&] { enqueue_update(end_old, bound, m); }, &nk);
+                if (!ex) {
+                    use_graphs = false;
+                    enqueue_update(end_old, bound, m);
+                    return;
+                }
+                it = g_update.emplace(key, std::make_pair(ex, nk)).first;
+            }
+            CUDA_CHECK(cudaGraphLaunch(it->second.first, C.stream));
+            C.kernels_launched += it->second.second;
+            return;
+        }
+        enqueue_update(end_old, bound, m);
+    }
+    bool gram_mode() const {
+        // sharded runs need the in-kernel exchange (the peer-memory path); m is liblbfgs' default 6
+        return C.lbfgs_gram_opt && prm.m == kGramM && (!reduce || C.fuse_exchange());
+    }
+    // small problems (n <= 1024): pair + two-loop recursion as ONE single-CTA kernel (k_lbfgs_update_small)
+    bool small_mode() const {
+        return C.lbfgs_small_opt && n <= kSmallUpdateMaxN && prm.m == kSmallUpdateM && !reduce;
     }
 
    private:
@@ -545,14 +591,6 @@ class Lbfgs {
         k_lbfgs_combine<<<vec_blocks, kVecThreads, 0, C.stream>>>(b);
         C.kernels_launched += 2;
     }
-    bool gram_mode() const {
-        // sharded runs need the in-kernel exchange (the peer-memory path); m is liblbfgs' default 6
-        return C.lbfgs_gram_opt && prm.m == kGramM && (!reduce || C.fuse_exchange());
-    }
-    // small problems (n <= 1024): pair + two-loop recursion as ONE single-CTA kernel (k_lbfgs_update_small)
-    bool small_mode() const {
-        return C.lbfgs_small_opt && n <= kSmallUpdateMaxN && prm.m == kSmallUpdateM && !reduce;
-    }
     void enqueue_update_small(int end_old, int bound) {
         NvtxRange nvtx("bioen:lbfgs_update(small)");
         SmallUpdateArgs a{};
@@ -561,34 +599,6 @@ class Lbfgs {
         a.end = end_old; a.bound = bound; a.sc = C.sc.p;
         k_lbfgs_update_small<<<1, ((n + 31) / 32) * 32, 0, C.stream>>>(a);
         ++C.kernels_launched;
-    }
-    void update_direction(int end_old, int bound, int m) {
-        if (gram_mode()) {
-            enqueue_update_gram(end_old, bound);
-            return;
-        }
-        if (small_mode()) {
-            enqueue_update_small(end_old, bound);
-            return;
-        }
-        if (use_graphs) {
-            const int key = end_old * 64 + bound;
-            auto it = g_update.find(key);
-            if (it == g_update.end()) {
-                long long nk = 0;
-                cudaGraphExec_t ex = capture([&] { enqueue_update(end_old, bound, m); }, &nk);
-                if (!ex) {
-                    use_graphs = false;
-                    enqueue_update(end_old, bound, m);
-                    return;
-                }
-                it = g_update.emplace(key, std::make_pair(ex, nk)).first;
-            }
-            CUDA_CHECK(cudaGraphLaunch(it->second.first, C.stream));
-            C.kernels_launched += it->second.second;
-            return;
-        }
-        enqueue_update(end_old, bound, m);
     }
 
     // the recursion of lbfgs.c:572-598 as 2*bound+1 fused kernels; the last one also leaves g.d in SC_DGINIT

@@ -765,7 +765,8 @@ __global__ void __launch_bounds__(kVecThreads) k_lbfgs_twoloop(const TwoLoopArgs
 // fixture of the reference's test-suite): k_lbfgs_pair + the 2*bound+1 kernels of the two-loop recursion as ONE
 // single-CTA kernel.  Thread j owns element j of every vector and keeps d_j, g_j and the six (s, y) pairs in
 // registers; the 2*bound+2 dot products are block reductions (one __syncthreads each), the coefficients are formed from
-// the same raw dot products in the same order as k_lbfgs_twoloop does, and the same scalar-file slots are written.
+// the same raw dot products in the same order as k_lbfgs_twoloop does, and the same scalar-file outputs are written
+// (ys, yy, the ys and raw s.d rings, g.d; the second loop's dots stay in registers instead of SC_BETA / SC_BETA2).
 // 15 launches of ~3 us become one of ~5 us -- at these sizes the update, not the evaluation, was most of an iteration.
 // For n <= 256 (one block in the multi-kernel path as well) the result is bit-identical to that path.
 // ------------------------------------------------------------------------------------------------

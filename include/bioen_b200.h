@@ -327,6 +327,20 @@ int bioen_b200_selftest_num_slots(long long run, long long L, long long chunk);
  * log2 threads along the columns (column sums), log2 lanes per row (row sums), log2 lanes per row (table sums),
  * dynamic shared memory in bytes}. */
 int bioen_b200_selftest_slice_plan(int m, int n, int sms, long long max_dyn_smem, long long out[8]);
+/* device test hook: ONE L-BFGS direction update (new pair s = x - xp, y = g - gp into ring slot end_old, then the
+ * two-loop recursion over `bound` pairs, lbfgs.c:543-598) from a given state, on engine 0 (multi-kernel), 1 (single-CTA
+ * kernel, unsharded, n <= 1024), 2 (coefficient space with the resident Gram matrix, filled first from S and Y, its
+ * diagonal s_t . y_t from ys_ring; reachable states only: bound < 6 needs end_old = bound - 1) or 3
+ * (the batched planes of the theta scan; unsharded contexts), through the same host code as the minimisers.  n = N
+ * (BIOEN_B200_LOGW; this rank's columns when sharded) or M (BIOEN_B200_FORCES); m = 6; K problems (1 for engines 0-2,
+ * 1..32 for engine 3; engine 3 needs bioen_b200_set_logw / _set_forces first).  Row-major host arrays:
+ *   in      end_old[K] in 0..5, bound[K] in 1..6 (0: inactive problem, engine 3), x[K][n], g[K][n], ys_ring[K][m]
+ *   in/out  xp[K][n], gp[K][n], S[K][m][n], Y[K][m][n], d[K][n], scalars[K][64] (the scalar file; its ys ring is
+ *           replaced by ys_ring on input)
+ * An inactive problem's arrays come back as they went in. */
+int bioen_b200_selftest_lbfgs_update(bioen_b200_ctx *ctx, int engine, int method, int K, const int *end_old,
+                                     const int *bound, const double *x, const double *g, double *xp, double *gp,
+                                     double *S, double *Y, const double *ys_ring, double *d, double *scalars);
 
 /* multi-GPU: one process per GPU, N sharded.  Rank 0 creates the id, the host layer broadcasts it. */
 int bioen_b200_nccl_unique_id(char id[128]);
@@ -366,6 +380,9 @@ long long bioen_b200_kernels_launched(bioen_b200_ctx *ctx);
  * run on the slice kernel now; 8: bytes of device memory held by the context's copies of yTilde (row-major +
  * structure-major + fp32); 9: 1 in structure-major-only mode.  Returns -1 for an unknown `what`. */
 long long bioen_b200_query(bioen_b200_ctx *ctx, int what);
+/* copy `count` doubles of a device buffer the context holds (tests): what = 0 the scalar file (64), 1 weights, 2
+ * averages, 3 / 4 the forces method's per-structure vectors, 5 the L-BFGS store of the last minimisation,
+ * [g | xp | gp | d | s_0..s_5 | y_0..y_5] with each vector's n rounded up to 16 */
 int bioen_b200_debug_read(bioen_b200_ctx *ctx, int what, double *out_host, size_t count);
 /* the context's cudaStream_t (for callers that enqueue their own work around the device entry points) */
 void *bioen_b200_stream(bioen_b200_ctx *ctx);

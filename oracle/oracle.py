@@ -501,6 +501,25 @@ def _ls_morethuente(evaluate, x, f, g, s, stp, xp, p):
             width = abs(sty - stx)
 
 
+def lbfgs_two_loop(g, S, Yv, ys_arr, end, bound, ys, yy):
+    """liblbfgs' two-loop recursion (lbfgs.c:572-598): d = -H g over the `bound` newest pairs of the ring (S, Yv),
+    the newest in slot end - 1; ys_arr[j] = y_j.s_j, and ys, yy of the newest pair scale H0."""
+    m = len(ys_arr)
+    alpha = np.zeros(m)
+    d = -np.asarray(g, dtype=np.float64)
+    j = end
+    for _ in range(bound):
+        j = (j + m - 1) % m
+        alpha[j] = float(np.dot(S[j], d)) / ys_arr[j]
+        d += (-alpha[j]) * Yv[j]
+    d *= ys / yy
+    for _ in range(bound):
+        beta = float(np.dot(Yv[j], d)) / ys_arr[j]
+        d += (alpha[j] - beta) * S[j]
+        j = (j + 1) % m
+    return d
+
+
 def lbfgs(fg, x0, **params):
     """liblbfgs `lbfgs()` (lbfgs.c:245-641) restated for NumPy vectors.
 
@@ -529,7 +548,7 @@ def lbfgs(fg, x0, **params):
     g = np.empty(n)
     xp, gp = np.empty(n), np.empty(n)
     S, Yv = np.zeros((m, n)), np.zeros((m, n))
-    ys_arr, alpha = np.zeros(m), np.zeros(m)
+    ys_arr = np.zeros(m)
     pf = np.zeros(p["past"]) if p["past"] > 0 else None
 
     fx = evaluate(x, g)
@@ -579,17 +598,7 @@ def lbfgs(fg, x0, **params):
         bound = m if m <= k else k
         k += 1
         end = (end + 1) % m
-        d[:] = -g
-        j = end
-        for _ in range(bound):
-            j = (j + m - 1) % m
-            alpha[j] = float(np.dot(S[j], d)) / ys_arr[j]
-            d += (-alpha[j]) * Yv[j]
-        d *= ys / yy
-        for _ in range(bound):
-            beta = float(np.dot(Yv[j], d)) / ys_arr[j]
-            d += (alpha[j] - beta) * S[j]
-            j = (j + 1) % m
+        d[:] = lbfgs_two_loop(g, S, Yv, ys_arr, end, bound, ys, yy)
         step = 1.0
     info.update(fx=fx, code=code, evaluations=nev[0])
     return info

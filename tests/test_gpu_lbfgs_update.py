@@ -1,0 +1,449 @@
+"""GPU: every L-BFGS direction-update engine against the extended-precision two-loop recursion (tests/hp_twoloop.py).
+
+The end points of a minimisation forgive almost any error in the direction (L-BFGS converges with a wrong H, only
+slower), and bit-identity of two engines shows they agree, not that either is right.  Here each engine's update is
+checked on its own:
+
+(a) synthetic states through bioen_b200_selftest_lbfgs_update, on every regime of tests/lbfgs_regimes.py and every
+    (end_old, bound): the multi-kernel engine (k_lbfgs_pair + k_lbfgs_twoloop), the single-CTA kernel, the
+    coefficient-space (Gram) engine on reachable states, the batched engine of the theta scan with every problem of
+    one launch at its own (end, bound) and some inactive, and the sharded engines through dist.LocalGroup.  s, y, xp,
+    gp must be bitwise, ys, yy, the raw s_j . d ring and g . d and every component of d under |gpu - ref| <= C u scale.
+(b) the drivers' own histories: opt_lbfgs stopped after k = 1 .. 14 iterations (the ring wraps twice) under every line
+    search, with the small, Gram, speculative-trial and CUDA-graph switches; the store the minimiser leaves (debug
+    read 5) must continue the run of k - 1 iterations bit for bit, and its d must be the reference recursion on its own
+    S, Y and gradient.
+"""
+import ctypes
+import os
+from collections import OrderedDict
+
+import numpy as np
+import pytest
+
+import hp_reference as H
+import hp_twoloop as T
+import lbfgs_regimes as R
+from conftest import load_golden
+
+pytestmark = [pytest.mark.gpu,
+              pytest.mark.skipif(not H.available(), reason="np.longdouble is not the x86-64 80-bit format")]
+
+os.environ.setdefault("BIOEN_B200_P2P_TIMEOUT_S", "30")
+
+# One constant for every engine and regime; the benign regime sets the baseline (C >= 4x its largest ratio, printed by
+# test_zz_report).  The Gram engine is judged by its own scale (hp_twoloop.gram); its ratio against the vector
+# recursion's scale is reported, not asserted.
+C = 16
+LOGW, FORCES = 0, 1
+MULTI, SMALL, GRAM, BATCHED = 0, 1, 2, 3
+OPT_FUSED_EXCHANGE, OPT_LBFGS_GRAM, OPT_LBFGS_SMALL, OPT_LBFGS_SPECULATIVE = 4, 6, 9, 10
+SC_YS, SC_YY, SC_DGINIT, SC_YS0, SC_ALPHA0 = 16, 17, 19, 24, 40
+MAXIMUMITERATION = -997
+M = T.M
+# the scalar-file slots an update writes: ys, yy, g.d, the ys ring and the raw s.d ring
+LBFGS_SLOTS = [SC_YS, SC_YY, SC_DGINIT] + list(range(SC_YS0, SC_YS0 + M)) + list(range(SC_ALPHA0, SC_ALPHA0 + M))
+
+# where the vector kernels' grid stops growing (148 SMs x 4 blocks of 256 threads) and the grid-stride loop takes a
+# second lap
+GRID_END = 148 * 4 * 256
+MULTI_N = [1, 5, 255, 256, 257, 1025, 4003, GRID_END, GRID_END + 1, 1000003]
+SMALL_N = [1, 31, 32, 33, 255, 256, 257, 1000, 1023, 1024]
+GRAM_N = [n for n in MULTI_N if n <= 1025]
+BIG = 100000
+BIG_STATES = [(0, 1), (3, 4), (5, 6), (2, 6)]     # large n: a few states keep the reference's time down
+
+WORST = {}             # (engine, benign?) -> largest ratio
+GRAM_VS_VECTOR = {}    # regime -> largest ratio of the Gram engine against the vector recursion's scale
+
+
+def _record(key, regime, r):
+    k = (key, regime == "benign")
+    WORST[k] = max(WORST.get(k, 0.0), r)
+
+
+class _Cache:
+    def __init__(self, size=3):
+        self.size, self.items = size, OrderedDict()
+
+    def get(self, key, make):
+        if key in self.items:
+            self.items.move_to_end(key)
+            return self.items[key]
+        while len(self.items) >= self.size:
+            self.items.popitem(last=False)[1].close()
+        self.items[key] = make()
+        return self.items[key]
+
+    def close(self):
+        while self.items:
+            self.items.popitem()[1].close()
+
+
+@pytest.fixture(scope="module")
+def cache():
+    c = _Cache()
+    yield c
+    c.close()
+
+
+_REFS = OrderedDict()
+
+
+def _state_ref(regime, n, end_old, bound, seed=0):
+    key = (regime, n, end_old, bound, seed)
+    if key not in _REFS:
+        st = R.state(regime, n, end_old, bound, seed)
+        ref = T.update(st["x"], st["xp"], st["g"], st["gp"], st["S"], st["Y"], st["ys_ring"], end_old, bound)
+        _REFS[key] = (st, ref)
+        while len(_REFS) > 64:
+            _REFS.popitem(last=False)
+    return _REFS[key]
+
+
+def _hook(p, engine, states, method=LOGW, lo=0, hi=None):
+    """run bioen_b200_selftest_lbfgs_update on K = len(states) problems (columns lo:hi of each: a rank's slice); an
+    entry None is an inactive problem.  Returns the inputs and the outputs (xp, gp, S, Y, d, sc)."""
+    from bioen_b200 import _lib
+    K = len(states)
+    live = next(s for s in states if s is not None)
+    hi = live["x"].size if hi is None else hi
+    n = hi - lo
+    rng = np.random.default_rng(n + K)
+    pick = lambda s, k, shape: (rng.standard_normal(shape) if s is None else s[k][..., lo:hi])
+    inp = dict(
+        x=np.ascontiguousarray([pick(s, "x", n) for s in states]),
+        g=np.ascontiguousarray([pick(s, "g", n) for s in states]),
+        xp=np.ascontiguousarray([pick(s, "xp", n) for s in states]),
+        gp=np.ascontiguousarray([pick(s, "gp", n) for s in states]),
+        S=np.ascontiguousarray([pick(s, "S", (M, n)) for s in states]),
+        Y=np.ascontiguousarray([pick(s, "Y", (M, n)) for s in states]),
+        ys=np.ascontiguousarray([np.full(M, 5.0) if s is None else s["ys_ring"] for s in states]),
+        d=np.full((K, n), 3.25),                 # d is written before it is read
+        sc=np.full((K, 64), 1.5))
+    inp["sc"][:, SC_YS0:SC_YS0 + M] = inp["ys"]
+    end = (ctypes.c_int * K)(*[0 if s is None else s["end_old"] for s in states])
+    bnd = (ctypes.c_int * K)(*[0 if s is None else s["bound"] for s in states])
+    out = {k: inp[k].copy() for k in ("xp", "gp", "S", "Y", "d", "sc")}
+    lib = _lib.load()
+    _lib.check(lib.bioen_b200_selftest_lbfgs_update(
+        p._ctx, engine, method, K, end, bnd, _lib.ptr(inp["x"]), _lib.ptr(inp["g"]), _lib.ptr(out["xp"]),
+        _lib.ptr(out["gp"]), _lib.ptr(out["S"]), _lib.ptr(out["Y"]), _lib.ptr(inp["ys"]), _lib.ptr(out["d"]),
+        _lib.ptr(out["sc"])), "selftest_lbfgs_update")
+    return inp, out
+
+
+def _check(engine, regime, st, ref, S, Y, xp, gp, d, sc, gram=False):
+    """one problem's outputs (full length) against the reference; returns the largest ratio"""
+    end_old, bound = st["end_old"], st["bound"]
+    assert np.array_equal(S[end_old], ref["s"]) and np.array_equal(Y[end_old], ref["y"]), "new pair not bitwise"
+    assert np.array_equal(xp, st["x"]) and np.array_equal(gp, st["g"]), "xp <- x, gp <- g not bitwise"
+    for t in range(M):
+        if t != end_old:
+            assert np.array_equal(S[t], st["S"][t]) and np.array_equal(Y[t], st["Y"][t]), ("ring slot changed", t)
+    assert sc[SC_YS0 + end_old] == sc[SC_YS] or not np.isfinite(sc[SC_YS])
+    if gram:
+        gr = T.gram(st["g"], ref["S"], ref["Y"], end_old, bound, st["ys_ring"])
+        r = dict(ys=T.ratio(sc[SC_YS], gr["ys"], gr["s_ys"]), yy=T.ratio(sc[SC_YY], gr["yy"], gr["s_yy"]),
+                 dg=T.ratio(sc[SC_DGINIT], gr["dg"], gr["s_dg"]), d=T.ratio(d, gr["d"], gr["s_d"]))
+        vec = max(T.ratio(d, ref["d"], ref["s_d"]), T.ratio(sc[SC_DGINIT], ref["dg"], ref["s_dg"]))
+        GRAM_VS_VECTOR[regime] = max(GRAM_VS_VECTOR.get(regime, 0.0), vec)
+    else:
+        r = dict(ys=T.ratio(sc[SC_YS], ref["ys"], ref["s_ys"]), yy=T.ratio(sc[SC_YY], ref["yy"], ref["s_yy"]),
+                 dg=T.ratio(sc[SC_DGINIT], ref["dg"], ref["s_dg"]), d=T.ratio(d, ref["d"], ref["s_d"]))
+        for j, a in ref["alpha"].items():
+            r["alpha%d" % j] = T.ratio(sc[SC_ALPHA0 + j], a, ref["s_alpha"][j])
+    worst = max(r.values())
+    _record(engine, regime, worst)
+    assert worst <= C, (regime, end_old, bound, {k: "%.3g" % v for k, v in r.items() if v > C})
+    return worst
+
+
+def _single(n):
+    import bioen_b200
+    return bioen_b200.Problem(shape=(4, n))
+
+
+def _run_single(cache, engine, n, regime, states):
+    p = cache.get(("single", n), lambda: _single(n))
+    for end_old, bound in states:
+        st, ref = _state_ref(regime, n, end_old, bound)
+        _, out = _hook(p, engine, [st])
+        _check(engine, regime, st, ref, out["S"][0], out["Y"][0], out["xp"][0], out["gp"][0], out["d"][0],
+               out["sc"][0], gram=(engine == GRAM))
+        if engine == SMALL and n <= 256:
+            # the documented claim: bit-identical to the multi-kernel engine up to 256 variables
+            # (the scalar file's outputs: the single-CTA kernel keeps the second loop's dots in registers, the
+            # multi-kernel engine passes them through SC_BETA / SC_BETA2)
+            _, o0 = _hook(p, MULTI, [st])
+            assert o0["d"].tobytes() == out["d"].tobytes() and \
+                o0["sc"][0, LBFGS_SLOTS].tobytes() == out["sc"][0, LBFGS_SLOTS].tobytes(), (end_old, bound)
+
+
+@pytest.mark.parametrize("regime", R.REGIMES)
+@pytest.mark.parametrize("n", MULTI_N)
+def test_multi_kernel(cache, n, regime):
+    _run_single(cache, MULTI, n, regime, R.ALL_STATES if n < BIG else BIG_STATES)
+
+
+@pytest.mark.parametrize("regime", R.REGIMES)
+@pytest.mark.parametrize("n", SMALL_N)
+def test_small(cache, n, regime):
+    _run_single(cache, SMALL, n, regime, R.ALL_STATES)
+
+
+@pytest.mark.parametrize("regime", R.REGIMES)
+@pytest.mark.parametrize("n", GRAM_N)
+def test_gram(cache, n, regime):
+    """reachable states only: the Gram kernels treat slots [0, bound) as the valid ones"""
+    _run_single(cache, GRAM, n, regime, R.REACHABLE)
+
+
+@pytest.mark.parametrize("regime", R.REGIMES)
+@pytest.mark.parametrize("n", [5, 777, 4003])
+@pytest.mark.parametrize("K", [1, 7, 8, 9, 32])
+def test_batched(cache, K, n, regime):
+    """one launch of the theta scan's update engine: problem q at its own (end_old, bound), every fifth inactive (its
+    planes and scalar row must come back untouched)"""
+    import bioen_b200
+
+    def make():
+        rng = np.random.default_rng(n)
+        p = bioen_b200.Problem(rng.standard_normal((8, n)))
+        p.set_logw(np.zeros(n), rng.standard_normal(8), 1.0)
+        return p
+    p = cache.get(("batched", n), make)
+    ri = R.REGIMES.index(regime)
+    states, refs = [], []
+    for q in range(K):
+        if K > 1 and q % 5 == 4:
+            states.append(None)
+            refs.append(None)
+            continue
+        end_old, bound = R.ALL_STATES[(7 * q + 5 * ri + n) % len(R.ALL_STATES)]
+        st, ref = _state_ref(regime, n, end_old, bound, seed=q)
+        states.append(st)
+        refs.append(ref)
+    inp, out = _hook(p, BATCHED, states)
+    for q, (st, ref) in enumerate(zip(states, refs)):
+        if st is None:
+            for k in ("xp", "gp", "S", "Y", "d", "sc"):
+                assert out[k][q].tobytes() == inp[k][q].tobytes(), ("inactive problem changed", q, k)
+            continue
+        _check(BATCHED, regime, st, ref, out["S"][q], out["Y"][q], out["xp"][q], out["gp"][q], out["d"][q],
+               out["sc"][q])
+
+
+SHARDED = [(2, 257, MULTI, 1), (2, 4003, MULTI, 0), (3, 4003, MULTI, 1), (3, 4003, MULTI, 0), (3, 1000, MULTI, 1),
+           (2, 4003, GRAM, 1), (3, 1025, GRAM, 1)]
+
+
+@pytest.mark.parametrize("regime", R.REGIMES)
+@pytest.mark.parametrize("world,n,engine,fused", SHARDED)
+def test_sharded(cache, world, n, engine, fused, regime):
+    """N split unevenly over 2 or 3 ranks of one process; the dot products are exchanged in-kernel (fused) or by
+    separate all-reduces.  Every rank returns the same scalar file bit for bit; d is gathered before the check."""
+    from bioen_b200 import dist as D
+    grp = cache.get(("group", world, n), lambda: D.LocalGroup(np.random.default_rng(n).standard_normal((4, n)), world))
+    grp.call(lambda r, p, lo, hi: p.set_option(OPT_FUSED_EXCHANGE, fused))
+    try:
+        for end_old, bound in R.REACHABLE:
+            st, ref = _state_ref(regime, n, end_old, bound)
+            res = grp.call(lambda r, p, lo, hi: _hook(p, engine, [st], lo=lo, hi=hi)[1])
+            for o in res[1:]:
+                assert o["sc"].tobytes() == res[0]["sc"].tobytes(), "ranks disagree on the scalar file"
+            cat = lambda k: np.concatenate([o[k][0] for o in res], axis=-1)
+            _check((engine, "sharded"), regime, st, ref, cat("S"), cat("Y"), cat("xp"), cat("gp"), cat("d"),
+                   res[0]["sc"][0], gram=(engine == GRAM))
+    finally:
+        grp.call(lambda r, p, lo, hi: p.set_option(OPT_FUSED_EXCHANGE, 1))
+
+
+def test_hook_refuses_bad_input(cache):
+    import bioen_b200
+    st, _ = _state_ref("benign", 1025, 0, 1)
+    with pytest.raises(RuntimeError, match="small engine"):
+        _hook(cache.get(("single", 1025), lambda: _single(1025)), SMALL, [st])
+    st5, _ = _state_ref("benign", 5, 0, 1)
+    with pytest.raises(RuntimeError, match="K must be"):
+        _hook(cache.get(("single", 5), lambda: _single(5)), MULTI, [st5, st5])
+    bad = dict(st5, bound=7)
+    with pytest.raises(RuntimeError, match="bound"):
+        _hook(cache.get(("single", 5), lambda: _single(5)), MULTI, [bad])
+    unreachable, _ = _state_ref("benign", 5, 2, 4)
+    with pytest.raises(RuntimeError, match="reachable states only"):
+        _hook(cache.get(("single", 5), lambda: _single(5)), GRAM, [unreachable])
+    from bioen_b200 import dist as D
+    with D.LocalGroup(np.random.default_rng(0).standard_normal((4, 10)), 2) as grp:
+        errs = grp.call(lambda r, p, lo, hi: _refused(p, lo, hi))
+    assert all("unsharded" in e for e in errs), errs
+    with bioen_b200.Problem(shape=(4, 5)) as p:
+        with pytest.raises(RuntimeError, match="log-weights data not set"):
+            _hook(p, BATCHED, [st5])
+
+
+def _refused(p, lo, hi):
+    st = R.state("benign", 10, 0, 1)
+    try:
+        _hook(p, BATCHED, [st], lo=lo, hi=hi)
+    except RuntimeError as e:
+        return str(e)
+    return "ran"
+
+
+# ---- (b) the drivers' own histories ---------------------------------------------------------------------------------
+def _datasets():
+    rng = np.random.default_rng(7)
+    out = OrderedDict()
+    d = load_golden("data_forces_M64xN64")
+    out["forces_M64xN64"] = (FORCES, d["yTilde"], d["w0"].ravel(), d["YTilde"].ravel(), d["theta"],
+                             d["forces_init"].ravel(), 1)
+    d = load_golden("data_potra_part_1_logw_M808xN80")
+    out["potra_logw_M808xN80"] = (LOGW, d["yTilde"], d["G"].ravel(), d["YTilde"].ravel(), d["theta"],
+                                  d["GInit"].ravel(), 1)
+    y = rng.standard_normal((28, 5001))
+    G = 0.3 * rng.standard_normal(5001)
+    out["synthetic_logw_28x5001"] = (LOGW, y, G, y @ np.full(5001, 1 / 5001) + 0.3 * rng.standard_normal(28), 2.0,
+                                     G + 0.1 * rng.standard_normal(5001), 1)
+    y = rng.standard_normal((1000, 777))
+    w0 = rng.random(777) + 0.1
+    out["synthetic_forces_1000x777"] = (FORCES, y, w0 / w0.sum(), y @ (w0 / w0.sum()) + 0.3 * rng.standard_normal(1000),
+                                        5.0, 0.01 * rng.standard_normal(1000), 1)
+    y = rng.standard_normal((300, 4003))
+    G = 0.3 * rng.standard_normal(4003)
+    out["sharded3_logw_300x4003"] = (LOGW, y, G, y @ np.full(4003, 1 / 4003) + 0.3 * rng.standard_normal(300), 2.0,
+                                     G + 0.1 * rng.standard_normal(4003), 3)
+    return out
+
+
+DATASETS = _datasets()
+TOGGLES = ["default", "small_off", "gram", "speculative_off", "graphs"]
+
+
+def _toggle_cases():
+    out = []
+    for name, ds in DATASETS.items():
+        for tog in TOGGLES:
+            if ds[6] > 1 and tog in ("small_off", "graphs"):
+                continue                      # sharded: no small engine, no graph replays
+            out.append(pytest.param(name, tog, id="%s-%s" % (name, tog)))
+    return out
+
+
+def _store(p, n):
+    np_ = (n + 15) // 16 * 16
+    raw = p.debug_read(5, np_ * (4 + 2 * M))
+    v = lambda i: raw[i * np_:i * np_ + n]
+    return dict(g=v(0), xp=v(1), gp=v(2), d=v(3), S=np.array([v(4 + t) for t in range(M)]),
+                Y=np.array([v(4 + M + t) for t in range(M)]))
+
+
+def _driver_ref(st, sc, k, gram):
+    """the reference two-loop on the device's own ring after k - 1 updates (newest pair in slot (k - 2) mod 6)"""
+    end, bound = (k - 1) % M, min(M, k - 1)
+    new = (k - 2) % M
+    sl, yl = T._ld(st["S"][new]), T._ld(st["Y"][new])
+    ys, s_ys = T._dot(yl, sl)
+    yy, s_yy = T._dot(yl, yl)
+    if gram:
+        return T.gram(st["gp"], st["S"], st["Y"], new, bound, sc[SC_YS0:SC_YS0 + M])
+    ring, s_ring = T._ld(sc[SC_YS0:SC_YS0 + M]).copy(), np.zeros(M, dtype=T.LD)
+    ring[new], s_ring[new] = ys, s_ys
+    return T.two_loop(st["gp"], st["S"], st["Y"], ring, s_ring, end, bound, ys, s_ys, yy, s_yy)
+
+
+@pytest.mark.parametrize("linesearch", [0, 1, 2, 3])
+@pytest.mark.parametrize("name,toggle", _toggle_cases())
+def test_driver_histories(cache, name, toggle, linesearch):
+    import bioen_b200
+    from bioen_b200 import dist as D
+    method, y, a, Yt, theta, x0, world = DATASETS[name]
+    n = y.shape[0] if method == FORCES else y.shape[1]
+    if world > 1:
+        obj = cache.get(("group", world, name), lambda: D.LocalGroup(y, world))
+    else:
+        obj = cache.get(("driver", name), lambda: bioen_b200.Problem(y))
+
+    def setup(p, lo, hi):
+        if method == LOGW:
+            p.set_logw(a[lo:hi], Yt, theta)
+        else:
+            p.set_forces(a, Yt, theta)
+        p.set_option(OPT_LBFGS_SMALL, 0 if toggle == "small_off" else 1)
+        p.set_option(OPT_LBFGS_GRAM, 1 if toggle == "gram" else 0)
+        p.set_option(OPT_LBFGS_SPECULATIVE, 0 if toggle == "speculative_off" else 1)
+
+    def run(p, lo, hi, k):
+        xs = x0[lo:hi] if method == LOGW else x0
+        x, _, code, _ = p.opt_lbfgs(xs, max_iterations=k, linesearch=linesearch, past=0, epsilon=1e-12)
+        m = hi - lo if method == LOGW else n
+        return x, code, _store(p, m), p.scalars()
+
+    env = os.environ.get("BIOEN_B200_GRAPHS")
+    if toggle == "graphs":
+        os.environ["BIOEN_B200_GRAPHS"] = "1"
+    try:
+        if world > 1:
+            obj.call(lambda r, p, lo, hi: setup(p, lo, hi))
+        else:
+            setup(obj, 0, y.shape[1])
+        xs, stores = [x0], []
+        for k in range(1, 15):
+            if world > 1:
+                res = obj.call(lambda r, p, lo, hi: run(p, lo, hi, k) if method == LOGW else run(p, 0, n, k))
+                for o in res[1:]:     # (the evaluations leave rank-local partial sums in other slots)
+                    assert o[3][LBFGS_SLOTS].tobytes() == res[0][3][LBFGS_SLOTS].tobytes(), "ranks disagree"
+                x = np.concatenate([o[0] for o in res])
+                code, sc = res[0][1], res[0][3]
+                st = {key: np.concatenate([o[2][key] for o in res], axis=-1) for key in res[0][2]}
+            else:
+                x, code, st, sc = run(obj, 0, y.shape[1], k)
+            if code != MAXIMUMITERATION:
+                break                                  # stopped before k iterations: no k-iteration state to check
+            # the run of k - 1 iterations is a bitwise prefix of this one
+            assert np.array_equal(st["xp"], xs[k - 1]), ("xp is not x_{k-1}", k)
+            if k >= 2:
+                new = (k - 2) % M
+                assert np.array_equal(st["S"][new], xs[k - 1] - xs[k - 2]), ("newest pair", k)
+                prev = stores[-1]
+                for t in range(min(M, k - 2)):
+                    slot = (k - 3 - t) % M
+                    if slot != new:
+                        assert np.array_equal(st["S"][slot], prev["S"][slot]) and \
+                            np.array_equal(st["Y"][slot], prev["Y"][slot]), ("older pair changed", k, slot)
+                ref = _driver_ref(st, sc, k, toggle == "gram")
+                r = T.ratio(st["d"], ref["d"], ref["s_d"])
+                _record(("driver", "gram" if toggle == "gram" else "vector"), "benign", r)
+                assert r <= C, (k, r)
+            xs.append(x)
+            stores.append(st)
+        assert len(xs) >= 4, "fewer than three iterations ran"
+    finally:
+        if env is None:
+            os.environ.pop("BIOEN_B200_GRAPHS", None)
+        else:
+            os.environ["BIOEN_B200_GRAPHS"] = env
+        if world > 1:
+            obj.call(lambda r, p, lo, hi: (p.set_option(OPT_LBFGS_GRAM, 0), p.set_option(OPT_LBFGS_SMALL, 1),
+                                           p.set_option(OPT_LBFGS_SPECULATIVE, 1)))
+        else:
+            for o, v in ((OPT_LBFGS_GRAM, 0), (OPT_LBFGS_SMALL, 1), (OPT_LBFGS_SPECULATIVE, 1)):
+                obj.set_option(o, v)
+
+
+def test_zz_report():
+    """the largest |gpu - ref| / (u scale) per engine, benign regime and edge regimes (run with -s to see it)"""
+    names = {MULTI: "multi-kernel", SMALL: "small", GRAM: "Gram (own scale)", BATCHED: "batched",
+             (MULTI, "sharded"): "multi-kernel sharded", (GRAM, "sharded"): "Gram sharded (own scale)",
+             ("driver", "vector"): "driver histories", ("driver", "gram"): "driver histories, Gram"}
+    print("\nlargest |gpu - ref| / (u * scale), C = %d" % C)
+    for key, name in names.items():
+        b, e = WORST.get((key, True)), WORST.get((key, False))
+        if b is not None or e is not None:
+            print("  %-28s benign %8.3g   edge regimes %8.3g" % (name, b or 0.0, e or 0.0))
+    if GRAM_VS_VECTOR:
+        print("  Gram against the vector recursion's scale: " +
+              ", ".join("%s %.3g" % (k, v) for k, v in GRAM_VS_VECTOR.items()))
+    benign = [v for (key, is_b), v in WORST.items() if is_b]
+    if benign:
+        assert C >= 4 * max(benign), "C must be at least 4x the largest benign ratio"
