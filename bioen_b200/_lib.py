@@ -111,6 +111,7 @@ SIGNATURES = {
                                                    C.c_longlong, _ip, _ip, C.POINTER(C.c_longlong), _ip]),
     "bioen_b200_selftest_num_slots": (C.c_int, [C.c_longlong, C.c_longlong, C.c_longlong]),
     "bioen_b200_selftest_slice_plan": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_longlong, C.POINTER(C.c_longlong)]),
+    "bioen_b200_selftest_twoloop_schedule": (C.c_int, [C.c_int, C.c_int, C.c_int, _ip]),
     "bioen_b200_selftest_lbfgs_update": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _ip, _ip, _dp, _dp, _dp, _dp, _dp,
                                                    _dp, _dp, _dp, _dp]),
     "bioen_b200_nccl_unique_id": (C.c_int, [C.c_char_p]),

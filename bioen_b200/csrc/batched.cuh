@@ -411,12 +411,12 @@ __global__ void __launch_bounds__(kVecThreads) kb_pair(const BatchBufs b, const 
 struct KStep {
     signed char op[kBMaxK];        // 0 none, 1 active
     signed char init[kBMaxK];      // d = -g first
-    signed char u_kind[kBMaxK];    // 0 none, 1 S, 2 Y
+    signed char u_kind[kBMaxK];    // TL_NONE, TL_S, TL_Y (lbfgs.cuh)
     signed char u_slot[kBMaxK];
     signed char c_num[kBMaxK], c_den[kBMaxK], c2_num[kBMaxK];   // sc indices (c2 < 0: unused); csign below
     signed char csign[kBMaxK];
     signed char scale[kBMaxK];     // 1: d *= ys/yy
-    signed char v_kind[kBMaxK];    // 0 none, 1 S, 2 Y, 3 grad
+    signed char v_kind[kBMaxK];    // TL_NONE, TL_S, TL_Y, TL_G
     signed char v_slot[kBMaxK];
     signed char out[kBMaxK];
 };
@@ -430,8 +430,8 @@ __global__ void __launch_bounds__(kVecThreads) kb_twoloop(const BatchBufs b, con
     double* d = b.D + plane;
     const double* g = b.Gr + plane;
     auto hist = [&](int kind, int slot) -> const double* {
-        if (kind == 3) return g;
-        return (kind == 1 ? b.S : b.Yv) + ((size_t)slot * b.KP + k) * b.ldn;
+        if (kind == TL_G) return g;
+        return (kind == TL_S ? b.S : b.Yv) + ((size_t)slot * b.KP + k) * b.ldn;
     };
     const double* u = p.u_kind[k] ? hist(p.u_kind[k], p.u_slot[k]) : nullptr;
     const double* vv = p.v_kind[k] ? hist(p.v_kind[k], p.v_slot[k]) : nullptr;
@@ -1051,41 +1051,16 @@ class ThetaScan {
         for (int t = 0; t <= 2 * maxbound; ++t) {
             KStep st{};
             for (int q = 0; q < K; ++q) {
-                if (!upd.mask[q]) continue;
-                const int bnd = bound[q], end = (upd.slot[q] + 1) % m;   // the ring end after this update
-                if (t > 2 * bnd) continue;
-                auto js = [&](int i) { return ((end - 1 - i) % m + m) % m; };   // newest ... oldest
+                if (!upd.mask[q] || t > 2 * bound[q]) continue;
+                const TwoLoopStep s = two_loop_step(t, (upd.slot[q] + 1) % m, bound[q], m);
                 st.op[q] = 1;
-                st.c2_num[q] = -1;
-                if (t == 0) {
-                    st.init[q] = 1;
-                    st.v_kind[q] = 1; st.v_slot[q] = (signed char)js(0); st.out[q] = (signed char)(SC_ALPHA0 + js(0));
-                } else if (t <= bnd) {
-                    const int i = t - 1;
-                    st.u_kind[q] = 2; st.u_slot[q] = (signed char)js(i);
-                    st.c_num[q] = (signed char)(SC_ALPHA0 + js(i)); st.c_den[q] = (signed char)(SC_YS0 + js(i));
-                    st.csign[q] = -1;
-                    if (i + 1 < bnd) {
-                        st.v_kind[q] = 1; st.v_slot[q] = (signed char)js(i + 1);
-                        st.out[q] = (signed char)(SC_ALPHA0 + js(i + 1));
-                    } else {
-                        st.scale[q] = 1;
-                        st.v_kind[q] = 2; st.v_slot[q] = (signed char)js(i); st.out[q] = (signed char)SC_BETA;
-                    }
-                } else {
-                    const int i = bnd - (t - bnd);          // bnd-1 ... 0
-                    const int which = (t - bnd - 1) & 1;     // beta slots alternate
-                    st.u_kind[q] = 1; st.u_slot[q] = (signed char)js(i);
-                    st.c_num[q] = (signed char)(SC_ALPHA0 + js(i)); st.c_den[q] = (signed char)(SC_YS0 + js(i));
-                    st.csign[q] = 1;
-                    st.c2_num[q] = (signed char)(which ? SC_BETA2 : SC_BETA);
-                    if (i > 0) {
-                        st.v_kind[q] = 2; st.v_slot[q] = (signed char)js(i - 1);
-                        st.out[q] = (signed char)(which ? SC_BETA : SC_BETA2);
-                    } else {
-                        st.v_kind[q] = 3; st.out[q] = (signed char)SC_DGINIT;
-                    }
-                }
+                st.init[q] = (signed char)s.init;
+                st.u_kind[q] = (signed char)s.u_kind; st.u_slot[q] = (signed char)s.u_slot;
+                st.c_num[q] = (signed char)s.c_num; st.c_den[q] = (signed char)s.c_den; st.c2_num[q] = (signed char)s.c2_num;
+                st.csign[q] = (signed char)s.csign;
+                st.scale[q] = (signed char)s.scale;
+                st.v_kind[q] = (signed char)s.v_kind; st.v_slot[q] = (signed char)s.v_slot;
+                st.out[q] = (signed char)s.out;
             }
             kb_twoloop<<<gridv, kVecThreads, 0, C.stream>>>(B, st);
             if (reduce && !forces) {
@@ -1109,16 +1084,8 @@ class ThetaScan {
             return res;
         }
         started = true;
-        const int m = prm.m;
-        struct P {
-            int state = 0;   // 1 active, 0 done
-            int k = 1, end = 0;
-            double fx = 0, step = 0;
-            bool slope_known = false;
-            LineSearchState ls;
-            std::vector<double> pf;
-        };
-        std::vector<P> ps(K);
+        std::vector<LbfgsIteration> ps(K);
+        std::vector<char> active(K, 0);
         KVec kv{};
         for (int q = 0; q < KP; ++q) { kv.mask[q] = q < K; kv.theta[q] = q < K ? thetas[q] : 0.0; kv.stp[q] = 0.0; }
         for (int q = 0; q < K; ++q)
@@ -1129,29 +1096,21 @@ class ThetaScan {
         evaluate(kv, false);
         fetch();
         for (int q = 0; q < K; ++q) {
-            P& p = ps[q];
-            const double* h = hs(q);
-            p.fx = h[SC_F];
             ++res[q].evaluations;
-            if (prm.past > 0) { p.pf.assign(prm.past, 0.0); p.pf[0] = p.fx; }
-            double xnorm = std::sqrt(h[SC_XNORM2]), gnorm = std::sqrt(h[SC_GNORM2]);
-            if (xnorm < 1.0) xnorm = 1.0;
-            if (gnorm / xnorm <= prm.epsilon) { res[q].code = LBFGS_ALREADY_MINIMIZED; p.state = 0; kv.mask[q] = 0; continue; }
-            p.state = 1;
-            p.step = 1.0 / gnorm;
-            p.ls.start(prm, p.fx, -h[SC_GNORM2], p.step);
-            p.slope_known = true;
+            res[q].code = ps[q].first_point(prm, hs(q));
+            active[q] = res[q].code == 0;
+            kv.mask[q] = active[q];
         }
         kb_scale_copy<<<gridv, kVecThreads, 0, C.stream>>>(n, ldn, B.Gr, B.D, -1.0, kv);
         kb_scale_copy<<<gridv, kVecThreads, 0, C.stream>>>(n, ldn, B.X, B.XP, 1.0, kv);
         kb_scale_copy<<<gridv, kVecThreads, 0, C.stream>>>(n, ldn, B.Gr, B.GP, 1.0, kv);
 
-        auto any_active = [&] { for (auto& p : ps) if (p.state) return true; return false; };
+        auto any_active = [&] { for (char a : active) if (a) return true; return false; };
         while (any_active()) {
             ++rounds;
             for (int q = 0; q < K; ++q) {
-                kv.mask[q] = ps[q].state;
-                if (ps[q].state) kv.stp[q] = ps[q].ls.prepare();
+                kv.mask[q] = active[q];
+                if (active[q]) kv.stp[q] = ps[q].ls.prepare();
             }
             evaluate(kv, true);
             fetch();
@@ -1160,12 +1119,12 @@ class ThetaScan {
             bool any_upd = false, any_rev = false;
             std::vector<int> bound(K, 0);
             for (int q = 0; q < K; ++q) {
-                P& p = ps[q];
-                if (!p.state) continue;
+                if (!active[q]) continue;
+                LbfgsIteration& p = ps[q];
                 const double* h = hs(q);
                 ++res[q].evaluations;
                 int verdict;
-                if (!p.slope_known) {
+                if (!p.slope_known) {   // the first trial of a search brings the slope of its direction
                     p.slope_known = true;
                     p.ls.set_slope(h[SC_DGINIT]);
                     if (0 < h[SC_DGINIT]) verdict = LBFGSERR_INCREASEGRADIENT;
@@ -1174,41 +1133,20 @@ class ThetaScan {
                     verdict = p.ls.update(h[SC_F], h[SC_DG]);
                 }
                 if (verdict == 0) continue;   // next trial of the same search
-                // liblbfgs keeps the last trial's f in fx even when the search fails (lbfgs.c:466-481)
-                p.fx = h[SC_F];
+                int slot = 0;
+                const bool more = p.search_finished(verdict, h, slot, bound[q], res[q].code);
+                res[q].iterations = p.iterations;
+                if (more) {
+                    upd.mask[q] = 1;
+                    upd.slot[q] = slot;
+                    any_upd = true;
+                    continue;
+                }
+                active[q] = 0;
                 if (verdict < 0) {
-                    res[q].code = verdict;
-                    p.state = 0;
                     revert.mask[q] = 1;
                     any_rev = true;
-                    continue;
                 }
-                double xnorm = std::sqrt(h[SC_XNORM2]);
-                const double gnorm = std::sqrt(h[SC_GNORM2]);
-                ++res[q].iterations;
-                if (xnorm < 1.0) xnorm = 1.0;
-                if (gnorm / xnorm <= prm.epsilon) { res[q].code = LBFGS_SUCCESS; p.state = 0; continue; }
-                if (prm.past > 0) {
-                    if (prm.past <= p.k) {
-                        const double rate = (p.pf[p.k % prm.past] - p.fx) / p.fx;
-                        if (rate < prm.delta) { res[q].code = LBFGS_STOP; p.state = 0; continue; }
-                    }
-                    p.pf[p.k % prm.past] = p.fx;
-                }
-                if (prm.max_iterations != 0 && prm.max_iterations < p.k + 1) {
-                    res[q].code = LBFGSERR_MAXIMUMITERATION;
-                    p.state = 0;
-                    continue;
-                }
-                upd.mask[q] = 1;
-                upd.slot[q] = p.end;
-                any_upd = true;
-                bound[q] = (m <= p.k) ? m : p.k;
-                ++p.k;
-                p.end = (p.end + 1) % m;
-                p.step = 1.0;
-                p.slope_known = false;
-                p.ls.start(prm, p.fx, 0.0, 1.0);
             }
             if (any_rev) {
                 kb_scale_copy<<<gridv, kVecThreads, 0, C.stream>>>(n, ldn, B.XP, B.X, 1.0, revert);

@@ -509,9 +509,6 @@ static int run_lbfgs_dev(bioen_b200_ctx* ctx, int method, double* x_dev, lbfgs_c
         info[2] = opt.stats.gradients_skipped;   // of those evaluations: objective only (one pass over Y)
         info[3] = 0;
     }
-    if (opt.use_graphs && getenv("BIOEN_B200_GRAPH_TRACE"))
-        fprintf(stderr, "[bioen_b200 graphs] %.4f s wall, %d evals: host time inside cudaGraphLaunch %.2f ms, waiting %.2f ms\n",
-                secs, opt.stats.evaluations, opt.stats.gpu_eval_ms, 1e3 * opt.stats.host_wait_s);
     if (opt.trace)
         fprintf(stderr, "[bioen_b200 trace] lbfgs %.3f s wall: %d evals, GPU eval %.1f ms, GPU update+idle %.1f ms\n",
                 secs, opt.stats.evaluations, opt.stats.gpu_eval_ms, opt.stats.gpu_update_ms);
@@ -858,6 +855,18 @@ int bioen_b200_selftest_slice_plan(int m, int n, int sms, long long max_dyn_smem
     out[0] = p.nc; out[1] = p.ncs; out[2] = p.ms; out[3] = p.grid;
     out[4] = p.cx_log2; out[5] = p.l_log2; out[6] = p.lt_log2; out[7] = (long long)p.smem;
     return p.ok ? 1 : 0;
+}
+
+// host-only: the 2*bound+1 steps of the two-loop schedule (lbfgs.cuh, two_loop_step), 11 ints each
+int bioen_b200_selftest_twoloop_schedule(int end, int bound, int m, int* steps) {
+    if (m < 1 || m > 16 || bound < 1 || bound > m || end < 0 || end >= m) return -1;
+    for (int t = 0; t <= 2 * bound; ++t) {
+        const TwoLoopStep s = two_loop_step(t, end, bound, m);
+        const int v[11] = {s.init, s.u_kind, s.u_slot, s.v_kind, s.v_slot, s.c_num, s.c_den, s.csign, s.c2_num, s.scale,
+                           s.out};
+        for (int i = 0; i < 11; ++i) steps[11 * t + i] = v[i];
+    }
+    return 2 * bound + 1;
 }
 
 // One L-BFGS direction update from a given state, on the engine the minimisers would run it on (tests compare it with

@@ -72,7 +72,7 @@ struct NcclApi {
 // ---- peer-memory exchange ---------------------------------------------------------------------------------
 // Region owned by each rank (one cudaMalloc, mapped by every peer):
 //   [0, 128)    flags[src]  last epoch whose contribution rank `src` has delivered here (monotonic)
-//   [128, 136)  epoch       this rank's exchange counter (device side, so captured graphs replay correctly)
+//   [128, 136)  epoch       this rank's exchange counter (device side)
 //   [256, ...)  inbox[2][nranks][cap] doubles, indexed by epoch parity and source rank
 // Parity double buffering is enough: a rank can start exchange e+2 only after every peer has published e+1,
 // i.e. after every peer has finished reading exchange e.

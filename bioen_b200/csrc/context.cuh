@@ -135,7 +135,6 @@ class Context {
     int slice_mode = -1;                   // BIOEN_B200_OPT_SLICE: -1 / 1 on when the problem is eligible, 0 off
     long long slice_launches = 0;
     double* h_sc = nullptr;  // pinned
-    double* h_stp = nullptr; // pinned: step length of the next graph-replayed trial
 
     // structure-major copy + geometry of the fused two-pass forces kernels (fused_pass.cuh)
     DevBuf<double> Yt, fpart, flse;
@@ -211,8 +210,7 @@ class Context {
         ticket.alloc(4);
         lse_all.alloc(2 * 64);
         CUDA_CHECK(cudaHostAlloc(&h_sc, (SC_COUNT + 8) * sizeof(double), cudaHostAllocDefault));
-        memset(h_sc, 0, (SC_COUNT + 8) * sizeof(double));   // [SC_COUNT] step length, [SC_COUNT + 1] fetch sequence number
-        h_stp = h_sc + SC_COUNT;
+        memset(h_sc, 0, (SC_COUNT + 8) * sizeof(double));   // [SC_COUNT + 1] fetch sequence number
         CUDA_CHECK(cudaFuncSetAttribute(stream_pass_kernel<kRowPass, false>,
                                         cudaFuncAttributeMaxDynamicSharedMemorySize, kPassSmemBytes));
         CUDA_CHECK(cudaFuncSetAttribute(stream_pass_kernel<kRowPass, true>,
@@ -756,10 +754,10 @@ class Context {
         ++kernels_launched;
         if (nranks > 1) comm->allreduce_sum(msum.p, M + ntail, stream);
     }
-    void forces_eval_fused_f(double* x, const double* xp, const double* d, double stp, const double* stp_dev) {
+    void forces_eval_fused_f(double* x, const double* xp, const double* d, double stp) {
         NvtxRange nvtx("bioen:forces_eval_f(fused)");
         {
-            ForcesUpdateArgs a{M, x, xp, d, stp, ab.p, sc.p, stp_dev};
+            ForcesUpdateArgs a{M, x, xp, d, stp, ab.p, sc.p};
             k_forces_update<<<1, 1024, 0, stream>>>(a);
             ++kernels_launched;
         }
@@ -848,10 +846,9 @@ class Context {
     // ---- kernel launch helpers ---------------------------------------------------------------------
     const double* lse_pairs() const { return nranks > 1 ? lse_all.p : sc.p + SC_LSE_MAX; }
 
-    void launch_lse(double* x, const double* xp, const double* d, double stp, const double* w0, bool from_col,
-                    const double* stp_dev = nullptr) {
+    void launch_lse(double* x, const double* xp, const double* d, double stp, const double* w0, bool from_col) {
         LseArgs a{};
-        a.n = N; a.x = x; a.xp = xp; a.d = d; a.stp = stp; a.stp_dev = stp_dev; a.w0 = w0;
+        a.n = N; a.x = x; a.xp = xp; a.d = d; a.stp = stp; a.w0 = w0;
         a.col_partial = from_col ? partialB.p : nullptr;
         a.col_ld = Npad; a.col_L = nRT; a.col_chunk = col_chunk();
         a.write_xnorm = from_col ? 0 : 1;
@@ -947,13 +944,13 @@ class Context {
                !storage_fp32 && (ld % 2) == 0 && ld >= N && (reinterpret_cast<uintptr_t>(Y) & 15) == 0;
     }
     void launch_slice(int method, int mode, double* x, const double* xp, const double* d, double stp,
-                      const double* stp_dev, double* grad, const double* ddir) {
+                      double* grad, const double* ddir) {
         SliceArgs a{};
         a.method = method; a.mode = mode; a.M = M; a.N = N;
         a.nc = slice_pl.nc; a.ncs = slice_pl.ncs; a.ms = slice_pl.ms;
         a.cx_log2 = slice_pl.cx_log2; a.l_log2 = slice_pl.l_log2; a.lt_log2 = slice_pl.lt_log2;
         a.Y = Y; a.ld = ld;
-        a.x = x; a.xp = xp; a.d = d; a.stp = stp; a.stp_dev = stp_dev;
+        a.x = x; a.xp = xp; a.d = d; a.stp = stp;
         a.Gv = Gv.p; a.w = w.p; a.aux_n = aux_n.p; a.aux_n2 = aux_n2.p; a.grad = grad; a.ddir = ddir;
         a.Yobs = Yobs.p; a.ab = ab.p; a.avg = avg.p; a.theta = theta; a.sc = sc.p;
         a.tab = slice_tab.p; a.gtab = slice_gtab.p; a.part = slice_part.p; a.bar = pe_bar.p; a.ticket = ticket.p;
@@ -992,10 +989,10 @@ class Context {
         return true;
     }
     void launch_persistent(int method, int mode, double* x, const double* xp, const double* d, double stp,
-                           const double* stp_dev, double* grad, const double* ddir) {
+                           double* grad, const double* ddir) {
         if (!has_matrix()) throw std::logic_error("bioen_b200: yTilde has not been uploaded");
         if (slice_ok()) {
-            launch_slice(method, mode, x, xp, d, stp, stp_dev, grad, ddir);
+            launch_slice(method, mode, x, xp, d, stp, grad, ddir);
             return;
         }
         PEvalArgs a{};
@@ -1011,7 +1008,7 @@ class Context {
             a.col.interleave = 1;
             a.col.chunk = nRT;
         }
-        a.x = x; a.xp = xp; a.d = d; a.stp = stp; a.stp_dev = stp_dev;
+        a.x = x; a.xp = xp; a.d = d; a.stp = stp;
         a.Gv = Gv.p; a.w = w.p; a.aux_n = aux_n.p; a.aux_n2 = aux_n2.p; a.grad = grad; a.ddir = ddir;
         a.Yobs = Yobs.p; a.ab = ab.p; a.avg = avg.p; a.msum = msum.p; a.theta = theta; a.sc = sc.p;
         a.part = pe_part.p; a.bar = pe_bar.p; a.ticket = ticket.p;
@@ -1072,29 +1069,28 @@ class Context {
     // skip or defer the second pass over Y).  eval_gen changes with every objective evaluation.
     long long eval_gen = 0;
     bool lazy_gradient = true;   // BIOEN_B200_OPT_LAZY_GRADIENT: minimisers may use the split (results identical)
-    void logw_eval(double* x, const double* xp, const double* d, double stp, double* grad, const double* ddir,
-                   const double* stp_dev = nullptr) {
+    void logw_eval(double* x, const double* xp, const double* d, double stp, double* grad, const double* ddir) {
         if (grad && persistent_for(false)) {
             NvtxRange nvtx("bioen:logw_eval(persistent)");
             if (!have_logw) throw std::logic_error("bioen_b200: log-weights data not set");
             ++eval_gen;
-            launch_persistent(0, kPEvalBoth, x, xp, d, stp, stp_dev, grad, ddir);
+            launch_persistent(0, kPEvalBoth, x, xp, d, stp, grad, ddir);
             eval_fused = false;
             return;
         }
-        logw_eval_f(x, xp, d, stp, stp_dev);
+        logw_eval_f(x, xp, d, stp);
         if (grad) logw_eval_g(x, grad, ddir);
     }
-    void logw_eval_f(double* x, const double* xp, const double* d, double stp, const double* stp_dev = nullptr) {
+    void logw_eval_f(double* x, const double* xp, const double* d, double stp) {
         NvtxRange nvtx("bioen:logw_eval_f");
         if (!have_logw) throw std::logic_error("bioen_b200: log-weights data not set");
         ++eval_gen;
         if (persistent_for(false)) {
-            launch_persistent(0, kPEvalObjective, x, xp, d, stp, stp_dev, nullptr, nullptr);
+            launch_persistent(0, kPEvalObjective, x, xp, d, stp, nullptr, nullptr);
             eval_fused = nranks > 1;
             return;
         }
-        launch_lse(x, xp, d, stp, nullptr, false, stp_dev);
+        launch_lse(x, xp, d, stp, nullptr, false);
         const bool fused = fuse_exchange();
         eval_fused = fused;
         if (!fused) gather_lse();
@@ -1125,7 +1121,7 @@ class Context {
     void logw_eval_g(const double* x, double* grad, const double* ddir) {
         NvtxRange nvtx("bioen:logw_eval_g");
         if (persistent_for(false) && (nranks == 1 || eval_fused)) {
-            launch_persistent(0, kPEvalGradient, const_cast<double*>(x), nullptr, nullptr, 0.0, nullptr, grad, ddir);
+            launch_persistent(0, kPEvalGradient, const_cast<double*>(x), nullptr, nullptr, 0.0, grad, ddir);
             eval_fused = false;
             return;
         }
@@ -1186,34 +1182,33 @@ class Context {
     // ---- forces evaluation (c_bioen_kernels_forces.c:43-76) ----------------------------------------------
     // x (device, M): forces; formed as xp + stp*d when xp != nullptr.  The M-dimensional state is replicated
     // on every rank.  grad == nullptr -> objective only (two passes over Y).
-    void forces_eval(double* x, const double* xp, const double* d, double stp, double* grad, const double* ddir,
-                     const double* stp_dev = nullptr) {
+    void forces_eval(double* x, const double* xp, const double* d, double stp, double* grad, const double* ddir) {
         if (grad && have_forces && persistent_for(true)) {
             NvtxRange nvtx("bioen:forces_eval(persistent)");
             ++eval_gen;
             forces_x = x;
-            launch_persistent(1, kPEvalBoth, x, xp, d, stp, stp_dev, grad, ddir);
+            launch_persistent(1, kPEvalBoth, x, xp, d, stp, grad, ddir);
             return;
         }
-        forces_eval_f(x, xp, d, stp, stp_dev);
+        forces_eval_f(x, xp, d, stp);
         if (grad) forces_eval_g(grad, ddir);
     }
     double* forces_x = nullptr;   // the forces vector of the last objective half (persistent gradient half)
     bool forces_fused_now() const { return fused_ready && (allow_fused || yt_only); }
-    void forces_eval_f(double* x, const double* xp, const double* d, double stp, const double* stp_dev = nullptr) {
+    void forces_eval_f(double* x, const double* xp, const double* d, double stp) {
         if (!have_forces) throw std::logic_error("bioen_b200: forces data not set");
         ++eval_gen;
         if (forces_fused_now() && !slice_ok()) {
-            forces_eval_fused_f(x, xp, d, stp, stp_dev);
+            forces_eval_fused_f(x, xp, d, stp);
             return;
         }
         if (persistent_for(true)) {
             forces_x = x;
-            launch_persistent(1, kPEvalObjective, x, xp, d, stp, stp_dev, nullptr, nullptr);
+            launch_persistent(1, kPEvalObjective, x, xp, d, stp, nullptr, nullptr);
             return;
         }
         {
-            ForcesUpdateArgs a{M, x, xp, d, stp, ab.p, sc.p, stp_dev};
+            ForcesUpdateArgs a{M, x, xp, d, stp, ab.p, sc.p};
             k_forces_update<<<1, 1024, 0, stream>>>(a);
             ++kernels_launched;
         }
@@ -1238,7 +1233,7 @@ class Context {
             return;
         }
         if (persistent_for(true)) {
-            launch_persistent(1, kPEvalGradient, forces_x, nullptr, nullptr, 0.0, nullptr, grad, ddir);
+            launch_persistent(1, kPEvalGradient, forces_x, nullptr, nullptr, 0.0, grad, ddir);
             return;
         }
         launch_pass<kColPass, false>(nullptr, nullptr);                 // t_j = sum_i y_ij r_i
@@ -1272,7 +1267,7 @@ class Context {
             return;
         }
         ++eval_gen;
-        ForcesUpdateArgs u{M, x, nullptr, nullptr, 0.0, ab.p, sc.p, nullptr};
+        ForcesUpdateArgs u{M, x, nullptr, nullptr, 0.0, ab.p, sc.p};
         k_forces_update<<<1, 1024, 0, stream>>>(u);
         launch_pass<kColPass, false>(nullptr, nullptr);
         launch_lse(aux_n.p, nullptr, nullptr, 0.0, Gv.p, true);

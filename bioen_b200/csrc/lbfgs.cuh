@@ -13,10 +13,9 @@
 // With N sharded across GPUs the vector kernels see the local slice and the raw dot products are
 // all-reduced in-stream (forces: the M-dimensional state is replicated, nothing to reduce).
 #pragma once
-#include <chrono>
 #include <cmath>
 #include <cstdio>
-#include <map>
+#include <vector>
 
 #include "context.cuh"
 
@@ -74,7 +73,7 @@ struct LbfgsStats {
     int iterations = 0, evaluations = 0;
     int gradients_skipped = 0;   // trials whose gradient pass was not needed (sufficient-decrease test failed)
     double seconds = 0.0;
-    double gpu_eval_ms = 0.0, gpu_update_ms = 0.0, host_wait_s = 0.0;   // BIOEN_B200_TRACE=1
+    double gpu_eval_ms = 0.0, gpu_update_ms = 0.0;   // BIOEN_B200_TRACE=1
 };
 
 inline int lbfgs_check_params(int n, const LbfgsParams& p) {  // lbfgs.c:286-364
@@ -267,6 +266,126 @@ struct LineSearchState {
     }
 };
 
+// ------------------------------------------------------------------------------------------------
+// liblbfgs' iteration loop for one problem (lbfgs.c:412-598 without the vector arithmetic): the stop tests in their
+// order, the `past` ring of objective values and the position in the (s, y) ring.  Lbfgs::run drives one problem with
+// it, ThetaScan::run (batched.cuh) K problems in lockstep; each enqueues its own trials, updates and reverts.
+// ------------------------------------------------------------------------------------------------
+struct LbfgsIteration {
+    const LbfgsParams* prm = nullptr;
+    int k = 1, end = 0, iterations = 0;
+    double fx = 0.0;
+    std::vector<double> pf;     // objective of the last `past` iterations
+    LineSearchState ls;         // the running search
+    bool slope_known = false;   // false: ls waits for the slope g.d of the new direction (ls.set_slope)
+
+    // h: scalar file of the start point.  0: the first search is started (d = -g, step 1/||g||, slope -||g||^2);
+    // otherwise LBFGS_ALREADY_MINIMIZED.
+    int first_point(const LbfgsParams& p, const double* h) {
+        prm = &p;
+        fx = h[SC_F];
+        pf.assign(p.past > 0 ? p.past : 0, 0.0);
+        if (!pf.empty()) pf[0] = fx;
+        double xnorm = std::sqrt(h[SC_XNORM2]);
+        const double gnorm = std::sqrt(h[SC_GNORM2]);
+        if (xnorm < 1.0) xnorm = 1.0;
+        if (gnorm / xnorm <= p.epsilon) return LBFGS_ALREADY_MINIMIZED;
+        ls.start(p, fx, -h[SC_GNORM2], 1.0 / gnorm);
+        slope_known = true;
+        return 0;
+    }
+
+    // the search ended with `verdict` (!= 0); h: scalar file of its last trial.  true: the new pair goes to ring slot
+    // `slot`, the two-loop recursion runs over `bound` pairs, and the next search is started with step 1 and an
+    // unknown slope.  false: the minimisation ends with the liblbfgs code `code`; on a failed search (verdict < 0) the
+    // caller reverts x and g.
+    bool search_finished(int verdict, const double* h, int& slot, int& bound, int& code) {
+        // a failed search leaves its last trial's f in fx (lbfgs.c:466-481), except on a positive initial slope,
+        // where liblbfgs returns before the first trial
+        if (verdict != LBFGSERR_INCREASEGRADIENT) fx = h[SC_F];
+        code = verdict;
+        if (verdict < 0) return false;
+        ++iterations;   // the progress callback (c_bioen_kernels_logw.c:565-576)
+        double xnorm = std::sqrt(h[SC_XNORM2]);
+        const double gnorm = std::sqrt(h[SC_GNORM2]);
+        if (xnorm < 1.0) xnorm = 1.0;
+        if (gnorm / xnorm <= prm->epsilon) {
+            code = LBFGS_SUCCESS;
+            return false;
+        }
+        if (!pf.empty()) {
+            if (prm->past <= k && (pf[k % prm->past] - fx) / fx < prm->delta) {
+                code = LBFGS_STOP;
+                return false;
+            }
+            pf[k % prm->past] = fx;
+        }
+        if (prm->max_iterations != 0 && prm->max_iterations < k + 1) {
+            code = LBFGSERR_MAXIMUMITERATION;
+            return false;
+        }
+        code = 0;
+        slot = end;
+        bound = (prm->m <= k) ? prm->m : k;
+        ++k;
+        end = (end + 1) % prm->m;
+        ls.start(*prm, fx, 0.0, 1.0);
+        slope_known = false;
+        return true;
+    }
+};
+
+// ------------------------------------------------------------------------------------------------
+// The two-loop recursion of lbfgs.c:572-598 over the `bound` newest pairs of an m-slot ring whose newest pair sits in
+// slot end - 1, as 2*bound + 1 fused steps (k_lbfgs_twoloop, kb_twoloop).  Step t does
+//     d <- (init ? -g : d) + coef * u ;  d *= sc[SC_YS] / sc[SC_YY] when scale ;  sc[out] = v . d
+// with coef = csign * sc[c_num] / sc[c_den], minus sc[c2_num] / sc[c_den] when c2_num >= 0.  The alpha ring holds the
+// raw s_j . d, SC_BETA / SC_BETA2 alternately the raw y_j . d; the last step leaves g . d in SC_DGINIT.
+// ------------------------------------------------------------------------------------------------
+enum { TL_NONE = 0, TL_S = 1, TL_Y = 2, TL_G = 3 };   // a step's vectors: none, s_slot, y_slot, the gradient
+
+struct TwoLoopStep {
+    int init;
+    int u_kind, u_slot;       // u_kind TL_NONE: no axpy
+    int v_kind, v_slot;       // v_kind TL_NONE: no dot
+    int c_num, c_den, csign;
+    int c2_num;               // -1: unused
+    int scale;
+    int out;
+};
+
+inline TwoLoopStep two_loop_step(int t, int end, int bound, int m) {
+    auto js = [&](int i) { return ((end - 1 - i) % m + m) % m; };   // newest ... oldest
+    TwoLoopStep st{};
+    st.c2_num = -1;
+    if (t == 0) {                   // d = -g ; alpha_raw[j0] = s_j0 . d
+        st.init = 1;
+        st.v_kind = TL_S; st.v_slot = js(0); st.out = SC_ALPHA0 + js(0);
+    } else if (t <= bound) {        // d -= alpha_j y_j ; then either the next alpha, or (last) the H0 scaling and the first beta
+        const int i = t - 1;
+        st.u_kind = TL_Y; st.u_slot = js(i);
+        st.c_num = SC_ALPHA0 + js(i); st.c_den = SC_YS0 + js(i); st.csign = -1;
+        if (i + 1 < bound) {
+            st.v_kind = TL_S; st.v_slot = js(i + 1); st.out = SC_ALPHA0 + js(i + 1);
+        } else {
+            st.scale = 1;
+            st.v_kind = TL_Y; st.v_slot = js(i); st.out = SC_BETA;
+        }
+    } else {                        // d += (alpha_j - beta_j) s_j ; then the next beta, or (last) g.d
+        const int i = 2 * bound - t;              // bound-1 ... 0
+        const bool odd = (t - bound - 1) & 1;     // the beta slots alternate
+        st.u_kind = TL_S; st.u_slot = js(i);
+        st.c_num = SC_ALPHA0 + js(i); st.c_den = SC_YS0 + js(i); st.csign = 1;
+        st.c2_num = odd ? SC_BETA2 : SC_BETA;
+        if (i > 0) {
+            st.v_kind = TL_Y; st.v_slot = js(i - 1); st.out = odd ? SC_BETA : SC_BETA2;
+        } else {
+            st.v_kind = TL_G; st.out = SC_DGINIT;
+        }
+    }
+    return st;
+}
+
 class Lbfgs {
    public:
     Context& C;
@@ -277,18 +396,7 @@ class Lbfgs {
     LbfgsStats stats;
     bool trace = false;                                   // BIOEN_B200_TRACE: GPU time of evaluations vs updates
     cudaEvent_t tev[3] = {nullptr, nullptr, nullptr};
-    // CUDA graphs (single-GPU runs): one graph replays a whole line-search trial (step length H2D, the
-    // evaluation kernels, scalar file D2H), one graph per (ring slot, history length) replays the L-BFGS update
-    // (pair kernel + two-loop recursion): ~20 launches per iteration become 2.  Results are identical (the GPU
-    // test-suite passes with it), but on this driver the replays cost ~1 ms each, so it is opt-in:
-    // BIOEN_B200_GRAPHS=1.
-    bool use_graphs = false;
-    cudaGraphExec_t g_trial = nullptr;
-    long long g_trial_kernels = 0;
-    std::map<int, std::pair<cudaGraphExec_t, long long>> g_update;
     ~Lbfgs() {
-        if (g_trial) cudaGraphExecDestroy(g_trial);
-        for (auto& kv : g_update) cudaGraphExecDestroy(kv.second.first);
         for (auto& e : tev) if (e) cudaEventDestroy(e);
     }
 
@@ -308,71 +416,39 @@ class Lbfgs {
         NvtxRange nvtx("bioen:lbfgs");
         x = x_dev;
         trace = getenv("BIOEN_B200_TRACE") != nullptr;
-        {
-            // opt-in: measured on B200 / driver 580 the replays are SLOWER than plain launches here (config 1,
-            // N=1e5 x M=500: 0.73 s vs 0.12 s to the optimum, i.e. ~1 ms per cudaGraphLaunch of these graphs)
-            const char* e = getenv("BIOEN_B200_GRAPHS");
-            use_graphs = C.nranks == 1 && !trace && (e && e[0] == '1');
-        }
         int ret = lbfgs_check_params(n, prm);
         if (ret) { *fx_out = 0.0; return ret; }
-        const int m = prm.m;
         bind_store();
-        std::vector<double> pf(prm.past > 0 ? prm.past : 0);
         const double* h = C.h_sc;
 
         // initial evaluation (lbfgs.c:412)
         eval(nullptr, nullptr, 0.0, nullptr);
         C.fetch_scalars();
-        double fx = h[SC_F];
-        if (!pf.empty()) pf[0] = fx;
-        double xnorm = std::sqrt(h[SC_XNORM2]), gnorm = std::sqrt(h[SC_GNORM2]);
-        if (xnorm < 1.0) xnorm = 1.0;
-        if (gnorm / xnorm <= prm.epsilon) { *fx_out = fx; return LBFGS_ALREADY_MINIMIZED; }
-        // d = -g ; step = 1/||d|| ; dginit = g.d = -||g||^2
-        k_axpby<<<vec_blocks, kVecThreads, 0, C.stream>>>(n, -1.0, g, 0.0, nullptr, d);
-        double step = 1.0 / gnorm;
-        double dginit = -h[SC_GNORM2];
-        bool dginit_known = true;
+        LbfgsIteration it;
+        ret = it.first_point(prm, h);
+        if (ret) { *fx_out = it.fx; return ret; }
+        k_axpby<<<vec_blocks, kVecThreads, 0, C.stream>>>(n, -1.0, g, 0.0, nullptr, d);   // d = -g
         C.d2d(xp, x, n);
         C.d2d(gp, g, n);
 
-        int k = 1, end = 0;
         for (;;) {
             NvtxRange nvtx_it("bioen:lbfgs_iteration");
-            int ls = linesearch(fx, step, dginit, dginit_known);
-            if (ls < 0) {
+            const int verdict = linesearch(it);
+            int slot = 0, bound = 0;
+            const bool more = it.search_finished(verdict, h, slot, bound, ret);
+            stats.iterations = it.iterations;
+            if (verdict > 0 && verbose && it.iterations % 1000 == 0) printf("\t\tOpt Iteration %d\n", it.iterations);
+            if (verdict < 0) {
                 // revert to the previous point (lbfgs.c:475-481)
                 C.d2d(x, xp, n);
                 C.d2d(g, gp, n);
                 C.sync();
-                ret = ls;
-                break;
             }
-            xnorm = std::sqrt(h[SC_XNORM2]);
-            gnorm = std::sqrt(h[SC_GNORM2]);
-            ++stats.iterations;  // progress callback (c_bioen_kernels_logw.c:565-576)
-            if (verbose && stats.iterations % 1000 == 0) printf("\t\tOpt Iteration %d\n", stats.iterations);
-            if (xnorm < 1.0) xnorm = 1.0;
-            if (gnorm / xnorm <= prm.epsilon) { ret = LBFGS_SUCCESS; break; }
-            if (!pf.empty()) {
-                if (prm.past <= k) {
-                    const double rate = (pf[k % prm.past] - fx) / fx;
-                    if (rate < prm.delta) { ret = LBFGS_STOP; break; }
-                }
-                pf[k % prm.past] = fx;
-            }
-            if (prm.max_iterations != 0 && prm.max_iterations < k + 1) { ret = LBFGSERR_MAXIMUMITERATION; break; }
-
+            if (!more) break;
             // s, y, ys, yy; xp <- x, gp <- g (lbfgs.c:543-555, 462-463); then the two-loop recursion
-            const int bound = (m <= k) ? m : k;
-            update_direction(end, bound, m);
-            ++k;
-            end = (end + 1) % m;
-            step = 1.0;
-            dginit_known = false;  // sc[SC_DGINIT] is read at the start of the next line search
+            update_direction(slot, bound, prm.m);
         }
-        *fx_out = fx;
+        *fx_out = it.fx;
         return ret;
     }
 
@@ -395,35 +471,13 @@ class Lbfgs {
     }
 
     // the new pair into ring slot end_old and the two-loop recursion over `bound` pairs, on whichever engine the
-    // context selects (Gram, small, multi-kernel; CUDA graphs when enabled).  Also bioen_b200_selftest_lbfgs_update.
+    // context selects (Gram, small, multi-kernel).  Also bioen_b200_selftest_lbfgs_update.
     void update_direction(int end_old, int bound, int m) {
-        if (gram_mode()) {
-            enqueue_update_gram(end_old, bound);
-            return;
-        }
-        if (small_mode()) {
-            enqueue_update_small(end_old, bound);
-            return;
-        }
-        if (use_graphs) {
-            const int key = end_old * 64 + bound;
-            auto it = g_update.find(key);
-            if (it == g_update.end()) {
-                long long nk = 0;
-                cudaGraphExec_t ex = capture([&] { enqueue_update(end_old, bound, m); }, &nk);
-                if (!ex) {
-                    use_graphs = false;
-                    enqueue_update(end_old, bound, m);
-                    return;
-                }
-                it = g_update.emplace(key, std::make_pair(ex, nk)).first;
-            }
-            CUDA_CHECK(cudaGraphLaunch(it->second.first, C.stream));
-            C.kernels_launched += it->second.second;
-            return;
-        }
-        enqueue_update(end_old, bound, m);
+        if (gram_mode()) enqueue_update_gram(end_old, bound);
+        else if (small_mode()) enqueue_update_small(end_old, bound);
+        else enqueue_update(end_old, bound, m);
     }
+
     bool gram_mode() const {
         // sharded runs need the in-kernel exchange (the peer-memory path); m is liblbfgs' default 6
         return C.lbfgs_gram_opt && prm.m == kGramM && (!reduce || C.fuse_exchange());
@@ -480,68 +534,8 @@ class Lbfgs {
         return fetched;
     }
 
-    // ---- CUDA-graph plumbing ---------------------------------------------------------------------------
-    template <class F>
-    cudaGraphExec_t capture(F&& enqueue, long long* kernels) {
-        cudaGraph_t graph = nullptr;
-        cudaGraphExec_t exec = nullptr;
-        const long long k0 = C.kernels_launched;
-        if (cudaStreamBeginCapture(C.stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
-            cudaGetLastError();
-            return nullptr;
-        }
-        bool ok = true;
-        try {
-            enqueue();
-        } catch (...) {
-            ok = false;
-        }
-        if (cudaStreamEndCapture(C.stream, &graph) != cudaSuccess || !graph) ok = false;
-        if (ok && cudaGraphInstantiate(&exec, graph, 0) != cudaSuccess) ok = false;
-        if (graph) cudaGraphDestroy(graph);
-        *kernels = C.kernels_launched - k0;
-        C.kernels_launched = k0;          // nothing ran yet; replays are counted when launched
-        if (!ok) {
-            cudaGetLastError();
-            if (exec) cudaGraphExecDestroy(exec);
-            return nullptr;
-        }
-        return exec;
-    }
-
     // one line-search trial at x = xp + stp*d: evaluation + scalar read-back (host side of lbfgs.c:645-1001)
     void trial(double stp, const LineSearchState& ls) {
-        if (use_graphs) {
-            // BIOEN_B200_GRAPHS_NOMEMCPY=1 (diagnostics): keep the two tiny copies (step length in, scalar file out)
-            // OUTSIDE the graph, so that it holds kernel nodes only
-            static const bool nomemcpy = getenv("BIOEN_B200_GRAPHS_NOMEMCPY") != nullptr;
-            if (!g_trial) {
-                g_trial = capture([&] {
-                    if (!nomemcpy)
-                        CUDA_CHECK(cudaMemcpyAsync(C.sc.p + SC_STP, C.h_stp, sizeof(double), cudaMemcpyHostToDevice, C.stream));
-                    if (forces) C.forces_eval(x, xp, d, 0.0, g, d, C.sc.p + SC_STP);
-                    else C.logw_eval(x, xp, d, 0.0, g, d, C.sc.p + SC_STP);
-                    if (!nomemcpy) C.d2h(C.h_sc, C.sc.p, SC_COUNT);
-                }, &g_trial_kernels);
-                if (!g_trial) use_graphs = false;   // capture not possible here: plain launches from now on
-            }
-            if (g_trial) {
-                *C.h_stp = stp;
-                const auto t0 = std::chrono::steady_clock::now();
-                if (nomemcpy)
-                    CUDA_CHECK(cudaMemcpyAsync(C.sc.p + SC_STP, C.h_stp, sizeof(double), cudaMemcpyHostToDevice, C.stream));
-                CUDA_CHECK(cudaGraphLaunch(g_trial, C.stream));
-                if (nomemcpy) C.d2h(C.h_sc, C.sc.p, SC_COUNT);
-                const auto t1 = std::chrono::steady_clock::now();
-                C.kernels_launched += g_trial_kernels;
-                C.spin_sync();
-                const auto t2 = std::chrono::steady_clock::now();
-                stats.host_wait_s += std::chrono::duration<double>(t2 - t1).count();
-                stats.gpu_eval_ms += 1e3 * std::chrono::duration<double>(t1 - t0).count();   // host time in launch
-                ++stats.evaluations;
-                return;
-            }
-        }
         // More-Thuente reads the slope of every trial: plain f+g evaluation, one read-back
         // (not on the slice kernel: there a combined f+g launch costs ~4 us more than the objective alone, less than the
         // second launch and host round trip the split costs the ~87 % of trials whose gradient IS read)
@@ -601,84 +595,53 @@ class Lbfgs {
         ++C.kernels_launched;
     }
 
-    // the recursion of lbfgs.c:572-598 as 2*bound+1 fused kernels; the last one also leaves g.d in SC_DGINIT
+    // the recursion of lbfgs.c:572-598 as the 2*bound+1 fused kernels of two_loop_step
     void two_loop(int bound, int end, int m) {
         const bool fused = reduce && C.fuse_exchange();
-        auto launch = [&](TwoLoopArgs& a) {
-            a.n = n; a.d = d; a.g = g; a.partials = C.red_partials.p; a.ticket = C.ticket.p; a.sc = C.sc.p;
+        auto vec = [&](int kind, int slot) -> const double* {
+            return kind == TL_S ? S[slot] : kind == TL_Y ? Yv[slot] : kind == TL_G ? g : nullptr;
+        };
+        for (int t = 0; t <= 2 * bound; ++t) {
+            const TwoLoopStep st = two_loop_step(t, end, bound, m);
+            TwoLoopArgs a{};
+            a.n = n; a.d = d; a.g = g; a.init = st.init;
+            a.u = vec(st.u_kind, st.u_slot); a.c_num = st.c_num; a.c_den = st.c_den; a.csign = st.csign;
+            a.c2_num = st.c2_num; a.c2_den = st.c_den; a.c2sign = -1.0;
+            a.s_num = st.scale ? SC_YS : -1; a.s_den = SC_YY;
+            a.v = vec(st.v_kind, st.v_slot); a.out = st.out;
+            a.partials = C.red_partials.p; a.ticket = C.ticket.p; a.sc = C.sc.p;
             if (fused && a.v) a.p2p = C.p2p_dev(); else a.p2p.nranks = 1;
             k_lbfgs_twoloop<<<vec_blocks, kVecThreads, 0, C.stream>>>(a);
             ++C.kernels_launched;
             if (reduce && !fused && a.v) C.comm->allreduce_sum(C.sc.p + a.out, 1, C.stream);
-        };
-        std::vector<int> js(bound);
-        int j = end;
-        for (int i = 0; i < bound; ++i) { j = (j + m - 1) % m; js[i] = j; }   // newest ... oldest
-        {   // d = -g ; alpha_raw[j0] = s_j0 . d
-            TwoLoopArgs a{};
-            a.init = 1; a.u = nullptr; a.c_num = a.c_den = 0; a.c2_num = -1; a.s_num = -1;
-            a.v = S[js[0]]; a.out = SC_ALPHA0 + js[0];
-            launch(a);
-        }
-        for (int i = 0; i < bound; ++i) {
-            // d -= alpha_j y_j ; then either the next alpha, or (last) the H0 scaling and the first beta
-            TwoLoopArgs a{};
-            a.u = Yv[js[i]]; a.c_num = SC_ALPHA0 + js[i]; a.c_den = SC_YS0 + js[i]; a.csign = -1.0; a.c2_num = -1;
-            if (i + 1 < bound) {
-                a.s_num = -1; a.v = S[js[i + 1]]; a.out = SC_ALPHA0 + js[i + 1];
-            } else {
-                a.s_num = SC_YS; a.s_den = SC_YY; a.v = Yv[js[i]]; a.out = SC_BETA;
-            }
-            launch(a);
-        }
-        int beta_slot = SC_BETA;
-        for (int i = bound - 1; i >= 0; --i) {
-            // d += (alpha_j - beta_j) s_j ; then the next beta, or (last) g.d
-            TwoLoopArgs a{};
-            a.u = S[js[i]];
-            a.c_num = SC_ALPHA0 + js[i]; a.c_den = SC_YS0 + js[i]; a.csign = 1.0;
-            a.c2_num = beta_slot; a.c2_den = SC_YS0 + js[i]; a.c2sign = -1.0;
-            a.s_num = -1;
-            beta_slot = (beta_slot == SC_BETA) ? SC_BETA2 : SC_BETA;
-            if (i > 0) { a.v = Yv[js[i - 1]]; a.out = beta_slot; }
-            else { a.v = g; a.out = SC_DGINIT; }
-            launch(a);
         }
     }
 
-    // one line search (lbfgs.c:645-734 backtracking, 812-1001 More-Thuente) driven by LineSearchState: every
-    // trial is one f+g evaluation on the device and one 512-byte read-back.  On success h_sc holds the scalars
-    // of the accepted point.
-    int linesearch(double& f, double& stp, double& dginit, bool& dginit_known) {
+    // one line search (lbfgs.c:645-734 backtracking, 812-1001 More-Thuente) driven by it.ls: every trial is one f+g
+    // evaluation on the device and one 512-byte read-back.  Returns the verdict; h_sc holds the last trial's scalars.
+    int linesearch(LbfgsIteration& it) {
         const double* h = C.h_sc;
-        if (stp <= 0.) return LBFGSERR_INVALIDPARAMETERS;
         // g.d of the new direction was left in the scalar file (SC_DGINIT) by the update kernels.  The first trial
         // point xp + stp*d does not depend on it, so the trial is enqueued right behind the update and the slope
         // arrives with the trial's own scalars: one host round trip per iteration instead of two.  (The one case
         // where the slope matters beforehand -- 0 < g.d, LBFGSERR_INCREASEGRADIENT -- then costs one evaluation
         // that liblbfgs would not have made; x and g are restored by the caller as after any failed search.)
-        spec_slope = !dginit_known && !use_graphs && C.lbfgs_speculative;
-        if (!dginit_known && !spec_slope) {
+        spec_slope = !it.slope_known && C.lbfgs_speculative;
+        if (!it.slope_known && !spec_slope) {
             C.fetch_scalars();
-            dginit = h[SC_DGINIT];
-            dginit_known = true;
+            it.ls.set_slope(h[SC_DGINIT]);
+            it.slope_known = true;
         }
-        if (dginit_known && 0 < dginit) return LBFGSERR_INCREASEGRADIENT;
-        LineSearchState ls;
-        ls.start(prm, f, dginit_known ? dginit : 0.0, stp);
-        spec_ls = &ls;
+        if (it.slope_known && 0 < it.ls.dginit) return LBFGSERR_INCREASEGRADIENT;
+        spec_ls = &it.ls;
         for (;;) {
-            stp = ls.prepare();
-            trial(stp, ls);
+            trial(it.ls.prepare(), it.ls);
             if (spec_bad) {   // the slope that came with the first trial is positive
                 spec_bad = false;
-                dginit = h[SC_DGINIT];
-                dginit_known = true;
                 return LBFGSERR_INCREASEGRADIENT;
             }
-            if (!dginit_known) { dginit = ls.dginit; dginit_known = true; }
-            f = h[SC_F];
-            const int verdict = ls.update(f, h[SC_DG]);
+            it.slope_known = true;
+            const int verdict = it.ls.update(h[SC_F], h[SC_DG]);
             if (verdict != 0) return verdict;
         }
     }

@@ -43,7 +43,6 @@ struct PEvalArgs {
     const double* xp;
     const double* d;
     double stp;
-    const double* stp_dev;
     const double* Gv;    // G (logw) / w0 (forces)
     double* w;
     double* aux_n;       // forces: x_j, later E_j
@@ -95,7 +94,7 @@ __device__ __forceinline__ void peval_grid_barrier(const PEvalArgs& a, unsigned 
     __syncthreads();
     ++nbar;
     if (threadIdx.x == 0) {
-        // Sense-reversing barrier that needs no state from the host (so captured CUDA graphs replay it correctly):
+        // Sense-reversing barrier that needs no state from the host:
         // a.bar[0] counts arrivals, a.bar[16] (its own cache line) is the generation.  Every CTA reads the generation
         // BEFORE it arrives; the CTA that completes the count resets it and publishes generation + 1; the others poll
         // the generation word, so the spinning loads do not contend with the arriving atomics.
@@ -213,7 +212,6 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
     double* mypart = a.part + (size_t)b * kPSlots;
     int mk = 0;
     peval_mark(a, mk);
-    const double stp = a.stp_dev ? __ldg(a.stp_dev) : a.stp;
     const bool sharded = a.p2p.nranks > 1;
 
     if (a.method == 0) {
@@ -224,7 +222,7 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
             if (vec) {
                 for (int j = j0; j < a.N; j += jstride) {
                     double x;
-                    if (a.xp) { x = fma(stp, a.d[j], a.xp[j]); a.x[j] = x; }
+                    if (a.xp) { x = fma(a.stp, a.d[j], a.xp[j]); a.x[j] = x; }
                     else x = a.x[j];
                     xn = fma(x, x, xn);
                     if (x > m) { s = s * exp(m - x) + 1.0; m = x; }
@@ -416,7 +414,7 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
             double c[1] = {0.0};
             for (int i = tid; i < a.M; i += kPEvalThreads) {
                 double x;
-                if (a.xp) { x = fma(stp, a.d[i], a.xp[i]); a.x[i] = x; }
+                if (a.xp) { x = fma(a.stp, a.d[i], a.xp[i]); a.x[i] = x; }
                 else x = a.x[i];
                 reinterpret_cast<double2*>(a.ab)[i] = make_double2(x, 0.0);
                 c[0] = fma(x, x, c[0]);

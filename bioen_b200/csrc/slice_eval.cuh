@@ -54,7 +54,6 @@ struct SliceArgs {
     const double* xp;
     const double* d;
     double stp;
-    const double* stp_dev;
     const double* Gv;    // G (logw) / w0 (forces)
     double* w;
     double* aux_n;       // forces: x_j, later E_j
@@ -267,7 +266,6 @@ __global__ void __launch_bounds__(kSliceThreads, 1) slice_eval_kernel(const Slic
             cp_async16(sl + (size_t)i * ncs + 2 * q, src + (size_t)i * a.ld + 2 * q);
         }
     }
-    const double stp = a.stp_dev ? __ldg(a.stp_dev) : a.stp;
     const double theta = a.theta;
     if (a.mode != kPEvalGradient)
         for (int i = tid; i < M; i += kSliceThreads) vobs[i] = a.Yobs[i];
@@ -282,7 +280,7 @@ __global__ void __launch_bounds__(kSliceThreads, 1) slice_eval_kernel(const Slic
             for (int jj = tid; jj < nv; jj += kSliceThreads) {
                 const int j = c0 + jj;
                 double x;
-                if (a.xp) { x = fma(stp, a.d[j], a.xp[j]); a.x[j] = x; }
+                if (a.xp) { x = fma(a.stp, a.d[j], a.xp[j]); a.x[j] = x; }
                 else x = a.x[j];
                 vx[jj] = x;
                 vg[jj] = a.Gv[j];
@@ -412,7 +410,7 @@ __global__ void __launch_bounds__(kSliceThreads, 1) slice_eval_kernel(const Slic
             double c[1] = {0.0};
             for (int i = tid; i < M; i += kSliceThreads) {
                 double x;
-                if (a.xp) { x = fma(stp, a.d[i], a.xp[i]); if (b == 0) a.x[i] = x; }
+                if (a.xp) { x = fma(a.stp, a.d[i], a.xp[i]); if (b == 0) a.x[i] = x; }
                 else x = a.x[i];
                 vr[i] = x;
                 c[0] = fma(x, x, c[0]);

@@ -37,7 +37,7 @@ enum ScalarSlot {
     SC_DGINIT = 19,   // g . d for the new direction
     SC_DNORM2 = 20,   // ||d||^2 (initial step)
     SC_BETA2 = 21,    // second-loop dots alternate between SC_BETA and SC_BETA2
-    SC_STP = 22,      // trial step length when an evaluation is replayed from a CUDA graph
+    // 22, 23 unused
     SC_YS0 = 24,      // ys[m] ring, up to 16 entries
     SC_ALPHA0 = 40,   // raw s_j . d ring, up to 16 entries
     SC_TMP0 = 56,     // generic outputs of vec_dot etc.
@@ -103,7 +103,6 @@ struct LseArgs {
     const double* xp;    // nullptr: x is used as is
     const double* d;
     double stp;
-    const double* stp_dev;   // non-null: the step length is read from device memory (CUDA-graph replays)
     const double* w0;    // nullptr for logw
     // forces: x_j is first assembled from the column-pass partial sums
     const double* col_partial;  // nullptr: x already holds the values
@@ -119,7 +118,6 @@ __global__ void __launch_bounds__(kVecThreads) k_update_lse(const LseArgs a) {
     __shared__ double red[3 * 32];
     __shared__ bool is_last;
     double m = -DBL_MAX, s = 0.0, xn = 0.0;
-    const double stp = a.stp_dev ? __ldg(a.stp_dev) : a.stp;
     for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < a.n; j += gridDim.x * blockDim.x) {
         double x;
         if (a.col_partial) {
@@ -129,7 +127,7 @@ __global__ void __launch_bounds__(kVecThreads) k_update_lse(const LseArgs a) {
             for (int q = 0; q < ns; ++q) x += a.col_partial[(size_t)q * a.col_ld + j];
             a.x[j] = x;
         } else if (a.xp) {
-            x = fma(stp, a.d[j], a.xp[j]);
+            x = fma(a.stp, a.d[j], a.xp[j]);
             a.x[j] = x;
         } else {
             x = a.x[j];
@@ -602,17 +600,15 @@ struct ForcesUpdateArgs {
     double stp;
     double* ab;
     double* sc;
-    const double* stp_dev;   // non-null: step length from device memory (CUDA-graph replays)
 };
 
 __global__ void __launch_bounds__(1024) k_forces_update(const ForcesUpdateArgs a) {
     __shared__ double red[32];
     double v[1] = {0.0};
-    const double stp = a.stp_dev ? __ldg(a.stp_dev) : a.stp;
     for (int i = threadIdx.x; i < a.m; i += blockDim.x) {
         double x = a.x[i];
         if (a.xp) {
-            x = fma(stp, a.d[i], a.xp[i]);
+            x = fma(a.stp, a.d[i], a.xp[i]);
             a.x[i] = x;
         }
         reinterpret_cast<double2*>(a.ab)[i] = make_double2(x, 0.0);

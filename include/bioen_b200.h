@@ -327,6 +327,13 @@ int bioen_b200_selftest_num_slots(long long run, long long L, long long chunk);
  * log2 threads along the columns (column sums), log2 lanes per row (row sums), log2 lanes per row (table sums),
  * dynamic shared memory in bytes}. */
 int bioen_b200_selftest_slice_plan(int m, int n, int sms, long long max_dyn_smem, long long out[8]);
+/* host-only test hook: the schedule of the two-loop recursion over the `bound` newest pairs of an m-slot ring whose
+ * newest pair is in slot end - 1 (1 <= m <= 16, 1 <= bound <= m, 0 <= end < m).  Writes 2*bound + 1 steps of 11 ints,
+ * {init, u_kind, u_slot, v_kind, v_slot, c_num, c_den, csign, c2_num, scale, out}, to steps and returns their number
+ * (-1: arguments out of range).  One step is d <- (init ? -g : d) + coef * u ; d *= sc[16] / sc[17] when scale ;
+ * sc[out] = v . d, where coef = csign * sc[c_num] / sc[c_den] (- sc[c2_num] / sc[c_den] when c2_num >= 0), kinds are
+ * 0 none, 1 s_slot, 2 y_slot, 3 g, and sc is the 64-double scalar file (ys ring at 24, raw s.d ring at 40). */
+int bioen_b200_selftest_twoloop_schedule(int end, int bound, int m, int *steps);
 /* device test hook: ONE L-BFGS direction update (new pair s = x - xp, y = g - gp into ring slot end_old, then the
  * two-loop recursion over `bound` pairs, lbfgs.c:543-598) from a given state, on engine 0 (multi-kernel), 1 (single-CTA
  * kernel, unsharded, n <= 1024), 2 (coefficient space with the resident Gram matrix, filled first from S and Y, its

@@ -2,8 +2,13 @@
 
     python scripts/replicates_probe.py --dump DIR
         theta_scan outputs (X, fmin, codes, iterations) of seeded problems -- log-weights 100 x 20 000 and forces
-        300 x 4 000, K = 11, line searches 2 and 0 -- written to DIR/theta_scan_<method>_ls<k>.npz.  Two builds that
-        must compute the same theta scan give identical files.
+        300 x 4 000, K = 11, line searches 2 and 0 -- written to DIR/theta_scan_<method>_ls<k>.npz; opt_lbfgs
+        outputs (x, fmin, code, iterations, evaluations) of the same problems at theta = 1, at most 300 iterations,
+        for line searches 0-3 with
+        the single-CTA, speculative-trial and Gram update options each on and off, to DIR/opt_lbfgs_<method>.npz; and
+        both minimisers on a log-weights 8 x 40 problem whose backtracking searches end in
+        LBFGSERR_INCREASEGRADIENT, to DIR/increase_gradient.npz.  Two builds that must compute the same minimisations
+        give identical files.
 
     python scripts/replicates_probe.py --time DIR
         prints the device name and power limit, then times (host clock around work that ends in a device
@@ -16,6 +21,7 @@
         Records go to stdout and DIR/replicates_probe.jsonl.
 """
 import argparse
+import itertools
 import json
 import os
 import subprocess
@@ -27,6 +33,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
+OPT_LBFGS_GRAM, OPT_LBFGS_SMALL, OPT_LBFGS_SPECULATIVE = 6, 9, 10   # bioen_b200_set_option
 THETAS = np.array([1000.0, 300.0, 100.0, 30.0, 10.0, 3.0, 1.0, 0.3, 100.0, 10.0, 55.0])
 
 
@@ -48,7 +55,32 @@ def dump(out):
                 X, fmin, codes, info = p.theta_scan(THETAS, method=meth, linesearch=ls)
                 np.savez(os.path.join(out, "theta_scan_%s_ls%d.npz" % (name, ls)), X=X, fmin=fmin, codes=codes,
                          iterations=info["iterations"])
-                print("%s ls=%d: codes %s iterations %s" % (name, ls, list(codes), list(info["iterations"])))
+                print("%s ls=%d: codes %s iterations %s" % (name, ls, list(codes), list(info["iterations"])), flush=True)
+            res = {}
+            x0 = P["GInit"] if meth == LOGW else np.zeros(M)
+            for ls in range(4):
+                for small, spec, gram in itertools.product((1, 0), repeat=3):
+                    for opt, v in ((OPT_LBFGS_SMALL, small), (OPT_LBFGS_SPECULATIVE, spec), (OPT_LBFGS_GRAM, gram)):
+                        p.set_option(opt, v)
+                    x, fmin, code, info = p.opt_lbfgs(x0, method=meth, linesearch=ls, max_iterations=300)
+                    key = "ls%d_small%d_spec%d_gram%d" % (ls, small, spec, gram)
+                    res.update({key + "_x": x, key + "_fmin": fmin, key + "_code": code,
+                                key + "_iterations": info["iterations"], key + "_evaluations": info["evaluations"]})
+            np.savez(os.path.join(out, "opt_lbfgs_%s.npz" % name), **res)
+            print("%s opt_lbfgs: codes %s" % (name, sorted({int(v) for k, v in res.items() if k.endswith("_code")})),
+                  flush=True)
+    P = O.synthetic_problem(8, 40, seed=5)
+    thetas = np.array([0.01, 1.0, 100.0])
+    with bioen_b200.Problem(P["yTilde"]) as p:
+        p.set_logw(P["G"], P["YTilde"], 1.0)
+        X, fmin, codes, info = p.theta_scan(thetas, x0=P["GInit"], linesearch=1)
+        res = dict(scan_X=X, scan_fmin=fmin, scan_codes=codes, scan_iterations=info["iterations"])
+        for q, th in enumerate(thetas):
+            p.set_theta(th)
+            x, f, code, info = p.opt_lbfgs(P["GInit"], linesearch=1)
+            res.update({"opt%d_x" % q: x, "opt%d_fmin" % q: f, "opt%d_code" % q: code})
+        np.savez(os.path.join(out, "increase_gradient.npz"), **res)
+        print("increase_gradient: scan codes %s" % list(codes))
 
 
 def emit(out, rec):

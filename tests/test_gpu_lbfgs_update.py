@@ -10,7 +10,7 @@ checked on its own:
     one launch at its own (end, bound) and some inactive, and the sharded engines through dist.LocalGroup.  s, y, xp,
     gp must be bitwise, ys, yy, the raw s_j . d ring and g . d and every component of d under |gpu - ref| <= C u scale.
 (b) the drivers' own histories: opt_lbfgs stopped after k = 1 .. 14 iterations (the ring wraps twice) under every line
-    search, with the small, Gram, speculative-trial and CUDA-graph switches; the store the minimiser leaves (debug
+    search, with the small, Gram, speculative-trial and lazy-gradient switches; the store the minimiser leaves (debug
     read 5) must continue the run of k - 1 iterations bit for bit, and its d must be the reference recursion on its own
     S, Y and gradient.
 """
@@ -37,7 +37,7 @@ os.environ.setdefault("BIOEN_B200_P2P_TIMEOUT_S", "30")
 C = 16
 LOGW, FORCES = 0, 1
 MULTI, SMALL, GRAM, BATCHED = 0, 1, 2, 3
-OPT_FUSED_EXCHANGE, OPT_LBFGS_GRAM, OPT_LBFGS_SMALL, OPT_LBFGS_SPECULATIVE = 4, 6, 9, 10
+OPT_LAZY_GRADIENT, OPT_FUSED_EXCHANGE, OPT_LBFGS_GRAM, OPT_LBFGS_SMALL, OPT_LBFGS_SPECULATIVE = 3, 4, 6, 9, 10
 SC_YS, SC_YY, SC_DGINIT, SC_YS0, SC_ALPHA0 = 16, 17, 19, 24, 40
 MAXIMUMITERATION = -997
 M = T.M
@@ -317,15 +317,15 @@ def _datasets():
 
 
 DATASETS = _datasets()
-TOGGLES = ["default", "small_off", "gram", "speculative_off", "graphs"]
+TOGGLES = ["default", "small_off", "gram", "speculative_off", "lazy_off"]
 
 
 def _toggle_cases():
     out = []
     for name, ds in DATASETS.items():
         for tog in TOGGLES:
-            if ds[6] > 1 and tog in ("small_off", "graphs"):
-                continue                      # sharded: no small engine, no graph replays
+            if ds[6] > 1 and tog == "small_off":
+                continue                      # sharded: no small engine
             out.append(pytest.param(name, tog, id="%s-%s" % (name, tog)))
     return out
 
@@ -372,6 +372,7 @@ def test_driver_histories(cache, name, toggle, linesearch):
         p.set_option(OPT_LBFGS_SMALL, 0 if toggle == "small_off" else 1)
         p.set_option(OPT_LBFGS_GRAM, 1 if toggle == "gram" else 0)
         p.set_option(OPT_LBFGS_SPECULATIVE, 0 if toggle == "speculative_off" else 1)
+        p.set_option(OPT_LAZY_GRADIENT, 0 if toggle == "lazy_off" else 1)
 
     def run(p, lo, hi, k):
         xs = x0[lo:hi] if method == LOGW else x0
@@ -379,9 +380,6 @@ def test_driver_histories(cache, name, toggle, linesearch):
         m = hi - lo if method == LOGW else n
         return x, code, _store(p, m), p.scalars()
 
-    env = os.environ.get("BIOEN_B200_GRAPHS")
-    if toggle == "graphs":
-        os.environ["BIOEN_B200_GRAPHS"] = "1"
     try:
         if world > 1:
             obj.call(lambda r, p, lo, hi: setup(p, lo, hi))
@@ -419,15 +417,11 @@ def test_driver_histories(cache, name, toggle, linesearch):
             stores.append(st)
         assert len(xs) >= 4, "fewer than three iterations ran"
     finally:
-        if env is None:
-            os.environ.pop("BIOEN_B200_GRAPHS", None)
-        else:
-            os.environ["BIOEN_B200_GRAPHS"] = env
+        defaults = ((OPT_LBFGS_GRAM, 0), (OPT_LBFGS_SMALL, 1), (OPT_LBFGS_SPECULATIVE, 1), (OPT_LAZY_GRADIENT, 1))
         if world > 1:
-            obj.call(lambda r, p, lo, hi: (p.set_option(OPT_LBFGS_GRAM, 0), p.set_option(OPT_LBFGS_SMALL, 1),
-                                           p.set_option(OPT_LBFGS_SPECULATIVE, 1)))
+            obj.call(lambda r, p, lo, hi: [p.set_option(o, v) for o, v in defaults])
         else:
-            for o, v in ((OPT_LBFGS_GRAM, 0), (OPT_LBFGS_SMALL, 1), (OPT_LBFGS_SPECULATIVE, 1)):
+            for o, v in defaults:
                 obj.set_option(o, v)
 
 

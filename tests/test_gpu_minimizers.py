@@ -254,6 +254,29 @@ def test_theta_scan_ragged_shapes(oracle, M, N, K):
             assert rel(fo, fmin[q]) < 1e-11 or codes[q] < 0
 
 
+def test_increasing_gradient_keeps_the_last_accepted_objective(oracle):
+    """A search that ends in LBFGSERR_INCREASEGRADIENT (the new direction is not a descent direction) returns before
+    its first trial in liblbfgs: x is the last accepted point and fmin its objective.  The minimisers enqueue that
+    trial before the slope is known; its objective must not become fmin.  Backtracking (linesearch 1) on this seeded
+    problem ends so at theta = 0.01 (7 iterations) and theta = 1."""
+    import bioen_b200
+    P = oracle.synthetic_problem(8, 40, seed=5)
+    thetas = [0.01, 1.0]
+    with bioen_b200.Problem(P["yTilde"]) as p:
+        p.set_logw(P["G"], P["YTilde"], 1.0)
+        X, fmin, codes, info = p.theta_scan(thetas, x0=P["GInit"], linesearch=1)
+        for q, th in enumerate(thetas):
+            ref = oracle.lbfgs(lambda x: oracle.logw_fg(x, P["G"], P["yTilde"], P["YTilde"], th), P["GInit"],
+                               linesearch=1)
+            assert ref["code"] == -994
+            p.set_theta(th)
+            x1, f1, c1, _ = p.opt_lbfgs(P["GInit"], linesearch=1)
+            for x, f, code in ((X[q], fmin[q], codes[q]), (x1, f1, c1)):
+                assert code == -994, (th, code)
+                assert rel(f, ref["fx"]) < 1e-11, (th, f, ref["fx"])
+                assert rel(f, p.objective(x)) < 1e-11, (th, f, p.objective(x))
+
+
 def test_theta_scan_errors_and_chunking(oracle):
     import bioen_b200
     from bioen_b200 import optimize

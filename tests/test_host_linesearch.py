@@ -94,3 +94,53 @@ def test_fletcher_interpolation_matches_gsl_restatement(oracle):
             want = oracle._interpolate(a, fa, fpa, b, fb, fpb, lo, hi, order)
             got = lib.bioen_b200_selftest_interpolate(a, fa, fpa, b, fb, fpb, lo, hi, order)
             assert got == want or (math.isnan(got) and math.isnan(want)), (a, fa, fpa, b, fb, fpb, lo, hi, order)
+
+
+def _run_two_loop_schedule(steps, g, S, Y, sc):
+    """Execute the steps of bioen_b200_selftest_twoloop_schedule in NumPy with the oracle's operations: each dot product
+    is np.dot(v, d), each quotient a separate division, each axpy d + coef*u."""
+    ring = {1: S, 2: Y}
+    d = None
+    for init, u_kind, u_slot, v_kind, v_slot, c_num, c_den, csign, c2_num, scale, out in steps:
+        if init:
+            d = -g
+        if u_kind:
+            coef = float(csign) * (sc[c_num] / sc[c_den])
+            if c2_num >= 0:
+                coef = coef - sc[c2_num] / sc[c_den]
+            d = d + coef * ring[u_kind][u_slot]
+        if scale:
+            d = d * (sc[16] / sc[17])
+        if v_kind:
+            sc[out] = float(np.dot(g if v_kind == 3 else ring[v_kind][v_slot], d))
+    return d, sc
+
+
+def test_two_loop_schedule_matches_oracle_recursion(oracle):
+    """The two-loop schedule the minimisers launch (csrc/lbfgs.cuh two_loop_step; one entry per fused kernel step),
+    run step by step in NumPy, reproduces the oracle's two-loop recursion bit for bit for every ring length m, ring end
+    and history length.  Unused scalar-file entries are NaN, so a step that reads a slot nothing wrote shows up."""
+    lib = _lib.load()
+    rng = np.random.default_rng(7)
+    n = 5
+    steps = np.zeros(33 * 11, dtype=np.int32)
+    sp = steps.ctypes.data_as(C.POINTER(C.c_int))
+    for m in range(1, 17):
+        for end in range(m):
+            for bound in range(1, m + 1):
+                count = lib.bioen_b200_selftest_twoloop_schedule(end, bound, m, sp)
+                assert count == 2 * bound + 1, (m, end, bound, count)
+                g = rng.standard_normal(n)
+                S, Y = rng.standard_normal((m, n)), rng.standard_normal((m, n))
+                ys_arr = rng.uniform(0.5, 2.0, m)
+                newest = (end - 1) % m
+                yy = rng.uniform(0.5, 2.0)
+                sc = np.full(64, np.nan)
+                sc[24:24 + m] = ys_arr
+                sc[16], sc[17] = ys_arr[newest], yy
+                d, sc = _run_two_loop_schedule(steps[:11 * count].reshape(count, 11), g, S, Y, sc)
+                want = oracle.lbfgs_two_loop(g, S, Y, ys_arr, end, bound, ys_arr[newest], yy)
+                assert np.array_equal(d, want), (m, end, bound)
+                assert sc[19] == float(np.dot(g, want)), (m, end, bound)   # g.d for the next line search
+    for bad in ((0, 1, 0), (0, 0, 6), (0, 7, 6), (6, 1, 6), (-1, 1, 6), (0, 17, 17)):
+        assert lib.bioen_b200_selftest_twoloop_schedule(*bad, sp) == -1, bad
