@@ -40,7 +40,8 @@ class visual_params(C.Structure):  # c_bioen_common.h:89-92
 
 
 class bioen_b200_batch(C.Structure):  # include/bioen_b200.h: per-problem inputs of a batch (NULL = shared vector)
-    _fields_ = [("K", C.c_int), ("thetas", _dp), ("YTilde", _dp), ("row_weights", _dp), ("w0", _dp)]
+    _fields_ = [("K", C.c_int), ("thetas", _dp), ("YTilde", _dp), ("row_weights", _dp), ("w0", _dp),
+                ("row_scale", _dp), ("row_offset", _dp)]
 
 
 # name -> (restype, argtypes); mirrors include/bioen_b200.h one to one (tests/test_abi.py checks the set)

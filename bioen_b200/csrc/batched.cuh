@@ -2,7 +2,8 @@
 // evaluation become skinny fp64 GEMMs  avg[M x K] = Y . W[N x K]  and  c[N x K] = Yt . R[M x K]  and yTilde is
 // streamed from HBM once per pass for all K problems instead of K times.  The problems differ in theta and start
 // point (the theta scan, the L-curve) and, optionally, in YTilde, in observable weights c_i of chi^2 = 1/2 sum c r^2,
-// and (forces) in the reference weights w0: bootstrap and cross-validation replicates (DESIGN.md section 4g).  This is the only place the library uses tensor cores:
+// and (forces) in the reference weights w0: bootstrap and cross-validation replicates (DESIGN.md section 4g), and in a
+// row-affine transform a_i yTilde_ij + b_i of the matrix: nuisance parameters (section 4c).  This is the only place the library uses tensor cores:
 // fp64 has no tcgen05 kind on Blackwell, so the GEMMs are warp-level DMMA (mma.sync.m8n8k4.f64) fed by TMA.
 //
 // What the reference does for the same job: a Python loop over theta calling find_optimum once per value
@@ -218,6 +219,11 @@ struct BatchBufs {
     const double* Yobs;         // YTilde
     long long yld = 0;          // 0 or ldo
     const double* Cw = nullptr; // [KP][ldo] observable weights c_k,i: chi^2 = 1/2 sum_i c r^2, gradients use c r
+    // [KP][ldo] row-affine transform of problem k (both set or both nullptr = identity): problem k's matrix is
+    // a_i yTilde_ij + b_i, so its averages are a_i avg_i + b_i with avg = yTilde . w of the RESIDENT matrix (sum w = 1).
+    // avgk keeps the untransformed avg (kbf_grad reads it); the residual planes Rf carry a c r.
+    const double* As = nullptr;
+    const double* Bo = nullptr;
     // forces scan only: the variables are M-dimensional planes; these are the structure-axis work planes
     int nN = 0;                 // structures
     long long ldN = 0;
@@ -316,16 +322,20 @@ __global__ void __launch_bounds__(1024) kb_finalize(const BatchBufs b, const KVe
     __shared__ double red[2 * 32];
     const double* Y = b.Yobs + (size_t)k * b.yld;
     const double* c = b.Cw ? b.Cw + (size_t)k * b.ldo : nullptr;
+    const double* a = b.As ? b.As + (size_t)k * b.ldo : nullptr;
+    const double* o = b.Bo ? b.Bo + (size_t)k * b.ldo : nullptr;
     double v[2] = {0.0, 0.0};
     for (int i = threadIdx.x; i < m; i += blockDim.x) {
         double s = 0.0;
         for (int q = 0; q < nseg; ++q) s += b.avgp[((size_t)q * b.KP + k) * ldo + i];
         b.avgk[(size_t)k * b.ldo + i] = s;
-        const double r = s - Y[i];
+        // d chi^2 / d g_j = w_j sum_i (a c r)_i (y_ij - avg_i): the offsets cancel, the sum uses the resident avg
+        const double r = (a ? fma(a[i], s, o[i]) : s) - Y[i];
         const double cr = c ? c[i] * r : r;
-        b.Rf[frag_index(i, k, b.NT)] = cr;
+        const double acr = a ? a[i] * cr : cr;
+        b.Rf[frag_index(i, k, b.NT)] = acr;
         v[0] = fma(cr, r, v[0]);
-        v[1] = fma(cr, s, v[1]);
+        v[1] = fma(acr, s, v[1]);
     }
     block_sum<2>(v, red);
     if (threadIdx.x == 0) {
@@ -337,7 +347,7 @@ __global__ void __launch_bounds__(1024) kb_finalize(const BatchBufs b, const KVe
         sc[SC_CHI2] = chi2;
         sc[SC_PRIOR] = prior;
         sc[SC_F] = prior + chi2;
-        sc[SC_TMP0 + 1] = v[1];   // sum_i r_i avg_i
+        sc[SC_TMP0 + 1] = v[1];   // sum_i (a c r)_i avg_i
     }
 }
 
@@ -469,11 +479,14 @@ __global__ void __launch_bounds__(256) kbf_prepare(const BatchBufs b, const KVec
     double* x = b.X + (size_t)k * b.ldn;
     const double* xp = b.XP + (size_t)k * b.ldn;
     const double* d = b.D + (size_t)k * b.ldn;
+    // row-affine planes: x_j = sum_i (a_i y_ij + b_i) f_i = (Yt (a f))_j + sum_i b_i f_i, and a shift common to all j
+    // leaves the weights, lr_j and KL unchanged, so the GEMM gets a f; ||x||^2 stays the norm of the variables f
+    const double* a = b.As ? b.As + (size_t)k * b.ldo : nullptr;
     double v[1] = {0.0};
     for (int i = threadIdx.x; i < b.n; i += blockDim.x) {
         double xi = x[i];
         if (move) { xi = fma(p.stp[k], d[i], xp[i]); x[i] = xi; }
-        b.Ff[frag_index(i, k, b.NT)] = xi;
+        b.Ff[frag_index(i, k, b.NT)] = a ? a[i] * xi : xi;
         v[0] = fma(xi, xi, v[0]);
     }
     block_sum<1>(v, red);
@@ -558,14 +571,18 @@ __global__ void __launch_bounds__(1024) kbf_finalize(const BatchBufs b, const KV
     __shared__ double red[32];
     const double* Y = b.Yobs + (size_t)k * b.yld;
     const double* c = b.Cw ? b.Cw + (size_t)k * b.ldo : nullptr;
+    const double* a = b.As ? b.As + (size_t)k * b.ldo : nullptr;
+    const double* o = b.Bo ? b.Bo + (size_t)k * b.ldo : nullptr;
     double v[1] = {0.0};
     for (int i = threadIdx.x; i < m; i += blockDim.x) {
         double s = 0.0;
         for (int q = 0; q < nseg; ++q) s += b.avgp[((size_t)q * b.KP + k) * b.ldo + i];
         b.avgk[(size_t)k * b.ldo + i] = s;
-        const double r = s - Y[i];
+        const double r = (a ? fma(a[i], s, o[i]) : s) - Y[i];
         const double cr = c ? c[i] * r : r;
-        b.Rf[frag_index(i, k, b.NT)] = cr;      // t_j = sum_i y_ij c_i r_i: kbf_E and kbf_grad need nothing else
+        // t_j = sum_i y_ij (a c r)_i: kbf_E and kbf_grad need nothing else.  With offsets the exact t_j has one more
+        // term, sum_i b_i c_i r_i, common to all j; it drops out of grad because sum_j (y'_ij - avg'_i) w_j = 0
+        b.Rf[frag_index(i, k, b.NT)] = a ? a[i] * cr : cr;
         v[0] = fma(cr, r, v[0]);
     }
     block_sum<1>(v, red);
@@ -612,7 +629,8 @@ __global__ void __launch_bounds__(kVecThreads) kbf_E(const BatchBufs b, const KV
                 [=](const double(&t)[1]) { sc[SC_TMP0 + 1] = t[0]; });
 }
 
-// grad_i = sum_j y_ij E_j - avg_i sum_j E_j, plus grad.d and ||grad||^2   (one block per problem)
+// grad_i = sum_j y_ij E_j - avg_i sum_j E_j, plus grad.d and ||grad||^2   (one block per problem).  Row-affine
+// planes: grad_i = sum_j (y'_ij - avg'_i) E_j = a_i (sum_j y_ij E_j - avg_i sum_j E_j) with the resident avg (avgk)
 __global__ void __launch_bounds__(1024) kbf_grad(const BatchBufs b, const KVec p, int m, int nseg) {
     const int k = blockIdx.x;
     if (!p.mask[k]) return;
@@ -621,11 +639,13 @@ __global__ void __launch_bounds__(1024) kbf_grad(const BatchBufs b, const KVec p
     const double sumE = sc[SC_TMP0 + 1];
     double* gr = b.Gr + (size_t)k * b.ldn;
     const double* d = b.D + (size_t)k * b.ldn;
+    const double* a = b.As ? b.As + (size_t)k * b.ldo : nullptr;
     double v[2] = {0.0, 0.0};
     for (int i = threadIdx.x; i < m; i += blockDim.x) {
         double s = 0.0;
         for (int q = 0; q < nseg; ++q) s += b.avgp[((size_t)q * b.KP + k) * b.ldo + i];
-        const double gv = s - b.avgk[(size_t)k * b.ldo + i] * sumE;
+        const double gu = s - b.avgk[(size_t)k * b.ldo + i] * sumE;
+        const double gv = a ? a[i] * gu : gu;
         gr[i] = gv;
         v[0] = fma(gv, d[i], v[0]);
         v[1] = fma(gv, gv, v[1]);
@@ -686,6 +706,8 @@ struct BatchPlanes {
     const double* YTilde = nullptr;        // [K][M]  observed data (noise replicates)
     const double* row_weights = nullptr;   // [K][M]  c_k,i >= 0 (observable resampling, held-out folds)
     const double* w0 = nullptr;            // [K][N]  reference weights >= 0 (structure resampling), forces only
+    const double* row_scale = nullptr;     // [K][M]  a_k,i, finite: problem k's matrix is a_k,i yTilde_ij + b_k,i
+    const double* row_offset = nullptr;    // [K][M]  b_k,i, finite (nuisance parameters, nuisance.theta_series)
 };
 
 // Host-side checks of a batch's planes (before anything is allocated or enqueued)
@@ -702,6 +724,12 @@ inline void check_planes(const BatchPlanes& in, int K, int M, int N, bool forces
         if (in.YTilde)
             for (int i = 0; i < M; ++i)
                 if (!std::isfinite(in.YTilde[(size_t)k * M + i])) bad("YTilde must be finite", k, i);
+        if (in.row_scale)
+            for (int i = 0; i < M; ++i)
+                if (!std::isfinite(in.row_scale[(size_t)k * M + i])) bad("row_scale must be finite", k, i);
+        if (in.row_offset)
+            for (int i = 0; i < M; ++i)
+                if (!std::isfinite(in.row_offset[(size_t)k * M + i])) bad("row_offset must be finite", k, i);
         if (in.row_weights)
             for (int i = 0; i < M; ++i) {
                 const double c = in.row_weights[(size_t)k * M + i];
@@ -735,6 +763,7 @@ class ThetaScan {
     long long ldn, ldN;
     DevBuf<double> planes, hist, Wf, Rf, avgp, scb, partials, nplanes, Ff, avgk, redbuf, lsebuf, lse_all;
     DevBuf<double> yplanes, cplanes, wplanes;   // per-problem YTilde, row weights, w0 (allocated when given)
+    DevBuf<double> aplanes, bplanes;            // per-problem row scale and offset (both, when either is given)
     bool started = false;       // run() got past the parameter check: the X planes hold the problems' points
     int vblocksN = 1;
     bool reduce = false;        // N sharded over ranks
@@ -806,6 +835,13 @@ class ThetaScan {
         if (in.YTilde) { B.Yobs = upload_planes(yplanes, in.YTilde, MM, B.ldo); B.yld = B.ldo; }
         if (in.row_weights) B.Cw = upload_planes(cplanes, in.row_weights, MM, B.ldo);
         if (in.w0) { B.G = upload_planes(wplanes, in.w0, NN, ldN); B.gld = ldN; }
+        if (in.row_scale || in.row_offset) {
+            // the kernels take the transform as one pair: the missing half is the identity's
+            const std::vector<double> ones(in.row_scale ? 0 : (size_t)K * MM, 1.0);
+            const std::vector<double> zeros(in.row_offset ? 0 : (size_t)K * MM, 0.0);
+            B.As = upload_planes(aplanes, in.row_scale ? in.row_scale : ones.data(), MM, B.ldo);
+            B.Bo = upload_planes(bplanes, in.row_offset ? in.row_offset : zeros.data(), MM, B.ldo);
+        }
         reduce = C.nranks > 1;
         if (reduce) {
             redbuf.alloc((size_t)KP * gRow.ldo + 4 * KP);

@@ -650,6 +650,8 @@ static BatchPlanes batch_planes(const bioen_b200_ctx* ctx, const bioen_b200_batc
     in.YTilde = batch->YTilde;
     in.row_weights = batch->row_weights;
     in.w0 = batch->w0;
+    in.row_scale = batch->row_scale;
+    in.row_offset = batch->row_offset;
     return in;
 }
 

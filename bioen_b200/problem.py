@@ -374,13 +374,16 @@ class Problem:
                                                  rounds=int(stats[0]), gemm_launches=int(stats[1]),
                                                  seconds=float(stats[2]))
 
-    # ---- batched replicates: K <= 32 problems with per-problem YTilde, observable weights, w0 ----------------------
-    def _batch(self, method, thetas, X, YTilde, row_weights, w0):
+    # ---- batched replicates: K <= 32 problems with per-problem YTilde, observable weights, w0, row transform --------
+    _PLANES = ("YTilde", "row_weights", "w0", "row_scale", "row_offset")
+
+    def _batch(self, method, thetas, X, YTilde, row_weights, w0, row_scale=None, row_offset=None):
         """The bioen_b200_batch of a call and the arrays it points to: thetas (K,), X (K, n), and (K, M) / (K, N)
         planes or None.  A scalar theta and single vectors are broadcast; K comes from whichever argument has rows."""
         n = self._dim(method)
         args = [("thetas", np.asarray(thetas, dtype=np.float64), 0), ("x", np.asarray(X, dtype=np.float64), n),
-                ("YTilde", YTilde, self.m), ("row_weights", row_weights, self.m), ("w0", w0, self.n)]
+                ("YTilde", YTilde, self.m), ("row_weights", row_weights, self.m), ("w0", w0, self.n),
+                ("row_scale", row_scale, self.m), ("row_offset", row_offset, self.m)]
         args = [(name, None if a is None else np.asarray(a, dtype=np.float64), width) for name, a, width in args]
         Ks = {a.shape[0] for name, a, width in args if a is not None and a.ndim == (1 if width == 0 else 2)} - {1}
         if len(Ks) > 1:
@@ -398,19 +401,24 @@ class Problem:
                 raise ValueError("%s must have shape %s or %s, got %s" % (name, want[1:] or "()", want, a.shape))
             out[name] = np.ascontiguousarray(np.broadcast_to(a, want))
         b = _lib.bioen_b200_batch(K, _lib.ptr(out["thetas"]), *(None if out[k] is None else _lib.ptr(out[k])
-                                                                   for k in ("YTilde", "row_weights", "w0")))
+                                                                   for k in self._PLANES))
         return K, n, b, out
 
-    def batch_minimize(self, thetas, x0=None, YTilde=None, row_weights=None, w0=None, method=None, verbose=0, **cfg):
+    def batch_minimize(self, thetas, x0=None, YTilde=None, row_weights=None, w0=None, method=None, verbose=0,
+                       row_scale=None, row_offset=None, **cfg):
         """Minimise up to 32 problems that share yTilde TOGETHER (the theta scan's lockstep L-BFGS and batched fp64
         tensor-core evaluations).  Per problem k, optionally: YTilde[k] (M,) in place of the shared YTilde,
-        observable weights row_weights[k] (M,) >= 0 with chi^2 = 1/2 sum_i c_i r_i^2, and (forces only) reference
-        weights w0[k] (N,) >= 0.  Scalars / single vectors are broadcast.  Returns (X (K, n), fmin (K,), codes (K,),
-        info) like theta_scan; info also holds averages (K, M) = yTilde . w, chi2 (K,) and kl (K,) at the returned
-        points (NaN when the L-BFGS parameters are refused)."""
+        observable weights row_weights[k] (M,) >= 0 with chi^2 = 1/2 sum_i c_i r_i^2, (forces only) reference
+        weights w0[k] (N,) >= 0, and a row-affine transform row_scale[k], row_offset[k] (M,) (finite; default ones
+        and zeros): problem k is the one of the matrix row_scale[k][:, None] * yTilde + row_offset[k][:, None], e.g.
+        nuisance parameters (bioen_b200.nuisance.theta_series), while the resident matrix stays as it is.  Scalars /
+        single vectors are broadcast.  Returns (X (K, n), fmin (K,), codes (K,), info) like theta_scan; info also
+        holds averages (K, M) = yTilde . w of the RESIDENT matrix (problem k's own averages are
+        row_scale[k] * averages[k] + row_offset[k]), chi2 (K,) and kl (K,) at the returned points (NaN when the
+        L-BFGS parameters are refused)."""
         method = self._method(method)
         K, n, b, a = self._batch(method, thetas, np.zeros(self._dim(method)) if x0 is None else x0, YTilde,
-                                 row_weights, w0)
+                                 row_weights, w0, row_scale, row_offset)
         p = dict(LBFGS_DEFAULTS)
         p.update(cfg)
         c = _lib.lbfgs_config_params(**{k: p[k] for k, _ in _lib.lbfgs_config_params._fields_})
@@ -428,11 +436,13 @@ class Problem:
                                                  rounds=int(stats[0]), gemm_launches=int(stats[1]),
                                                  seconds=float(stats[2]), averages=avg, chi2=chi2, kl=kl)
 
-    def batch_evaluate(self, X, thetas, YTilde=None, row_weights=None, w0=None, gradient=True, method=None):
+    def batch_evaluate(self, X, thetas, YTilde=None, row_weights=None, w0=None, gradient=True, method=None,
+                       row_scale=None, row_offset=None):
         """One batched evaluation of up to 32 problems (arguments as batch_minimize) at the points X (K, n).
-        Returns (f (K,), grad (K, n) or None, dict(averages (K, M), chi2 (K,), kl (K,)))."""
+        Returns (f (K,), grad (K, n) or None, dict(averages (K, M), chi2 (K,), kl (K,))); averages as batch_minimize:
+        yTilde . w of the resident matrix."""
         method = self._method(method)
-        K, n, b, a = self._batch(method, thetas, X, YTilde, row_weights, w0)
+        K, n, b, a = self._batch(method, thetas, X, YTilde, row_weights, w0, row_scale, row_offset)
         f, chi2, kl = np.empty(K), np.empty(K), np.empty(K)
         g = np.empty((K, n), dtype=np.float64) if gradient else None
         avg = np.empty((K, self.m), dtype=np.float64)

@@ -271,18 +271,27 @@ int bioen_b200_theta_scan(bioen_b200_ctx *ctx, int method, int K, const double *
  *   row_weights [K][M]  observable weights c_i >= 0, finite: chi^2 = 1/2 sum_i c_i r_i^2 (resampled or held-out rows)
  *   w0          [K][N]  reference weights >= 0, finite, positive sum (resampled structures); BIOEN_B200_FORCES only:
  *                       the log-weights parametrisation cannot represent a structure of weight zero
- * Invalid arrays, and sharded contexts, are refused before anything runs. */
+ *   row_scale   [K][M]  a_i, finite (zeros allowed); NULL = all ones
+ *   row_offset  [K][M]  b_i, finite; NULL = all zeros.  Problem k is the one of the matrix a_i yTilde_ij + b_i
+ *                       (row-affine nuisance parameters: DEER modulation depth, scattering scale factor) while the
+ *                       resident yTilde is neither read twice nor changed.  Its averages are a_i avg_i + b_i; the avg
+ *                       outputs below stay yTilde . w of the RESIDENT matrix.
+ * Invalid arrays, and sharded contexts, are refused before anything runs.  Fields may be added at the end of the
+ * struct: zero-initialise it (e.g. `bioen_b200_batch b = {0};`) so that fields a caller does not know are NULL. */
 typedef struct bioen_b200_batch {
     int K;
     const double *thetas;        /* [K] */
     const double *YTilde;
     const double *row_weights;
     const double *w0;
+    const double *row_scale;
+    const double *row_offset;
 } bioen_b200_batch;
 
 /* lockstep L-BFGS of the batch: x0_host / x_host, fmin, codes, info, stats as for bioen_b200_theta_scan (which is this
  * call with every array NULL).  Then one objective evaluation at the returned points gives, per problem,
- * avg[K][M] = yTilde . w(x_k), chi2[K] (with the row weights) and kl[K] (the relative entropy, without theta); each
+ * avg[K][M] = yTilde . w(x_k) of the resident matrix, chi2[K] (with the row weights and the row-affine transform)
+ * and kl[K] (the relative entropy, without theta); each
  * may be NULL.  All three are NaN when the L-BFGS parameters are refused. */
 int bioen_b200_batch_minimize(bioen_b200_ctx *ctx, int method, const bioen_b200_batch *batch, const double *x0_host,
                               double *x_host, lbfgs_config_params config, visual_params visual, double *fmin,
