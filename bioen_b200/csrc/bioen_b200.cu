@@ -311,8 +311,8 @@ int bioen_b200_set_option(bioen_b200_ctx* ctx, int option, int value) {
     return guarded("bioen_b200_set_option", [&] {
         ctx->pending_gen = -1;   // a pending objective-only evaluation is not continued across a change of path
         switch (option) {
-            case BIOEN_B200_OPT_FUSED_FORCES: ctx->C.allow_fused = value != 0; break;
-            case BIOEN_B200_OPT_LAZY_GRADIENT: ctx->C.lazy_gradient = value != 0; break;
+            case BIOEN_B200_OPT_FUSED_FORCES: ctx->C.options.allow_fused = value != 0; break;
+            case BIOEN_B200_OPT_LAZY_GRADIENT: ctx->C.options.lazy_gradient = value != 0; break;
             case BIOEN_B200_OPT_P2P:
                 if (ctx->comm) {
                     if (ctx->comm->is_local() && !value)
@@ -320,13 +320,13 @@ int bioen_b200_set_option(bioen_b200_ctx* ctx, int option, int value) {
                     ctx->comm->use_p2p = value != 0;
                 }
                 break;
-            case BIOEN_B200_OPT_FUSED_EXCHANGE: ctx->C.fuse_allowed = value != 0; break;
-            case BIOEN_B200_OPT_PERSISTENT: ctx->C.persistent_mode = value; break;
-            case BIOEN_B200_OPT_LBFGS_GRAM: ctx->C.lbfgs_gram_opt = value != 0; break;
-            case BIOEN_B200_OPT_SLICE: ctx->C.slice_mode = value; break;
-            case BIOEN_B200_OPT_LBFGS_SMALL: ctx->C.lbfgs_small_opt = value != 0; break;
-            case BIOEN_B200_OPT_LBFGS_SPECULATIVE: ctx->C.lbfgs_speculative = value != 0; break;
-            case BIOEN_B200_OPT_FETCH_ZEROCOPY: ctx->C.fetch_zero_copy = value != 0; break;
+            case BIOEN_B200_OPT_FUSED_EXCHANGE: ctx->C.options.fuse_allowed = value != 0; break;
+            case BIOEN_B200_OPT_PERSISTENT: ctx->C.options.persistent_mode = value; break;
+            case BIOEN_B200_OPT_LBFGS_GRAM: ctx->C.options.lbfgs_gram_opt = value != 0; break;
+            case BIOEN_B200_OPT_SLICE: ctx->C.options.slice_mode = value; break;
+            case BIOEN_B200_OPT_LBFGS_SMALL: ctx->C.options.lbfgs_small_opt = value != 0; break;
+            case BIOEN_B200_OPT_LBFGS_SPECULATIVE: ctx->C.options.lbfgs_speculative = value != 0; break;
+            case BIOEN_B200_OPT_FETCH_ZEROCOPY: ctx->C.options.fetch_zero_copy = value != 0; break;
             case BIOEN_B200_OPT_STRUCTURE_MAJOR_ONLY:
                 CUDA_CHECK(cudaSetDevice(ctx->C.device));
                 if (value) ctx->C.enter_yt_only();
@@ -361,7 +361,7 @@ int bioen_b200_eval(bioen_b200_ctx* ctx, int method, const double* x_host, doubl
         // store it straight through the mapped host pointer while the pass is still streaming -- the 8*N bytes cross
         // PCIe under the pass instead of in a copy after it.
         bool direct = false;
-        if (grad_host && method == BIOEN_B200_LOGW && C.colgrad_eligible() && !getenv("BIOEN_B200_NO_ZEROCOPY")) {
+        if (grad_host && method == BIOEN_B200_LOGW && C.colgrad_eligible()) {
             cudaPointerAttributes attr{};
             if (cudaPointerGetAttributes(&attr, grad_host) == cudaSuccess && attr.type == cudaMemoryTypeHost &&
                 attr.devicePointer && (reinterpret_cast<uintptr_t>(attr.devicePointer) & 15) == 0) {
@@ -443,7 +443,7 @@ int bioen_b200_affine_rows(bioen_b200_ctx* ctx, const double* scale_host, const 
         const bool had_fused = C.fused_ready;
         C.fused_ready = false;
         C.yt_valid = false;
-        if (had_fused && C.have_forces && C.allow_fused) C.prepare_fused();
+        if (had_fused && C.have_forces && C.options.allow_fused) C.prepare_fused();
         C.sync();
     });
 }
@@ -764,23 +764,9 @@ int bioen_b200_read_stream_peak(bioen_b200_ctx* ctx, int reps, double* gbs) {
         cudaEvent_t e0, e1;
         CUDA_CHECK(cudaEventCreate(&e0));
         CUDA_CHECK(cudaEventCreate(&e1));
-        // default: 2 blocks of 1024 threads per SM, 8 loads in flight per thread (256 KB per SM).  The environment
-        // variable exists for the sensitivity study in DESIGN.md ("U,blocks-per-SM", U in {1,2,4,8})
-        int U = 8, bps = 2, order = -1;
-        if (const char* e = getenv("BIOEN_B200_READ_VARIANT")) sscanf(e, "%d,%d", &U, &bps);
-        if (const char* e = getenv("BIOEN_B200_READ_ORDER")) order = atoi(e);   // tile orders of k_read_tiles
-        const int blocks = prop.multiProcessorCount * (bps == 1 ? 1 : 2);
+        const int blocks = prop.multiProcessorCount * 2;
         const double2* p = reinterpret_cast<const double2*>(C.Y);
-        auto launch = [&] {
-            if (order >= 0) {
-                k_read_tiles<<<blocks, 1024, 0, C.stream>>>(C.Y, C.ld, C.M, C.nRT, C.nCB, order, sink.p);
-                return;
-            }
-            if (U == 1) k_read_stream<1><<<blocks, 1024, 0, C.stream>>>(p, n2, sink.p);
-            else if (U == 2) k_read_stream<2><<<blocks, 1024, 0, C.stream>>>(p, n2, sink.p);
-            else if (U == 4) k_read_stream<4><<<blocks, 1024, 0, C.stream>>>(p, n2, sink.p);
-            else k_read_stream<8><<<blocks, 1024, 0, C.stream>>>(p, n2, sink.p);
-        };
+        auto launch = [&] { k_read_stream<<<blocks, 1024, 0, C.stream>>>(p, n2, sink.p); };
         launch();
         double total = 0.0;
         if (reps < 1) reps = 1;
@@ -834,9 +820,11 @@ double bioen_b200_selftest_interpolate(double a, double fa, double fpa, double b
 }
 
 // host-only: the tile sequence one CTA of a matrix pass walks (stream_pass.cuh, TileWalk) and the slot it writes its
-// partial sums to -- the same code the kernel runs, for CPU tests of coverage and of the slot bookkeeping
+// partial sums to -- the same code the kernel runs, for CPU tests of coverage and of the slot bookkeeping.
+// -1: the row pass has no interleaved order.
 long long bioen_b200_selftest_tilewalk(int pass_mode, int nRT, int nCB, int grid, long long chunk, int interleave,
                                        int cta, long long max_tiles, int* rt, int* cb, long long* slot, int* closes) {
+    if (pass_mode == kRowPass && interleave) return -1;
     PassArgs a{};
     a.nRT = nRT; a.nCB = nCB; a.T = (long long)nRT * nCB; a.chunk = chunk; a.interleave = interleave;
     TileWalk tw;
@@ -952,9 +940,9 @@ int bioen_b200_selftest_lbfgs_update(bioen_b200_ctx* ctx, int engine, int method
             throw std::invalid_argument("bioen_b200: the Gram engine takes reachable states only (bound < 6 needs "
                                         "end_old = bound - 1)");
         // select the engine through the context's switches, as a minimisation would see them; restored below
-        const bool gram0 = C.lbfgs_gram_opt, small0 = C.lbfgs_small_opt;
-        C.lbfgs_gram_opt = engine == 2;
-        C.lbfgs_small_opt = engine == 1;
+        const bool gram0 = C.options.lbfgs_gram_opt, small0 = C.options.lbfgs_small_opt;
+        C.options.lbfgs_gram_opt = engine == 2;
+        C.options.lbfgs_small_opt = engine == 1;
         try {
             opt.x = ctx->x_for(method);
             opt.bind_store();
@@ -1002,12 +990,12 @@ int bioen_b200_selftest_lbfgs_update(bioen_b200_ctx* ctx, int engine, int method
             C.d2h(scalars, C.sc.p, SC_COUNT);
             C.sync();
         } catch (...) {
-            C.lbfgs_gram_opt = gram0;
-            C.lbfgs_small_opt = small0;
+            C.options.lbfgs_gram_opt = gram0;
+            C.options.lbfgs_small_opt = small0;
             throw;
         }
-        C.lbfgs_gram_opt = gram0;
-        C.lbfgs_small_opt = small0;
+        C.options.lbfgs_gram_opt = gram0;
+        C.options.lbfgs_small_opt = small0;
     });
 }
 
@@ -1215,6 +1203,20 @@ long long bioen_b200_query(bioen_b200_ctx* ctx, int what) {
         case 7: return C.slice_ok() ? 1 : 0;
         case 8: return (long long)((C.Yown.p ? C.Yown.n * 8 : 0) + (C.Yt.p ? C.Yt.n * 8 : 0) + (C.Y32.p ? C.Y32.n * 4 : 0));
         case 9: return C.yt_only ? 1 : 0;
+        case 10: {
+            const ContextOptions& o = C.options;
+            const ContextOptions d{};
+            auto bit = [](bool differs, int option) { return differs ? 1LL << option : 0LL; };
+            return bit(o.allow_fused != d.allow_fused, BIOEN_B200_OPT_FUSED_FORCES) |
+                   bit(o.lazy_gradient != d.lazy_gradient, BIOEN_B200_OPT_LAZY_GRADIENT) |
+                   bit(o.fuse_allowed != d.fuse_allowed, BIOEN_B200_OPT_FUSED_EXCHANGE) |
+                   bit(o.persistent_mode != d.persistent_mode, BIOEN_B200_OPT_PERSISTENT) |
+                   bit(o.lbfgs_gram_opt != d.lbfgs_gram_opt, BIOEN_B200_OPT_LBFGS_GRAM) |
+                   bit(o.slice_mode != d.slice_mode, BIOEN_B200_OPT_SLICE) |
+                   bit(o.lbfgs_small_opt != d.lbfgs_small_opt, BIOEN_B200_OPT_LBFGS_SMALL) |
+                   bit(o.lbfgs_speculative != d.lbfgs_speculative, BIOEN_B200_OPT_LBFGS_SPECULATIVE) |
+                   bit(o.fetch_zero_copy != d.fetch_zero_copy, BIOEN_B200_OPT_FETCH_ZEROCOPY);
+        }
         default: return -1;
     }
 }
@@ -1254,7 +1256,7 @@ struct TempProblem {
         ctx = bioen_b200_create(m, n, default_device());
         if (!ctx) throw std::runtime_error(g_last_error);
         try {
-            ctx->C.allow_fused = fused;
+            ctx->C.options.allow_fused = fused;
             if (yTilde) ctx->C.upload_matrix(yTilde, (size_t)n);
         } catch (...) {
             bioen_b200_destroy(ctx);

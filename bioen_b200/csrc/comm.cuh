@@ -10,9 +10,9 @@
 // The exchanges are tiny (3 ... M+3 doubles) and sit on the critical path of every evaluation and of every
 // L-BFGS dot product, so their cost is pure latency.  NCCL needs ~25-30 us for one; the path therefore carries its
 // own exchange over NVLink peer memory (k_p2p_exchange below): every rank owns an inbox that its peers map through
-// CUDA IPC, one small kernel stores the rank's contribution straight into every peer's inbox, publishes a
-// release-flag, waits for the peers' flags and combines the inboxes in rank order (so all ranks hold bit-identical
-// results).  NCCL is kept for the bootstrap (handle exchange), for messages larger than the inbox, and as the
+// CUDA IPC, one small kernel stores the rank's contribution straight into every peer's inbox, each value tagged
+// with the exchange's epoch, waits until the peers' values of that epoch have arrived and combines the inboxes in
+// rank order (so all ranks hold bit-identical results).  NCCL is kept for the bootstrap (handle exchange), for messages larger than the inbox, and as the
 // collective path when peer mapping is not available (BIOEN_B200_P2P=0 forces it).
 #pragma once
 #include <dlfcn.h>
@@ -88,7 +88,6 @@ struct P2PDev {
     int rank, nranks;
     long long cap;
     unsigned long long timeout_ns;
-    int ll;   // 1: flag-in-data ("LL") delivery, 0: data + fence + flag
 };
 
 struct P2PArgs {
@@ -98,14 +97,6 @@ struct P2PArgs {
     int count, op;
 };
 
-__device__ __forceinline__ void st_release_sys(unsigned long long* p, unsigned long long v) {
-    asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ unsigned long long ld_acquire_sys(const unsigned long long* p) {
-    unsigned long long v;
-    asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
 __device__ __forceinline__ unsigned long long global_timer_ns() {
     unsigned long long t;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
@@ -119,69 +110,14 @@ __device__ __forceinline__ unsigned long long global_timer_ns() {
 // combines the contributions itself (in rank order: all ranks get bit-identical results) and must not start the
 // NEXT exchange before it has finished reading (guaranteed by stream order / by being the same block).
 // *fail is set when a peer did not arrive within the timeout (the caller poisons its result with NaN).
-__device__ __forceinline__ const double* p2p_deliver_and_wait_fenced(const P2PDev& a, const double* send, int count,
-                                                                     int* fail) {
-    __shared__ unsigned long long s_epoch;
-    __shared__ int s_fail;
-    unsigned char* me = a.region[a.rank];
-    const int tid = threadIdx.x, nthr = blockDim.x, R = a.nranks;
-    __syncthreads();   // `send` may have been produced by other threads of this block
-    if (tid == 0) {
-        unsigned long long* ep = reinterpret_cast<unsigned long long*>(me + 128);
-        s_epoch = *ep + 1;
-        *ep = s_epoch;
-        s_fail = 0;
-    }
-    __syncthreads();
-    const unsigned long long epoch = s_epoch;
-    const size_t par = (size_t)(epoch & 1);
-    // Read each value ONCE (up to four independent loads in flight per thread), then store it to every inbox.  A loop
-    // "for every rank: dst[i] = send[i]" re-reads send[] per rank, and because dst may alias send the compiler keeps
-    // every load behind the previous store: R x count/nthr serialised L2 round trips (measured: 19.7 us of a 1005-double
-    // exchange between 2 ranks; the same exchange takes ~5 us this way).
-    const size_t slot = (par * R + a.rank) * a.cap;
-    for (int i0 = tid; i0 < count; i0 += 4 * nthr) {
-        double v[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int i = i0 + u * nthr;
-            v[u] = i < count ? send[i] : 0.0;
-        }
-        for (int r = 0; r < R; ++r) {
-            double* dst = reinterpret_cast<double*>(a.region[r] + kP2PHeaderBytes) + slot;
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int i = i0 + u * nthr;
-                if (i < count) dst[i] = v[u];
-            }
-        }
-    }
-    __threadfence_system();
-    __syncthreads();
-    if (tid < R) {
-        st_release_sys(reinterpret_cast<unsigned long long*>(a.region[tid]) + a.rank, epoch);
-        const unsigned long long* flag = reinterpret_cast<const unsigned long long*>(me) + tid;
-        const unsigned long long t0 = global_timer_ns();
-        while (ld_acquire_sys(flag) < epoch) {
-            if (global_timer_ns() - t0 > a.timeout_ns) {  // a peer never arrived: poison the result, do not hang
-                s_fail = 1;
-                break;
-            }
-        }
-    }
-    __syncthreads();
-    *fail = s_fail;
-    return reinterpret_cast<const double*>(me + kP2PHeaderBytes) + par * R * a.cap;
-}
-
-// The same exchange with the flag travelling INSIDE the data (the idea of NCCL's LL protocol): every double is sent
-// as one 16-byte cell {lo32 | epoch32 << 32, hi32 | epoch32 << 32}; each 8-byte half is written atomically, so a
-// receiver that sees the current epoch in both halves has the value -- no system-wide fence after the stores, no
-// separate flag store, no flag poll: one NVLink one-way latency instead of store + fence round trip + flag.  The
-// received values are unpacked into the plain inbox so callers read them exactly as in the fenced variant.
+// The flag travels INSIDE the data (the idea of NCCL's LL protocol): every double is sent as one 16-byte cell
+// {lo32 | epoch32 << 32, hi32 | epoch32 << 32}; each 8-byte half is written atomically, so a receiver that sees the
+// current epoch in both halves has the value -- no system-wide fence after the stores, no separate flag store, no
+// flag poll: one NVLink one-way latency instead of store + fence round trip + flag.  The received values are
+// unpacked into the plain inbox, which callers read.
 // Region: the LL cells live behind the plain inbox ([2][R][cap] doubles), [2][R][cap] cells of 16 bytes.
-__device__ __forceinline__ const double* p2p_deliver_and_wait_ll(const P2PDev& a, const double* send, int count,
-                                                                 int* fail) {
+__device__ __forceinline__ const double* p2p_deliver_and_wait(const P2PDev& a, const double* send, int count,
+                                                              int* fail) {
     __shared__ unsigned long long s_epoch;
     __shared__ int s_fail;
     unsigned char* me = a.region[a.rank];
@@ -198,6 +134,10 @@ __device__ __forceinline__ const double* p2p_deliver_and_wait_ll(const P2PDev& a
     const unsigned long long tag = (epoch & 0xffffffffull) << 32;
     const size_t par = (size_t)(epoch & 1);
     const size_t plain_bytes = (size_t)2 * R * a.cap * sizeof(double);
+    // Read each value ONCE (up to four independent loads in flight per thread), then store it to every inbox.  A loop
+    // "for every rank: dst[i] = send[i]" re-reads send[] per rank, and because dst may alias send the compiler keeps
+    // every load behind the previous store: R x count/nthr serialised L2 round trips (measured: 19.7 us of a 1005-double
+    // exchange between 2 ranks; the same exchange takes ~5 us this way).
     const size_t slot = (par * R + a.rank) * a.cap;
     for (int i0 = tid; i0 < count; i0 += 4 * nthr) {
         unsigned long long lo[4], hi[4];
@@ -242,11 +182,6 @@ __device__ __forceinline__ const double* p2p_deliver_and_wait_ll(const P2PDev& a
     __syncthreads();
     *fail = s_fail;
     return plain;
-}
-
-__device__ __forceinline__ const double* p2p_deliver_and_wait(const P2PDev& a, const double* send, int count,
-                                                              int* fail) {
-    return a.ll ? p2p_deliver_and_wait_ll(a, send, count, fail) : p2p_deliver_and_wait_fenced(a, send, count, fail);
 }
 
 __device__ __forceinline__ double p2p_nan() { return __longlong_as_double(0x7ff8000000000000LL); }
@@ -310,7 +245,6 @@ class Comm {
     unsigned char* mapped[kP2PMaxRanks] = {};
     long long cap = 0;
     long long p2p_launches = 0;
-    bool use_ll = true;       // flag-in-data delivery (BIOEN_B200_EXCHANGE_LL=0 selects data + fence + flag)
     int local_group_id = -1;  // >= 0: in-process group (no NCCL, no IPC)
     unsigned long long timeout_ns = 120ull * 1000000000ull;  // generous: ranks may be skewed by host-side setup
 
@@ -339,13 +273,11 @@ class Comm {
             const double sec = atof(e);
             if (sec > 0) timeout_ns = (unsigned long long)(sec * 1e9);
         }
-        if (const char* e = getenv("BIOEN_B200_EXCHANGE_LL")) use_ll = e[0] != '0';
     }
     // what the producing kernels need to run an exchange themselves; nranks = 1 switches their exchange code off
     P2PDev dev_args() const {
         P2PDev d{};
         d.rank = rank; d.nranks = (p2p && use_p2p) ? nranks : 1; d.cap = cap; d.timeout_ns = timeout_ns;
-        d.ll = use_ll ? 1 : 0;
         for (int r = 0; r < nranks && r < kP2PMaxRanks; ++r) d.region[r] = mapped[r];
         return d;
     }

@@ -83,15 +83,28 @@ inline PFN_encodeTiled get_encode_tiled() {
 
 inline int round_up(long long a, long long b) { return (int)(((a + b - 1) / b) * b); }
 
+// The context's settings of bioen_b200_set_option, at their defaults.  A context taken from the reuse cache gets a
+// fresh record (Context::reset_for_reuse), so no setting outlives the problem it was made for.
+struct ContextOptions {
+    bool allow_fused = true;         // BIOEN_B200_OPT_FUSED_FORCES: 0 forces the four-pass tile kernels
+    bool lazy_gradient = true;       // BIOEN_B200_OPT_LAZY_GRADIENT: minimisers may use the split (results identical)
+    bool fuse_allowed = true;        // BIOEN_B200_OPT_FUSED_EXCHANGE
+    int persistent_mode = -1;        // BIOEN_B200_OPT_PERSISTENT: -1 auto (by size), 0 off, 1 on
+    bool lbfgs_gram_opt = false;     // BIOEN_B200_OPT_LBFGS_GRAM: coefficient-space update
+    int slice_mode = -1;             // BIOEN_B200_OPT_SLICE: -1 / 1 on when the problem is eligible, 0 off
+    bool lbfgs_small_opt = true;     // BIOEN_B200_OPT_LBFGS_SMALL: single-kernel update for n <= 1024
+    bool lbfgs_speculative = true;   // BIOEN_B200_OPT_LBFGS_SPECULATIVE: 0 fetches the initial slope first
+    bool fetch_zero_copy = true;     // BIOEN_B200_OPT_FETCH_ZEROCOPY: 0 fetches the scalar file with a copy
+};
+
 class Context {
    public:
     int M, N;            // local matrix shape (N = this rank's columns)
     long long N_total;   // all columns over all ranks
     long long ld = 0;    // row stride of Y in doubles
     int Mpad, Npad, nRT, nCB;
-    bool interleave_row = false, interleave_col = false;
-    // `chunk` as the readers of the pass partials need it (pass_num_slots)
-    long long row_chunk() const { return interleave_row ? -(long long)grid : chunk; }
+    bool interleave_col = false;
+    // `chunk` as the readers of the column-pass partials need it (pass_num_slots)
     long long col_chunk() const { return interleave_col ? (long long)nRT : chunk; }
     int device, num_sms;
     cudaStream_t stream = nullptr;
@@ -122,17 +135,13 @@ class Context {
     DevBuf<double> pe_part;
     DevBuf<unsigned long long> pe_bar;
     bool coop_ok = false;
-    int persistent_mode = -1;              // BIOEN_B200_OPT_PERSISTENT: -1 auto (by size), 0 off, 1 on
-    double persistent_max_bytes = 0.6e9;   // auto: matrices up to this size per GPU (BIOEN_B200_PERSISTENT_MAX_MB)
+    static constexpr double kPersistentMaxBytes = 0.6e9;   // auto: matrices up to this size per GPU
     long long persistent_launches = 0;
     DevBuf<double> colgrad_part;           // per-CTA scalars of the column pass with the gradient epilogue
-    bool colgrad_opt = true;               // BIOEN_B200_COLGRAD=0: column pass + separate k_logw_grad
-    DevBuf<unsigned long long> pe_trace;   // BIOEN_B200_PERSISTENT_TRACE: phase-boundary timestamps of CTA 0
     // shared-memory-resident evaluation kernel for small matrices (slice_eval.cuh)
     DevBuf<double> slice_tab, slice_gtab, slice_part;
     SlicePlan slice_pl;
     bool slice_coop = false;
-    int slice_mode = -1;                   // BIOEN_B200_OPT_SLICE: -1 / 1 on when the problem is eligible, 0 off
     long long slice_launches = 0;
     double* h_sc = nullptr;  // pinned
 
@@ -140,14 +149,11 @@ class Context {
     DevBuf<double> Yt, fpart, flse;
     DevBuf<double> lbfgs_store;   // g, xp, gp, d, s[m], y[m] of the device L-BFGS (lbfgs.cuh)
     DevBuf<double> lbfgs_gram, lbfgs_gram_partials;   // coefficient-space update (BIOEN_B200_OPT_LBFGS_GRAM)
-    bool lbfgs_gram_opt = false;
-    bool lbfgs_small_opt = true;     // BIOEN_B200_OPT_LBFGS_SMALL: single-kernel update for n <= 1024
-    bool lbfgs_speculative = true;   // BIOEN_B200_LBFGS_SPECULATIVE=0: fetch the initial slope before the first trial
     long long ldt = 0, f_nslab = 0, f_chunk = 0;
     int f_C = 0, f_stages = 0, f_grid = 0, f_KI = 0, f_smem = 0, f_T = 1, f_rows = 0, f_rows_per_cta = 1;
     bool f_team = false;
     bool fused_ready = false, yt_valid = false;
-    bool allow_fused = true;   // bioen_b200_set_option: 0 forces the four-pass tile kernels
+    ContextOptions options;
     double theta = 0.0;
     bool have_logw = false, have_forces = false;
     long long passes_launched = 0, kernels_launched = 0;
@@ -183,18 +189,11 @@ class Context {
         // window of the matrix at a time.  Measured at N = 1e6 x M = 1e3, 40 steps each, one box, back to back
         // (round 2): contiguous 431.6 evals/s (2.3171 ms), column pass interleaved 435.4 (2.2970 ms), row pass
         // interleaved 426.7 (2.3434 ms: 148 partial-sum slots per row tile), both 430.2.  So the COLUMN pass deals its
-        // runs round-robin by default (needs nCB >= 4 * grid), the row pass keeps contiguous chunks.
-        // BIOEN_B200_PASS_ORDER = contiguous | icol | irow | interleave overrides.
-        {
-            const char* e = getenv("BIOEN_B200_PASS_ORDER");
-            const bool ok = nCB >= 4LL * grid;
-            interleave_row = ok && e && e[0] == 'i' && (e[1] == 'n' || e[1] == 'r');
-            interleave_col = ok && (!e || (e[0] == 'i' && (e[1] == 'n' || e[1] == 'c')));
-        }
-        slotsA = interleave_row ? grid : slots(nCB);
+        // runs round-robin (needs nCB >= 4 * grid), the row pass keeps contiguous chunks.
+        interleave_col = nCB >= 4LL * grid;
+        slotsA = slots(nCB);
         slotsB = slots(nRT);
-        int vb = 4;   // resident 256-thread blocks per SM for the O(N) kernels (measured: 2, 8, 16 are no faster)
-        if (const char* e = getenv("BIOEN_B200_VEC_BLOCKS")) vb = std::max(1, atoi(e));
+        const int vb = 4;   // resident 256-thread blocks per SM for the O(N) kernels (measured: 2, 8, 16 are no faster)
         vec_blocks_n = std::min((N + kVecThreads - 1) / kVecThreads, num_sms * vb);
         vec_blocks_m = std::min((M + kVecThreads - 1) / kVecThreads, num_sms * vb);
 
@@ -232,7 +231,6 @@ class Context {
         CUDA_CHECK(cudaFuncSetAttribute(stream_colgrad_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                         kPassSmemBytesF32));
         colgrad_part.alloc((size_t)grid * 3 + 8);
-        if (const char* e = getenv("BIOEN_B200_COLGRAD")) colgrad_opt = e[0] != '0';
         CUDA_CHECK(cudaFuncSetAttribute(persistent_eval_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                         kPassSmemBytes));
         CUDA_CHECK(cudaFuncSetAttribute(persistent_eval_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -245,12 +243,6 @@ class Context {
             CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, persistent_eval_kernel<float>,
                                                                      kPEvalThreads, kPassSmemBytesF32));
             coop_ok = coop && (long long)per_sm * num_sms >= grid;
-            if (const char* e = getenv("BIOEN_B200_PERSISTENT")) persistent_mode = atoi(e);
-            if (const char* e = getenv("BIOEN_B200_LBFGS_GRAM")) lbfgs_gram_opt = e[0] == '1';
-            if (const char* e = getenv("BIOEN_B200_FETCH")) fetch_zero_copy = strcmp(e, "memcpy") != 0;
-            if (const char* e = getenv("BIOEN_B200_LBFGS_SMALL")) lbfgs_small_opt = e[0] != '0';
-            if (const char* e = getenv("BIOEN_B200_LBFGS_SPECULATIVE")) lbfgs_speculative = e[0] != '0';
-            if (const char* e = getenv("BIOEN_B200_PERSISTENT_MAX_MB")) persistent_max_bytes = atof(e) * 1.0e6;
             // slice kernel: plan once per context (M, N are fixed), tables only when the problem is eligible
             cudaFuncAttributes fa{};
             int optin = 0;
@@ -269,7 +261,6 @@ class Context {
                 slice_gtab.alloc((size_t)slice_pl.grid * slice_pl.ms);
                 slice_part.alloc((size_t)kSliceGP * 3 + 8);
             }
-            if (const char* e = getenv("BIOEN_B200_SLICE")) slice_mode = atoi(e);
         }
     }
 
@@ -288,17 +279,9 @@ class Context {
         have_logw = have_forces = false;
         fused_ready = false;
         yt_valid = false;
-        allow_fused = true;
-        lazy_gradient = true;
-        fuse_allowed = true;
+        options = ContextOptions{};
         eval_fused = false;
         forces_x = nullptr;
-        lbfgs_gram_opt = getenv("BIOEN_B200_LBFGS_GRAM") != nullptr && getenv("BIOEN_B200_LBFGS_GRAM")[0] == '1';
-        lbfgs_small_opt = !(getenv("BIOEN_B200_LBFGS_SMALL") && getenv("BIOEN_B200_LBFGS_SMALL")[0] == '0');
-        persistent_mode = -1;
-        if (const char* e = getenv("BIOEN_B200_PERSISTENT")) persistent_mode = atoi(e);
-        slice_mode = -1;
-        if (const char* e = getenv("BIOEN_B200_SLICE")) slice_mode = atoi(e);
         comm = nullptr;
         nranks = 1;
         N_total = N;
@@ -331,8 +314,7 @@ class Context {
         cudaPointerAttributes attr{};
         const bool pinned = cudaPointerGetAttributes(&attr, host) == cudaSuccess && attr.type == cudaMemoryTypeHost;
         cudaGetLastError();
-        const char* mode = getenv("BIOEN_B200_UPLOAD");   // "plain" forces one cudaMemcpy2D (diagnostics)
-        if (pinned || total < ((size_t)256 << 20) || (mode && !strcmp(mode, "plain"))) {
+        if (pinned || total < ((size_t)256 << 20)) {
             CUDA_CHECK(cudaMemcpy2DAsync(Y, ld * sizeof(double), host, ld_host * sizeof(double),
                                          (size_t)N * sizeof(double), M, cudaMemcpyHostToDevice, stream));
             sync();
@@ -372,9 +354,7 @@ class Context {
         const size_t buf_bytes = std::max(row_bytes, (size_t)32 << 20);
         const int rows_per_chunk = (int)std::max<size_t>(1, buf_bytes / row_bytes);
         const int nchunks = (M + rows_per_chunk - 1) / rows_per_chunk;
-        int want = kUpThreads;
-        if (const char* e = getenv("BIOEN_B200_UPLOAD_THREADS")) want = std::max(1, atoi(e));
-        const int nthreads = std::min(want, nchunks);
+        const int nthreads = std::min(kUpThreads, nchunks);
         const size_t lane_bytes = (size_t)rows_per_chunk * row_bytes;
         if ((int)up_lanes.size() < nthreads || (!up_lanes.empty() && up_lanes[0].bytes < lane_bytes)) {
             release_upload_lanes();
@@ -537,7 +517,7 @@ class Context {
         aux_n2.ensure(Npad + 8);  // lr_j
         have_forces = true;
         have_logw = false;        // Gv now holds w0
-        if (allow_fused && (Y || yt_only) && !storage_fp32 && !fused_ready) prepare_fused();
+        if (options.allow_fused && (Y || yt_only) && !storage_fp32 && !fused_ready) prepare_fused();
         if (yt_only && !fused_ready)
             throw std::logic_error("bioen_b200: structure-major-only mode: the fused forces kernels are not available "
                                    "for this problem (BIOEN_B200_OPT_FUSED_FORCES = 0, or M outside 256..~5500)");
@@ -656,10 +636,6 @@ class Context {
             // team variant: T warps per structure, 8/T independent teams per CTA.  Measured at M = 1000:
             // T = 1 (eight independent warps) 1.28 ms per pass, T = 2 1.34 ms, T = 4 2.1 ms.
             f_T = ldt <= 1024 ? 1 : ldt <= 2048 ? 2 : ldt <= 4096 ? 4 : 8;
-            if (const char* e = getenv("BIOEN_B200_FUSED_T")) {
-                const int t = atoi(e);
-                if ((t == 1 || t == 2 || t == 4 || t == 8) && ldt <= 1024LL * t) f_T = t;
-            }
             const int teams = kTWarps / f_T;
             const long long need = (ldt + 64LL * f_T - 1) / (64LL * f_T);
             f_KI = need <= 4 ? 4 : need <= 8 ? 8 : 16;
@@ -675,7 +651,6 @@ class Context {
                 const long long want = std::max(2LL, (131072 + per_stage / 2) / per_stage);
                 st = std::min(st, want);
             }
-            if (const char* e = getenv("BIOEN_B200_FUSED_STAGES")) st = std::min(st, (long long)std::max(2, atoi(e)));
             if (st >= 2) {
                 f_team = true;
                 f_stages = (int)st;
@@ -787,7 +762,9 @@ class Context {
         finalize_rows_from_msum(true, false);
     }
     // sharded fused forces path: exchanges issued inside the producing kernels (needs the peer-memory path)
-    bool fuse_exchange_forces() const { return nranks > 1 && comm && comm->fused_ok((size_t)M + 8) && fuse_allowed; }
+    bool fuse_exchange_forces() const {
+        return nranks > 1 && comm && comm->fused_ok((size_t)M + 8) && options.fuse_allowed;
+    }
     P2PDev p2p_dev_raw() const { ++comm->exchanges; return comm->dev_args(); }
     void rows_finish(bool scaled, int ntail, bool gradient, double* grad, const double* ddir) {
         RowsFinishArgs a{};
@@ -808,7 +785,7 @@ class Context {
         merge_fused_rows(false, 0);
         {
             ForcesGradArgs a{};
-            a.m = M; a.partial = nullptr; a.ld = Mpad; a.L = nCB; a.chunk = row_chunk(); a.msum = msum.p;
+            a.m = M; a.partial = nullptr; a.ld = Mpad; a.L = nCB; a.chunk = chunk; a.msum = msum.p;
             a.d = ddir; a.grad = grad; a.sc = sc.p;
             k_forces_grad<<<1, 1024, 0, stream>>>(a);
             ++kernels_launched;
@@ -817,7 +794,7 @@ class Context {
     // k_finalize_rows on an msum that is already slot-, CTA- and rank-reduced
     void finalize_rows_from_msum(bool is_forces, bool ab_with_avg) {
         FinalizeArgs a{};
-        a.m = M; a.partial = nullptr; a.ld = Mpad; a.L = nCB; a.chunk = row_chunk(); a.msum = msum.p;
+        a.m = M; a.partial = nullptr; a.ld = Mpad; a.L = nCB; a.chunk = chunk; a.msum = msum.p;
         a.Y = Yobs.p; a.ab = ab.p; a.avg = avg.p; a.ab_with_avg = ab_with_avg ? 1 : 0;
         a.is_forces = is_forces ? 1 : 0; a.theta = theta;
         a.partials = red_partials.p; a.ticket = ticket.p; a.sc = sc.p;
@@ -834,8 +811,9 @@ class Context {
     }
     // Sharded log-weights evaluation with the exchanges inside the producing kernels (peer-memory path only): the
     // normalisation pair travels with the row sums, so the objective half needs ONE exchange and no exchange launch.
-    bool fuse_exchange() const { return nranks > 1 && comm && comm->fused_ok((size_t)M + 5) && fuse_allowed; }
-    bool fuse_allowed = true;   // BIOEN_B200_OPT_FUSED_EXCHANGE
+    bool fuse_exchange() const {
+        return nranks > 1 && comm && comm->fused_ok((size_t)M + 5) && options.fuse_allowed;
+    }
     P2PDev p2p_dev() const {
         if (nranks > 1 && comm && fuse_exchange()) { ++comm->exchanges; return comm->dev_args(); }
         P2PDev d{};
@@ -863,7 +841,7 @@ class Context {
     void launch_pass(const double* vN, const double* vMb) {
         PassArgs a{};
         a.nRT = nRT; a.nCB = nCB; a.T = T; a.chunk = chunk;
-        a.interleave = ((MODE == kRowPass) ? interleave_row : interleave_col) ? 1 : 0;
+        a.interleave = (MODE == kColPass && interleave_col) ? 1 : 0;
         a.evict_first = evict_first;
         a.vN = vN; a.vMb = vMb; a.ab = ab.p;
         a.partial = (MODE == kRowPass) ? partialA.p : partialB.p;
@@ -885,7 +863,6 @@ class Context {
     // on this stream between begin_pass_timing() and end_pass_timing(), which returns the mean duration in ms
     std::vector<cudaEvent_t> pass_ev;
     size_t pass_ev_used = 0;
-    long long pass_ev_passes = 0;   // passes bracketed by the event pairs beyond one per pair (persistent kernel)
     bool pass_timing = false;
     void begin_pass_timing(int max_passes) {
         while (pass_ev.size() < (size_t)max_passes * 2) {
@@ -894,7 +871,6 @@ class Context {
             pass_ev.push_back(e);
         }
         pass_ev_used = 0;
-        pass_ev_passes = 0;
         pass_timing = true;
     }
     float end_pass_timing() {
@@ -908,18 +884,18 @@ class Context {
             total += t;
             ++cnt;
         }
-        return cnt ? (float)(total / (double)(cnt + pass_ev_passes)) : 0.f;
+        return cnt ? (float)(total / (double)cnt) : 0.f;
     }
     // finish a row pass that produced avg (logw: tail = 3 weighted sums, forces: tail = KL)
     void finalize_rows(bool is_forces, int ntail, bool ab_with_avg) {
         FinalizeArgs a{};
-        a.m = M; a.partial = partialA.p; a.ld = Mpad; a.L = nCB; a.chunk = row_chunk();
+        a.m = M; a.partial = partialA.p; a.ld = Mpad; a.L = nCB; a.chunk = chunk;
         a.Y = Yobs.p; a.ab = ab.p; a.avg = avg.p; a.ab_with_avg = ab_with_avg ? 1 : 0;
         a.is_forces = is_forces ? 1 : 0; a.theta = theta;
         a.partials = red_partials.p; a.ticket = ticket.p; a.sc = sc.p;
         a.tail = msum.p + M;
         if (nranks > 1) {
-            k_reduce_row_slots<<<vec_blocks_m, kVecThreads, 0, stream>>>(M, partialA.p, Mpad, nCB, row_chunk(), msum.p);
+            k_reduce_row_slots<<<vec_blocks_m, kVecThreads, 0, stream>>>(M, partialA.p, Mpad, nCB, chunk, msum.p);
             ++kernels_launched;
             comm->allreduce_sum(msum.p, M + ntail, stream);
             a.msum = msum.p;
@@ -940,8 +916,8 @@ class Context {
     // precedence over the persistent kernel AND over the fused two-pass forces kernels whenever the problem is small
     // enough (slice_plan); BIOEN_B200_OPT_PERSISTENT = 0 (stand-alone kernels) switches it off as well.
     bool slice_ok() const {
-        return slice_pl.ok && slice_coop && slice_mode != 0 && persistent_mode != 0 && nranks == 1 && Y != nullptr &&
-               !storage_fp32 && (ld % 2) == 0 && ld >= N && (reinterpret_cast<uintptr_t>(Y) & 15) == 0;
+        return slice_pl.ok && slice_coop && options.slice_mode != 0 && options.persistent_mode != 0 && nranks == 1 &&
+               Y != nullptr && !storage_fp32 && (ld % 2) == 0 && ld >= N && (reinterpret_cast<uintptr_t>(Y) & 15) == 0;
     }
     void launch_slice(int method, int mode, double* x, const double* xp, const double* d, double stp,
                       double* grad, const double* ddir) {
@@ -954,11 +930,6 @@ class Context {
         a.Gv = Gv.p; a.w = w.p; a.aux_n = aux_n.p; a.aux_n2 = aux_n2.p; a.grad = grad; a.ddir = ddir;
         a.Yobs = Yobs.p; a.ab = ab.p; a.avg = avg.p; a.theta = theta; a.sc = sc.p;
         a.tab = slice_tab.p; a.gtab = slice_gtab.p; a.part = slice_part.p; a.bar = pe_bar.p; a.ticket = ticket.p;
-        static const bool want_trace = getenv("BIOEN_B200_PERSISTENT_TRACE") != nullptr;
-        if (want_trace) {
-            if (!pe_trace.p) pe_trace.alloc(64);
-            a.trace = pe_trace.p;
-        }
         // algorithmic passes of the evaluation (the kernel reads the matrix once).  No per-pass events here: a launch is
         // a whole evaluation of ~20 us, and two timing events around it cost a visible share of that.
         const int npass = method == 0 ? (mode == kPEvalBoth ? 2 : 1) : (mode == kPEvalBoth ? 4 : 2);
@@ -969,21 +940,11 @@ class Context {
         ++kernels_launched;
         ++persistent_launches;
         ++slice_launches;
-        if (want_trace && (slice_launches % 16) == 0) {
-            unsigned long long h[40];
-            sync();
-            CUDA_CHECK(cudaMemcpy(h, pe_trace.p, sizeof(h), cudaMemcpyDeviceToHost));
-            fprintf(stderr, "[slice trace] method %d mode %d grid %d nc %d: phase boundaries (us since kernel start):",
-                    method, mode, slice_pl.grid, slice_pl.nc);
-            for (int k = 1; k < 40 && h[k] >= h[0] && h[k] - h[0] < 10000000ull; ++k) fprintf(stderr, " %.1f", (h[k] - h[0]) * 1e-3);
-            fprintf(stderr, "\n");
-            CUDA_CHECK(cudaMemset(pe_trace.p, 0, 64 * sizeof(unsigned long long)));
-        }
     }
     bool persistent_for(bool forces) const {
         if (slice_ok()) return true;
-        if (!coop_ok || persistent_mode == 0 || !has_matrix()) return false;
-        if (persistent_mode < 0 && matrix_bytes() > persistent_max_bytes) return false;
+        if (!coop_ok || options.persistent_mode == 0 || !has_matrix()) return false;
+        if (options.persistent_mode < 0 && matrix_bytes() > kPersistentMaxBytes) return false;
         if (forces) return nranks == 1 && !forces_fused_now();
         if (nranks > 1) return fuse_exchange() && !comm->is_local();
         return true;
@@ -1001,63 +962,27 @@ class Context {
         a.row.evict_first = evict_first; a.row.partial = partialA.p; a.row.ld = Mpad;
         a.col = a.row;
         a.col.partial = partialB.p; a.col.ld = Npad;
-        // experiment (BIOEN_B200_PERSISTENT_ICOL=1): deal the runs of the column pass round-robin as the stand-alone
-        // kernel does by default.  Measured at config 2 (0.4 GB): 150.2 us vs 149.1 us contiguous -- no gain for the
-        // matrix sizes this kernel is used for, so the contiguous order stays.
-        if (nCB >= 4LL * grid && getenv("BIOEN_B200_PERSISTENT_ICOL")) {
-            a.col.interleave = 1;
-            a.col.chunk = nRT;
-        }
         a.x = x; a.xp = xp; a.d = d; a.stp = stp;
         a.Gv = Gv.p; a.w = w.p; a.aux_n = aux_n.p; a.aux_n2 = aux_n2.p; a.grad = grad; a.ddir = ddir;
         a.Yobs = Yobs.p; a.ab = ab.p; a.avg = avg.p; a.msum = msum.p; a.theta = theta; a.sc = sc.p;
         a.part = pe_part.p; a.bar = pe_bar.p; a.ticket = ticket.p;
         if (method == 0 && nranks > 1) a.p2p = p2p_dev(); else a.p2p.nranks = 1;
-        static const bool want_trace = getenv("BIOEN_B200_PERSISTENT_TRACE") != nullptr;
-        if (want_trace) {
-            if (!pe_trace.p) pe_trace.alloc(64);
-            a.trace = pe_trace.p;
-        }
-        // (the kernel's own passes and their readers always use the contiguous tile order, whatever the stand-alone
-        // kernels of this context are configured for)
+        // The kernel's passes and their readers use the contiguous tile order for both passes: dealing the column
+        // pass's runs round-robin, as the stand-alone kernel does, measured 150.2 us vs 149.1 us contiguous at config 2
+        // (0.4 GB) -- no gain for the matrix sizes this kernel is used for.
+        // No per-launch events: a launch is a whole evaluation, so the callers that time evaluations
+        // (bioen_b200_time_evals) derive the per-pass figure from the step time instead of paying two timing events
+        // per launch inside the timed region.  Cooperative launch = the driver's guarantee that all CTAs are resident
+        // (the grid barriers need it).
         const int npass = method == 0 ? (mode == kPEvalBoth ? 2 : 1) : (mode == kPEvalBoth ? 4 : 2);
-        // per-launch events only on request (BIOEN_B200_PERSISTENT_EVENTS=1): a launch is a whole evaluation, so the
-        // callers that time evaluations (bioen_b200_time_evals) derive the per-pass figure from the step time instead
-        // of paying two timing events per launch inside the timed region
-        static const bool launch_events = getenv("BIOEN_B200_PERSISTENT_EVENTS") != nullptr;
-        const bool timed = launch_events && pass_timing && pass_ev_used + 2 <= pass_ev.size();
-        if (timed) CUDA_CHECK(cudaEventRecord(pass_ev[pass_ev_used++], stream));
-        // Cooperative launch = the driver's guarantee that all CTAs are resident (the grid barriers need it).
-        // BIOEN_B200_PERSISTENT_PLAIN=1 (diagnostics): an ordinary launch, which is resident as well when nothing
-        // else runs on the device (grid <= SM count, 1 CTA per SM) but is not guaranteed to be.
-        static const bool plain = getenv("BIOEN_B200_PERSISTENT_PLAIN") != nullptr;
-        if (plain) {
-            if (storage_fp32) persistent_eval_kernel<float><<<grid, kPEvalThreads, kPassSmemBytesF32, stream>>>(tmap, a);
-            else persistent_eval_kernel<double><<<grid, kPEvalThreads, kPassSmemBytes, stream>>>(tmap, a);
-            CUDA_CHECK(cudaGetLastError());
-        } else {
-            void* args[] = {(void*)&tmap, (void*)&a};
-            const void* fn = storage_fp32 ? (const void*)persistent_eval_kernel<float>
-                                          : (const void*)persistent_eval_kernel<double>;
-            CUDA_CHECK(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kPEvalThreads), args,
-                                                   (size_t)(storage_fp32 ? kPassSmemBytesF32 : kPassSmemBytes), stream));
-        }
-        if (timed) {
-            CUDA_CHECK(cudaEventRecord(pass_ev[pass_ev_used++], stream));
-            pass_ev_passes += npass - 1;   // one event pair brackets npass passes
-        }
+        void* args[] = {(void*)&tmap, (void*)&a};
+        const void* fn = storage_fp32 ? (const void*)persistent_eval_kernel<float>
+                                      : (const void*)persistent_eval_kernel<double>;
+        CUDA_CHECK(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kPEvalThreads), args,
+                                               (size_t)(storage_fp32 ? kPassSmemBytesF32 : kPassSmemBytes), stream));
         passes_launched += npass;
         ++kernels_launched;
         ++persistent_launches;
-        if (want_trace && (persistent_launches % 16) == 0) {
-            unsigned long long h[40];
-            sync();
-            CUDA_CHECK(cudaMemcpy(h, pe_trace.p, sizeof(h), cudaMemcpyDeviceToHost));
-            fprintf(stderr, "[persistent trace] method %d mode %d: phase boundaries (us since kernel start):", method, mode);
-            for (int k = 1; k < 40 && h[k] >= h[0] && h[k] - h[0] < 10000000ull; ++k) fprintf(stderr, " %.1f", (h[k] - h[0]) * 1e-3);
-            fprintf(stderr, "\n");
-            CUDA_CHECK(cudaMemset(pe_trace.p, 0, 64 * sizeof(unsigned long long)));
-        }
     }
 
     // ---- log-weights evaluation (c_bioen_kernels_logw.c:525-561) ------------------------------------------
@@ -1068,7 +993,6 @@ class Context {
     // that the gradient is not needed -- a backtracking trial that fails the Armijo test, GSL's f-then-df pattern --
     // skip or defer the second pass over Y).  eval_gen changes with every objective evaluation.
     long long eval_gen = 0;
-    bool lazy_gradient = true;   // BIOEN_B200_OPT_LAZY_GRADIENT: minimisers may use the split (results identical)
     void logw_eval(double* x, const double* xp, const double* d, double stp, double* grad, const double* ddir) {
         if (grad && persistent_for(false)) {
             NvtxRange nvtx("bioen:logw_eval(persistent)");
@@ -1105,7 +1029,7 @@ class Context {
         launch_pass<kRowPass, false>(w.p, nullptr);
         if (fused) {
             RowsExchangeArgs a{};
-            a.m = M; a.partial = partialA.p; a.ld = Mpad; a.L = nCB; a.chunk = row_chunk(); a.msum = msum.p;
+            a.m = M; a.partial = partialA.p; a.ld = Mpad; a.L = nCB; a.chunk = chunk; a.msum = msum.p;
             a.p2p = p2p_dev(); a.Y = Yobs.p; a.ab = ab.p; a.avg = avg.p; a.theta = theta; a.sc = sc.p;
             k_logw_rows_exchange_finalize<<<1, kRowsXThreads, 0, stream>>>(a);
             ++kernels_launched;
@@ -1115,7 +1039,7 @@ class Context {
     }
     // will logw_eval_g form the gradient inside the column pass (and so stream it out while the pass runs)?
     bool colgrad_eligible() const {
-        return colgrad_opt && (nranks == 1 || fuse_exchange()) && interleave_col && !persistent_for(false);
+        return (nranks == 1 || fuse_exchange()) && interleave_col && !persistent_for(false);
     }
     bool eval_fused = false;   // the last logw_eval_f left un-normalised e_j in `w` (fused sharded path)
     void logw_eval_g(const double* x, double* grad, const double* ddir) {
@@ -1128,7 +1052,7 @@ class Context {
         // single GPU, whole runs per CTA: the column pass forms the gradient itself (stream_colgrad_kernel)
         auto aligned16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
         const bool sharded_fused = nranks > 1 && eval_fused;
-        if (colgrad_opt && (nranks == 1 || sharded_fused) && interleave_col && aligned16(x) && aligned16(grad) &&
+        if ((nranks == 1 || sharded_fused) && interleave_col && aligned16(x) && aligned16(grad) &&
             aligned16(Gv.p) && aligned16(w.p)) {
             PassArgs pa{};
             pa.nRT = nRT; pa.nCB = nCB; pa.T = T; pa.chunk = chunk; pa.interleave = 1; pa.evict_first = evict_first;
@@ -1194,7 +1118,7 @@ class Context {
         if (grad) forces_eval_g(grad, ddir);
     }
     double* forces_x = nullptr;   // the forces vector of the last objective half (persistent gradient half)
-    bool forces_fused_now() const { return fused_ready && (allow_fused || yt_only); }
+    bool forces_fused_now() const { return fused_ready && (options.allow_fused || yt_only); }
     void forces_eval_f(double* x, const double* xp, const double* d, double stp) {
         if (!have_forces) throw std::logic_error("bioen_b200: forces data not set");
         ++eval_gen;
@@ -1247,10 +1171,10 @@ class Context {
         launch_pass<kRowPass, true>(aux_n.p, avg.p);                    // grad_i = sum_j (y_ij - avg_i) E_j
         {
             ForcesGradArgs a{};
-            a.m = M; a.partial = partialA.p; a.ld = Mpad; a.L = nCB; a.chunk = row_chunk();
+            a.m = M; a.partial = partialA.p; a.ld = Mpad; a.L = nCB; a.chunk = chunk;
             a.d = ddir; a.grad = grad; a.sc = sc.p;
             if (nranks > 1) {
-                k_reduce_row_slots<<<vec_blocks_m, kVecThreads, 0, stream>>>(M, partialA.p, Mpad, nCB, row_chunk(), msum.p);
+                k_reduce_row_slots<<<vec_blocks_m, kVecThreads, 0, stream>>>(M, partialA.p, Mpad, nCB, chunk, msum.p);
                 ++kernels_launched;
                 comm->allreduce_sum(msum.p, M, stream);
                 a.msum = msum.p;
@@ -1305,10 +1229,10 @@ class Context {
         launch_pass<kRowPass, true>(aux_n.p, avg.p);
         {
             ForcesGradArgs a{};
-            a.m = M; a.partial = partialA.p; a.ld = Mpad; a.L = nCB; a.chunk = row_chunk();
+            a.m = M; a.partial = partialA.p; a.ld = Mpad; a.L = nCB; a.chunk = chunk;
             a.d = nullptr; a.grad = grad; a.sc = sc.p;
             if (nranks > 1) {
-                k_reduce_row_slots<<<vec_blocks_m, kVecThreads, 0, stream>>>(M, partialA.p, Mpad, nCB, row_chunk(), msum.p);
+                k_reduce_row_slots<<<vec_blocks_m, kVecThreads, 0, stream>>>(M, partialA.p, Mpad, nCB, chunk, msum.p);
                 ++kernels_launched;
                 comm->allreduce_sum(msum.p, M, stream);
                 a.msum = msum.p;
@@ -1335,7 +1259,7 @@ class Context {
             return;
         }
         launch_pass<kRowPass, false>(w.p, nullptr);
-        k_reduce_row_slots<<<vec_blocks_m, kVecThreads, 0, stream>>>(M, partialA.p, Mpad, nCB, row_chunk(), msum.p);
+        k_reduce_row_slots<<<vec_blocks_m, kVecThreads, 0, stream>>>(M, partialA.p, Mpad, nCB, chunk, msum.p);
         ++kernels_launched;
         if (nranks > 1) comm->allreduce_sum(msum.p, M, stream);
         d2d(avg_out_dev, msum.p, M);
@@ -1347,13 +1271,6 @@ class Context {
     void spin_sync() {
         if (!fetch_ev) CUDA_CHECK(cudaEventCreateWithFlags(&fetch_ev, cudaEventDisableTiming));
         CUDA_CHECK(cudaEventRecord(fetch_ev, stream));
-        // BIOEN_B200_SPIN=0: block in the driver instead of spinning (frees the host core of every rank at the price
-        // of the driver's wake-up latency per line-search trial)
-        static const bool spin = !(getenv("BIOEN_B200_SPIN") && getenv("BIOEN_B200_SPIN")[0] == '0');
-        if (!spin) {
-            CUDA_CHECK(cudaEventSynchronize(fetch_ev));
-            return;
-        }
         cudaError_t e;
         while ((e = cudaEventQuery(fetch_ev)) == cudaErrorNotReady) {
         }
@@ -1363,12 +1280,11 @@ class Context {
     // straight into the page-locked host copy (mapped under unified addressing), fences at system scope and then
     // stores a sequence number; the host spins on that number.  This replaces a 512-byte copy-engine transfer + event
     // (several microseconds of DMA and driver latency) by posted PCIe writes from an SM -- visible at small problem
-    // sizes, where an evaluation takes ~20 us.  BIOEN_B200_OPT_FETCH_ZEROCOPY = 0 / BIOEN_B200_FETCH=memcpy: the copy.
-    bool fetch_zero_copy = true;
+    // sizes, where an evaluation takes ~20 us.  BIOEN_B200_OPT_FETCH_ZEROCOPY = 0: the copy.
     unsigned long long fetch_seq = 0;
     void fetch_scalars() {
         NvtxRange nvtx("bioen:fetch_scalars");
-        if (!fetch_zero_copy) {
+        if (!options.fetch_zero_copy) {
             d2h(h_sc, sc.p, SC_COUNT);
             spin_sync();
             return;

@@ -130,7 +130,7 @@ class VecOps {
     // fdf(x, g) for a caller that discards the gradient when f > f_limit (steepest_descent.c:117-127 retries with a
     // shorter step): the gradient half runs only when it will be kept
     double fdf_unless_above(double* x, double* g, double f_limit) {
-        if (!C.lazy_gradient) return fdf(x, g);
+        if (!C.options.lazy_gradient) return fdf(x, g);
         ++stats.n_fdf;
         if (forces) C.forces_eval_f(x, nullptr, nullptr, 0.0);
         else C.logw_eval_f(x, nullptr, nullptr, 0.0);
@@ -147,7 +147,7 @@ class VecOps {
     // df(x, g) for call sites where x still holds the point the immediately preceding f(x) evaluated
     // (directional_minimize.c evaluates f at a trial point and, if it is kept, the gradient there)
     void df_same_point(double* x, double* g) {
-        if (C.lazy_gradient && f_x == x && f_gen == C.eval_gen) df_continue(x, g);
+        if (C.options.lazy_gradient && f_x == x && f_gen == C.eval_gen) df_continue(x, g);
         else df(x, g);
     }
     void df(double* x, double* g) {
@@ -289,7 +289,7 @@ struct LineWrapper {
         if (alpha == df_key) return df_alpha;
         moveto(alpha);
         if (alpha != g_key) {
-            if (V.C.lazy_gradient && state_gen == V.C.eval_gen && alpha == state_key) V.df_continue(x_alpha, g_alpha);
+            if (V.C.options.lazy_gradient && state_gen == V.C.eval_gen && alpha == state_key) V.df_continue(x_alpha, g_alpha);
             else V.df(x_alpha, g_alpha);
             g_key = alpha;
         }

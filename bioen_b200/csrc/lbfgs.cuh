@@ -480,11 +480,11 @@ class Lbfgs {
 
     bool gram_mode() const {
         // sharded runs need the in-kernel exchange (the peer-memory path); m is liblbfgs' default 6
-        return C.lbfgs_gram_opt && prm.m == kGramM && (!reduce || C.fuse_exchange());
+        return C.options.lbfgs_gram_opt && prm.m == kGramM && (!reduce || C.fuse_exchange());
     }
     // small problems (n <= 1024): pair + two-loop recursion as ONE single-CTA kernel (k_lbfgs_update_small)
     bool small_mode() const {
-        return C.lbfgs_small_opt && n <= kSmallUpdateMaxN && prm.m == kSmallUpdateM && !reduce;
+        return C.options.lbfgs_small_opt && n <= kSmallUpdateMaxN && prm.m == kSmallUpdateM && !reduce;
     }
 
    private:
@@ -539,7 +539,7 @@ class Lbfgs {
         // More-Thuente reads the slope of every trial: plain f+g evaluation, one read-back
         // (not on the slice kernel: there a combined f+g launch costs ~4 us more than the objective alone, less than the
         // second launch and host round trip the split costs the ~87 % of trials whose gradient IS read)
-        if (!eval(xp, d, stp, d, (prm.linesearch != 0 && C.lazy_gradient && !C.slice_ok()) ? &ls : nullptr)) {
+        if (!eval(xp, d, stp, d, (prm.linesearch != 0 && C.options.lazy_gradient && !C.slice_ok()) ? &ls : nullptr)) {
             C.fetch_scalars();
             take_spec_slope();
         }
@@ -626,7 +626,7 @@ class Lbfgs {
         // arrives with the trial's own scalars: one host round trip per iteration instead of two.  (The one case
         // where the slope matters beforehand -- 0 < g.d, LBFGSERR_INCREASEGRADIENT -- then costs one evaluation
         // that liblbfgs would not have made; x and g are restored by the caller as after any failed search.)
-        spec_slope = !it.slope_known && C.lbfgs_speculative;
+        spec_slope = !it.slope_known && C.options.lbfgs_speculative;
         if (!it.slope_known && !spec_slope) {
             C.fetch_scalars();
             it.ls.set_slope(h[SC_DGINIT]);

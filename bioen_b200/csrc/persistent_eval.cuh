@@ -59,13 +59,7 @@ struct PEvalArgs {
     unsigned long long* bar;       // [0] arrival count, [16] generation (grid barrier)
     unsigned int* ticket;
     P2PDev p2p;          // nranks > 1: sharded log-weights run, exchanges inside the kernel
-    unsigned long long* trace;   // optional: CTA 0 stores %globaltimer at every phase boundary (diagnostics)
 };
-
-__device__ __forceinline__ void peval_mark(const PEvalArgs& a, int& k) {
-    if (a.trace && blockIdx.x == 0 && threadIdx.x == 0) a.trace[k] = global_timer_ns();
-    ++k;
-}
 
 // barriers a launch passes (diagnostics)
 __host__ __device__ inline int peval_num_barriers(int method, int mode, bool sharded) {
@@ -210,8 +204,6 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
     if (tid == kConsumerWarps * 32) prefetch_tensormap(&tmap);
     __syncthreads();
     double* mypart = a.part + (size_t)b * kPSlots;
-    int mk = 0;
-    peval_mark(a, mk);
     const bool sharded = a.p2p.nranks > 1;
 
     if (a.method == 0) {
@@ -231,7 +223,7 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
             }
             block_lse2(m, s, xn, red);
             if (tid == 0) { mypart[0] = m; mypart[1] = s; mypart[2] = xn; }
-            { peval_mark(a, mk); peval_grid_barrier(a, nbar); peval_mark(a, mk); }
+            peval_grid_barrier(a, nbar);
             // ---- V1: every CTA merges the G pairs in the same fixed order; weights and the prior sums
             m = -DBL_MAX; s = 0.0; xn = 0.0;
             for (int q = tid; q < G; q += kPEvalThreads) {
@@ -260,14 +252,14 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
             }
             block_sum<3>(v, red);
             if (tid == 0) { mypart[3] = v[0]; mypart[4] = v[1]; mypart[5] = v[2]; }
-            { peval_mark(a, mk); peval_grid_barrier(a, nbar); peval_mark(a, mk); }
+            peval_grid_barrier(a, nbar);
             // ---- P2: row pass  avg ~ Y . w
             {
                 PassArgs pa = a.row;
                 pa.vN = a.w;
                 peval_pass<kRowPass, false, T>(smem, &tmap, pa, prod, cons);
             }
-            { peval_mark(a, mk); peval_grid_barrier(a, nbar); peval_mark(a, mk); }
+            peval_grid_barrier(a, nbar);
             // ---- V3: finish the objective.  One GPU: EVERY CTA does it (identical values, fixed order; only CTA 0
             // writes the scalar file), which saves the grid barrier that would otherwise publish avg / ab to the
             // column pass.  Sharded: CTA 0 alone (it runs the exchange), then a barrier.
@@ -308,9 +300,7 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
                         a.msum[a.M + 3] = Mx; a.msum[a.M + 4] = S;
                     }
                     int fail;
-                    peval_mark(a, mk);
                     const double* in = p2p_deliver_and_wait(a.p2p, a.msum, a.M + 5, &fail);
-                    peval_mark(a, mk);
                     const long long cap = a.p2p.cap;
                     const int R = a.p2p.nranks;
                     if (tid == 0) {
@@ -354,8 +344,8 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
                 }
             }
             if (a.mode == kPEvalObjective) return;
-            if (sharded) { peval_mark(a, mk); peval_grid_barrier(a, nbar); peval_mark(a, mk); }
-            else { peval_mark(a, mk); peval_cta_fence(); peval_mark(a, mk); }   // (V5 reads <g>, <G> from the scalar file after the barrier that follows P4)
+            if (sharded) peval_grid_barrier(a, nbar);
+            else peval_cta_fence();   // (V5 reads <g>, <G> from the scalar file after the barrier that follows P4)
         }
         // ---- P4: column pass  c_j = sum_i r_i (y_ij - avg_i)
         {
@@ -363,7 +353,7 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
             pa.ab = a.ab;
             peval_pass<kColPass, true, T>(smem, &tmap, pa, prod, cons);
         }
-        { peval_mark(a, mk); peval_grid_barrier(a, nbar); peval_mark(a, mk); }
+        peval_grid_barrier(a, nbar);
         // ---- V5: gradient and its scalars; the CTA that arrives last finishes (and exchanges, sharded)
         {
             const double gbar = a.sc[SC_GBAR], Gbar = a.sc[SC_CAPGBAR];
@@ -384,7 +374,6 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
                 }
             }
             double v[3] = {dg, gn, gi};
-            peval_mark(a, mk);
             if (!grid_sum_max_last<2>(v, a.part, a.ticket, red)) return;
             if (!sharded) {
                 if (tid == 0) { a.sc[SC_DG] = v[0]; a.sc[SC_GNORM2] = v[1]; a.sc[SC_GINF] = v[2]; }
@@ -422,14 +411,14 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
             block_sum<1>(c, red);
             if (tid == 0 && b == 0) a.sc[SC_XNORM2] = c[0];
         }
-        { peval_mark(a, mk); peval_cta_fence(); peval_mark(a, mk); }
+        peval_cta_fence();
         // ---- P1: column pass  x_j = sum_i f_i y_ij
         {
             PassArgs pa = a.col;
             pa.ab = a.ab;
             peval_pass<kColPass, false, T>(smem, &tmap, pa, prod, cons);
         }
-        { peval_mark(a, mk); peval_grid_barrier(a, nbar); peval_mark(a, mk); }
+        peval_grid_barrier(a, nbar);
         // ---- V2: assemble x_j, CTA-local (max, sum w0 exp(x - max))
         double m = -DBL_MAX, s = 0.0, xn = 0.0;
         if (vec) {
@@ -445,7 +434,7 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
         }
         block_lse2(m, s, xn, red);
         if (tid == 0) { mypart[0] = m; mypart[1] = s; }
-        { peval_mark(a, mk); peval_grid_barrier(a, nbar); peval_mark(a, mk); }
+        peval_grid_barrier(a, nbar);
         // ---- V3: global (max, S); w_j, guarded log-ratio, KL
         m = -DBL_MAX; s = 0.0; xn = 0.0;
         for (int q = tid; q < G; q += kPEvalThreads)
@@ -473,14 +462,14 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
             block_sum<1>(v, red);
             if (tid == 0) mypart[3] = v[0];
         }
-        { peval_mark(a, mk); peval_grid_barrier(a, nbar); peval_mark(a, mk); }
+        peval_grid_barrier(a, nbar);
         // ---- P4: row pass  avg = Y . w
         {
             PassArgs pa = a.row;
             pa.vN = a.w;
             peval_pass<kRowPass, false, T>(smem, &tmap, pa, prod, cons);
         }
-        { peval_mark(a, mk); peval_grid_barrier(a, nbar); peval_mark(a, mk); }
+        peval_grid_barrier(a, nbar);
         // ---- V5 (every CTA, identical values; CTA 0 writes the scalars): avg, r, chi^2, objective; ab = {r_i, 0}
         if (a.mode == kPEvalObjective && b != 0) return;
         {
@@ -504,7 +493,7 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
             }
         }
         if (a.mode == kPEvalObjective) return;
-        { peval_mark(a, mk); peval_cta_fence(); peval_mark(a, mk); }
+        peval_cta_fence();
     }
     // ---- P6: column pass  t_j = sum_i r_i y_ij
     {
@@ -512,7 +501,7 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
         pa.ab = a.ab;
         peval_pass<kColPass, false, T>(smem, &tmap, pa, prod, cons);
     }
-    { peval_mark(a, mk); peval_grid_barrier(a, nbar); peval_mark(a, mk); }
+    peval_grid_barrier(a, nbar);
     // ---- V7: E_j = (theta (1 + lr_j) + t_j) w_j
     if (vec) {
         for (int j = j0; j < a.N; j += jstride) {
@@ -522,7 +511,7 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
             a.aux_n[j] = ((1.0 + a.aux_n2[j]) * a.theta + t) * a.w[j];
         }
     }
-    { peval_mark(a, mk); peval_grid_barrier(a, nbar); peval_mark(a, mk); }
+    peval_grid_barrier(a, nbar);
     // ---- P8: row pass  grad_i = sum_j (y_ij - avg_i) E_j
     {
         PassArgs pa = a.row;
@@ -530,7 +519,7 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
         pa.vMb = a.avg;
         peval_pass<kRowPass, true, T>(smem, &tmap, pa, prod, cons);
     }
-    { peval_mark(a, mk); peval_grid_barrier(a, nbar); peval_mark(a, mk); }
+    peval_grid_barrier(a, nbar);
     // ---- V9 (CTA 0): gradient and its scalars
     if (b == 0) {
         double dg = 0.0, gn = 0.0, gi = 0.0;
@@ -542,7 +531,6 @@ __global__ void __launch_bounds__(kPEvalThreads, 1)
         });
         block_sum2_max(dg, gn, gi, red);
         if (tid == 0) { a.sc[SC_DG] = dg; a.sc[SC_GNORM2] = gn; a.sc[SC_GINF] = gi; }
-        peval_mark(a, mk);
     }
 }
 

@@ -70,7 +70,6 @@ struct SliceArgs {
     double* part;        // [grid][3]                     scalars of the final grid reduction
     unsigned long long* bar;
     unsigned int* ticket;
-    unsigned long long* trace;
 };
 
 __device__ __forceinline__ void cp_async16(void* dst_smem, const void* src) {
@@ -78,11 +77,6 @@ __device__ __forceinline__ void cp_async16(void* dst_smem, const void* src) {
 }
 __device__ __forceinline__ void cp_async_commit_wait_all() {
     asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory");
-}
-
-__device__ __forceinline__ void slice_mark(const SliceArgs& a, int& k) {
-    if (a.trace && blockIdx.x == 0 && threadIdx.x == 0) a.trace[k] = global_timer_ns();
-    ++k;
 }
 
 // The one grid barrier of a launch: same sense-reversing scheme as peval_grid_barrier (arrival count + generation
@@ -253,8 +247,6 @@ __global__ void __launch_bounds__(kSliceThreads, 1) slice_eval_kernel(const Slic
     double* vg = vobs + Mp;                               // [nc]  G_j (logw) / w0_j (forces)
     double* vd = vg + nc;                                 // [nc]  logw: direction d_j of the slope grad . d
     double* mytab = a.tab + (size_t)b * ms;
-    int mk = 0;
-    slice_mark(a, mk);
 
     // ---- the slice: M rows x ceil2(nv) columns, 16-byte cp.async (row starts are 16-byte aligned: ld, c0, ncs even)
     {
@@ -305,12 +297,9 @@ __global__ void __launch_bounds__(kSliceThreads, 1) slice_eval_kernel(const Slic
             }
             cp_async_commit_wait_all();
             __syncthreads();
-            slice_mark(a, mk);
             slice_row_reduce<false>(sl, ncs, M, nv, ve, nullptr, a.l_log2,
                                     [&](int i, double sum) { mytab[kSliceHdr + i] = sum; });
-            slice_mark(a, mk);
             const bool ok = slice_grid_barrier(a.bar);
-            slice_mark(a, mk);
             // ---- B: every CTA combines the G contributions in CTA order (identical values everywhere)
             double mc = -DBL_MAX, t[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
             if (tid < G) {   // the six scalars of CTA `tid`, one L2 round trip
@@ -363,7 +352,6 @@ __global__ void __launch_bounds__(kSliceThreads, 1) slice_eval_kernel(const Slic
                 ve[jj] = w;
                 a.w[c0 + jj] = w;
             }
-            slice_mark(a, mk);
             if (a.mode == kPEvalObjective) return;
             __syncthreads();   // vr, vavg complete
         } else {
@@ -395,11 +383,9 @@ __global__ void __launch_bounds__(kSliceThreads, 1) slice_eval_kernel(const Slic
             gn = fma(gr, gr, gn);
             gi = fmax(gi, fabs(gr));
         }
-        slice_mark(a, mk);
         double v3[3] = {dg, gn, gi};
         if (!grid_sum_max_last<2>(v3, a.part, a.ticket, red)) return;
         if (tid == 0) { a.sc[SC_DG] = v3[0]; a.sc[SC_GNORM2] = v3[1]; a.sc[SC_GINF] = v3[2]; }
-        slice_mark(a, mk);
         return;
     }
 
@@ -421,7 +407,6 @@ __global__ void __launch_bounds__(kSliceThreads, 1) slice_eval_kernel(const Slic
         }
         cp_async_commit_wait_all();
         __syncthreads();
-        slice_mark(a, mk);
         slice_col_reduce<false>(sl, ncs, M, nv, vr, nullptr, vx, scratch, a.cx_log2);
         double m = -DBL_MAX;
         for (int jj = tid; jj < nv; jj += kSliceThreads) m = fmax(m, vx[jj]);
@@ -442,9 +427,7 @@ __global__ void __launch_bounds__(kSliceThreads, 1) slice_eval_kernel(const Slic
         __syncthreads();   // ve complete
         slice_row_reduce<false>(sl, ncs, M, nv, ve, nullptr, a.l_log2,
                                 [&](int i, double sum) { mytab[kSliceHdr + i] = sum; });
-        slice_mark(a, mk);
         const bool ok = slice_grid_barrier(a.bar);
-        slice_mark(a, mk);
         // ---- B: global (max, S), KL, avg, r, chi^2, objective -- in every CTA, CTA order
         double mc = -DBL_MAX, Sc = 0.0, Kc = 0.0, Uc = 0.0;
         if (tid < G) {
@@ -501,7 +484,6 @@ __global__ void __launch_bounds__(kSliceThreads, 1) slice_eval_kernel(const Slic
             a.aux_n2[j] = lr;
             a.aux_n[j] = x;
         }
-        slice_mark(a, mk);
         if (a.mode == kPEvalObjective) return;
         __syncthreads();   // vr, vavg, ve, vx complete
     } else {
@@ -528,7 +510,6 @@ __global__ void __launch_bounds__(kSliceThreads, 1) slice_eval_kernel(const Slic
         double* myg = a.gtab + (size_t)b * ms;
         slice_row_reduce<true>(sl, ncs, M, nv, ve, vavg, a.l_log2, [&](int i, double sum) { myg[i] = sum; });
     }
-    slice_mark(a, mk);
     // the CTA that arrives last adds the contributions in CTA order
     __syncthreads();
     if (tid == 0) {
@@ -561,7 +542,6 @@ __global__ void __launch_bounds__(kSliceThreads, 1) slice_eval_kernel(const Slic
             }
         }
     }
-    slice_mark(a, mk);
 }
 
 // ---- host side: geometry of a launch -------------------------------------------------------------------------

@@ -76,7 +76,7 @@ struct PassArgs {
     int nCB;            // number of column blocks ceil(N / kTileC)
     long long T;        // nRT * nCB
     long long chunk;    // tiles per CTA (contiguous order)
-    int interleave;     // 1: tiles (row pass) / whole runs (column pass) are dealt round-robin to the CTAs
+    int interleave;     // column pass only, 1: whole runs are dealt round-robin to the CTAs
     int evict_first;    // 1: stream yTilde through L2 with evict_first (matrix >> L2)
     const double* vN;   // ROW: v_j, length >= nCB*kTileC, zero padded
     const double* vMb;  // ROW with SUB: b_i, length >= nRT*kTileR, zero padded
@@ -85,13 +85,11 @@ struct PassArgs {
     long long ld;       // leading dimension of `partial`
 };
 
-// slots a run of length L starting at tile run*L occupies: first CTA and count.  chunk < 0 is how the readers of
-// an interleaved row pass are told that every one of the -chunk CTAs holds a slot of every run.
+// slots a run of length L starting at tile run*L occupies: first CTA and count
 __host__ __device__ inline long long pass_first_cta(long long run, long long L, long long chunk) {
-    return chunk < 0 ? 0 : (run * L) / chunk;
+    return (run * L) / chunk;
 }
 __host__ __device__ inline int pass_num_slots(long long run, long long L, long long chunk) {
-    if (chunk < 0) return (int)(-chunk);
     return (int)(((run + 1) * L - 1) / chunk - (run * L) / chunk) + 1;
 }
 
@@ -99,29 +97,24 @@ __host__ __device__ inline int pass_num_slots(long long run, long long L, long l
 // (row pass: the nCB tiles of a row tile; column pass: the nRT tiles of a column block).
 //   contiguous  CTA b owns tiles [b*chunk, (b+1)*chunk) of the run-major order: far-apart regions of the matrix
 //               are streamed at the same time.
-//   interleaved row pass: tile t goes to CTA t mod G; column pass: run r goes to CTA r mod G.  At any moment the
-//               whole chip reads one compact window of the matrix (every row a contiguous stretch of ~G KB), which
-//               the DRAM serves ~2-3 % faster (measured with a TMA-free probe, scripts/read_order_probe.py).
+//   interleaved (column pass only): run r goes to CTA r mod G.  At any moment the whole chip reads one compact
+//               window of the matrix (every row a contiguous stretch of ~G KB), which the DRAM serves ~2-3 % faster
+//               (measured with a TMA-free read probe).  Each run has one slot, written by the CTA that owns it.
 struct TileWalk {
     long long run, left, L;
-    int k, G, mode;   // mode 0 contiguous, 1 row-interleaved, 2 column-run-interleaved
+    int k, G;
+    bool interleaved;
     __host__ __device__ __forceinline__ void init(int pass_mode, const PassArgs& a, int b, int grid) {
         L = (pass_mode == kRowPass) ? a.nCB : a.nRT;
         G = grid;
-        if (!a.interleave) {
-            mode = 0;
+        interleaved = a.interleave != 0;
+        if (!interleaved) {
             const long long t0 = (long long)b * a.chunk;
             const long long t1 = (t0 + a.chunk < a.T) ? t0 + a.chunk : a.T;
             left = t1 > t0 ? t1 - t0 : 0;
             run = t0 / L;
             k = (int)(t0 - run * L);
-        } else if (pass_mode == kRowPass) {
-            mode = 1;
-            left = b < a.T ? (a.T - b + G - 1) / G : 0;
-            run = b / L;
-            k = (int)(b - run * L);
         } else {
-            mode = 2;
             const long long nruns = a.nCB;
             left = b < nruns ? ((nruns - b + G - 1) / G) * L : 0;
             run = b;
@@ -129,22 +122,16 @@ struct TileWalk {
         }
     }
     // does the current tile close the CTA's part of its run?
-    __host__ __device__ __forceinline__ bool closes_run() const {
-        return left == 1 || (mode == 1 ? (long long)k + G >= L : k + 1 == (int)L);
-    }
+    __host__ __device__ __forceinline__ bool closes_run() const { return left == 1 || k + 1 == (int)L; }
     __host__ __device__ __forceinline__ void advance() {
         --left;
-        if (mode == 1) {
-            long long kk = (long long)k + G;
-            while (kk >= L) { kk -= L; ++run; }
-            k = (int)kk;
-        } else if (++k == (int)L) {
+        if (++k == (int)L) {
             k = 0;
-            run += (mode == 2) ? G : 1;
+            run += interleaved ? G : 1;
         }
     }
     __host__ __device__ __forceinline__ long long slot(int b, long long chunk) const {
-        return mode == 0 ? (long long)b - pass_first_cta(run, L, chunk) : (mode == 1 ? b : 0);
+        return interleaved ? 0 : (long long)b - pass_first_cta(run, L, chunk);
     }
 };
 

@@ -180,8 +180,8 @@ int bioen_b200_set_theta(bioen_b200_ctx *ctx, double theta);
  * with the row sums: one exchange per objective half).  0 restores the three separate exchanges per evaluation.
  * BIOEN_B200_OPT_PERSISTENT (default -1 = by size; 0 off; 1 on): run an evaluation as ONE persistent cooperative
  * kernel (grid barriers between its phases, yTilde kept in L2 when it fits) instead of 6-11 kernel launches; auto
- * selects it for matrices up to 0.6 GB per GPU (environment: BIOEN_B200_PERSISTENT, BIOEN_B200_PERSISTENT_MAX_MB).
- * BIOEN_B200_OPT_LBFGS_GRAM (default 0; environment BIOEN_B200_LBFGS_GRAM=1): the L-BFGS direction update runs in
+ * selects it for matrices up to 0.6 GB per GPU.
+ * BIOEN_B200_OPT_LBFGS_GRAM (default 0): the L-BFGS direction update runs in
  * coefficient space -- 2 kernels and 1 exchange per iteration instead of 14 and 13.  Algebraically the two-loop
  * recursion of liblbfgs, but it rounds differently, so trajectories differ from the default path in the last bits.
  * BIOEN_B200_OPT_FP32_STORAGE (default 0; set to 1 AFTER the matrix is uploaded / generated): replace the resident fp64
@@ -189,16 +189,16 @@ int bioen_b200_set_theta(bioen_b200_ctx *ctx, double theta);
  * fp64, but the matrix entries carry fp32 rounding (relative 6e-8), so results are NOT within the 1e-11 parity bar
  * (measured: objective ~1e-8, gradient ~1e-7 relative; tests/test_gpu_fp32_storage.py).  Never the default.  The fused
  * forces kernels, the theta scan, downloads and row-affine transforms need the fp64 matrix and are unavailable.
- * BIOEN_B200_OPT_SLICE (default -1 = on when eligible; 0 off; environment BIOEN_B200_SLICE): problems small enough for
+ * BIOEN_B200_OPT_SLICE (default -1 = on when eligible; 0 off): problems small enough for
  * the CTAs to hold their columns of yTilde in shared memory (up to ~30 MB in all, e.g. every fixture of the
  * reference's test-suite and the ala5 example) run an evaluation as ONE cooperative kernel with ONE grid barrier: the
  * matrix is read once per launch and every sweep runs out of shared memory (csrc/slice_eval.cuh).  Takes precedence
  * over the persistent kernel and the fused forces kernels; BIOEN_B200_OPT_PERSISTENT = 0 disables it as well.
- * BIOEN_B200_OPT_LBFGS_SMALL (default 1; environment BIOEN_B200_LBFGS_SMALL=0): minimisations over at most 1024
+ * BIOEN_B200_OPT_LBFGS_SMALL (default 1): minimisations over at most 1024
  * variables (the forces method; log-weights with few structures) run the L-BFGS update -- the new (s, y) pair and the
  * two-loop recursion -- as ONE single-CTA kernel instead of 15 launches; same arithmetic, bit-identical up to 256
  * variables.
- * BIOEN_B200_OPT_LBFGS_SPECULATIVE (default 1; environment BIOEN_B200_LBFGS_SPECULATIVE=0): the first trial of a line
+ * BIOEN_B200_OPT_LBFGS_SPECULATIVE (default 1): the first trial of a line
  * search is enqueued behind the update without fetching the initial slope first (it arrives with the trial's scalars):
  * one host round trip per iteration instead of two.  Results are identical.
  * BIOEN_B200_OPT_STRUCTURE_MAJOR_ONLY (default 0; set to 1 before the matrix is uploaded / generated, or afterwards: the
@@ -209,9 +209,11 @@ int bioen_b200_set_theta(bioen_b200_ctx *ctx, double theta);
  * structure-major layout directly.  Available: forces evaluations and minimisers (256 <= M <= ~5500), weights,
  * averages, downloads; the log-weights method, the theta scan, row-affine transforms and the given-weights entry
  * points need the row-major matrix and fail with a message.
- * BIOEN_B200_OPT_FETCH_ZEROCOPY (default 1; environment BIOEN_B200_FETCH=memcpy): the 512-byte scalar file of an
+ * BIOEN_B200_OPT_FETCH_ZEROCOPY (default 1): the 512-byte scalar file of an
  * evaluation reaches the host through stores of a one-warp kernel into page-locked memory + a sequence number the host
- * spins on, instead of a copy-engine transfer and an event.  Same values; a few microseconds less per evaluation. */
+ * spins on, instead of a copy-engine transfer and an event.  Same values; a few microseconds less per evaluation.
+ * Options 1, 3, 4, 5, 6, 8, 9, 10 and 12 belong to the context; bioen_b200_create starts every one at its default
+ * (bioen_b200_query what = 10 reports which differ from it). */
 enum { BIOEN_B200_OPT_FUSED_FORCES = 1, BIOEN_B200_OPT_P2P = 2, BIOEN_B200_OPT_LAZY_GRADIENT = 3,
        BIOEN_B200_OPT_FUSED_EXCHANGE = 4, BIOEN_B200_OPT_PERSISTENT = 5, BIOEN_B200_OPT_LBFGS_GRAM = 6,
        BIOEN_B200_OPT_FP32_STORAGE = 7, BIOEN_B200_OPT_SLICE = 8, BIOEN_B200_OPT_LBFGS_SMALL = 9,
@@ -394,7 +396,8 @@ long long bioen_b200_kernels_launched(bioen_b200_ctx *ctx);
  * 4: bytes per element of the resident matrix (8, or 4 with BIOEN_B200_OPT_FP32_STORAGE); 5: one-launch evaluations
  * (persistent or slice kernel) so far; 6: of those, launches of the shared-memory slice kernel; 7: 1 if evaluations
  * run on the slice kernel now; 8: bytes of device memory held by the context's copies of yTilde (row-major +
- * structure-major + fp32); 9: 1 in structure-major-only mode.  Returns -1 for an unknown `what`. */
+ * structure-major + fp32); 9: 1 in structure-major-only mode; 10: bitmask with bit (1 << option) set for each of the
+ * options 1, 3, 4, 5, 6, 8, 9, 10 and 12 whose value differs from its default.  Returns -1 for an unknown `what`. */
 long long bioen_b200_query(bioen_b200_ctx *ctx, int what);
 /* copy `count` doubles of a device buffer the context holds (tests): what = 0 the scalar file (64), 1 weights, 2
  * averages, 3 / 4 the forces method's per-structure vectors, 5 the L-BFGS store of the last minimisation,

@@ -468,3 +468,20 @@ def test_zero_copy_scalar_fetch_is_transparent(oracle):
                 assert o[0][1] == out[0][0][1] and o[0][2] == out[0][0][2] and np.array_equal(o[0][0], out[0][0][0])
                 assert o[1][1] == out[0][1][1] and o[1][2] == out[0][1][2] and np.array_equal(o[1][0], out[0][1][0])
                 assert o[2] == out[0][2] and np.array_equal(o[3], out[0][3])
+
+
+def test_reused_context_starts_with_default_options():
+    """The options of bioen_b200_set_option live in one record of the context.  A small context is kept for reuse
+    when its Problem closes and handed to the next Problem of the same shape: that one must start with every option
+    at its default again (bioen_b200_query 10: bitmask of the options that differ from their defaults)."""
+    import bioen_b200
+    non_default = {1: 0, 3: 0, 4: 0, 5: 0, 6: 1, 8: 0, 9: 0, 10: 0, 12: 0}
+    d = load_golden("data_forces_M64xN64")
+    with bioen_b200.Problem(d["yTilde"]) as p:
+        assert p.query(10) == 0
+        for option, value in non_default.items():
+            p.set_option(option, value)
+        assert p.query(10) == sum(1 << option for option in non_default)
+        device = p.device
+    with bioen_b200.Problem(d["yTilde"], device=device) as q:
+        assert q.query(10) == 0

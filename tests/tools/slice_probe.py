@@ -1,6 +1,5 @@
 """Diagnostic (GPU box): device-timed f+g evaluations of small problems on the three launch paths -- stand-alone
-kernels (0), persistent kernel (1), shared-memory slice kernel (2).  BIOEN_B200_PERSISTENT_TRACE=1 adds the phase
-timestamps of CTA 0."""
+kernels (0), persistent kernel (1), shared-memory slice kernel (2)."""
 import os
 import sys
 
